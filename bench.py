@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 One "step" = one pass of the hot path over the whole tile: extract(/2000) -> bilinear(/2000) -> 14 tcgen05
 convolutions -> stitch(x2000) for every patch the rank owns.  Rank 0 prints ONE JSON line.
@@ -117,6 +118,28 @@ def cpu_sample(deep):
     return (444, 444) if deep else (892, 1340)
 
 
+DUMP_SAMPLE = 1 << 20          # rows (output pixels, parameters) kept by --dump-outputs from a larger array
+
+
+def sample_rows(n, limit=DUMP_SAMPLE, seed=20170928):
+    """A fixed, sorted set of at most `limit` row indices out of n, the same from run to run (numpy int64)."""
+    if n <= limit:
+        return np.arange(n)
+    return np.unique(np.random.RandomState(seed).randint(0, n, size=limit, dtype=np.int64))
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: write each array as dirname/<name>.npy (float32 / float64 only), at most 64 MB in all, so that two
+    builds can be compared output for output on the same seeded inputs."""
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values()), {k: a.dtype for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, total
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + '.npy'), np.ascontiguousarray(a))
+    log('dumped %d arrays (%.1f MB) to %s' % (len(arrays), total / 2 ** 20, dirname))
+
+
 def cpu_oracle_run(shape, steps, warmup, deep=False):
     """Time the CPU oracle end to end on an (H, W) 10 m synthetic scene; returns (Mpixel/s, s/step, threads, patches)."""
     import torch
@@ -192,12 +215,12 @@ def run_reference_train(args):
         return
     deep = args.model == 'vdsen2'
     n = 8 if deep else 32                                                # a bounded sample: one quarter of the DSen2 batch
-    sps, per, threads = cpu_train_run(deep, min(args.steps, 5), min(args.warmup, 1), n)
+    sps, per, threads = cpu_train_run(deep, args.steps, args.warmup, n)
     sample = ("%d patches of 32x32 (the GPU arm: %d per GPU) through the CPU oracle's step: torch-CPU fp32 autograd of the same "
               "graph, MAE, torch NAdam(momentum_decay=0.004) = the Keras-2 Nadam recurrence; %.2f s per step; TensorFlow/Keras "
               "not installable" % (n, 8 if deep else 128, per))
     line = {"impl": "reference", "metric": "train_samples_per_s", "value": sps, "unit": "samples/s", "n_gpus": args.gpus,
-            "steps": min(args.steps, 5), "warmup": min(args.warmup, 1), "ms_per_step": per * 1e3, "higher_is_better": True,
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": per * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "fp32", "data": "synthetic",
             "config": {"workload": "%s training step, MAE + Keras-2 Nadam, CPU sample of %d patches 32x32" % (
                 'VDSen2 (32x256)' if deep else 'DSen2 (6x128)', n), "batch_per_gpu": n, "cpu_sample_only": True},
@@ -298,6 +321,19 @@ def run_ours(args):
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     ms_step = ms_total / args.steps
     value = T * T / (ms_step * 1e-3) / 1e6
+    if args.dump_outputs:
+        # the super-resolved tile of the last timed step: a seeded sample of its pixels (all bands) and the full-resolution
+        # top-left corner, which spans several patch seams.  Each rank wrote only the pixels its patches own into a
+        # zero-filled canvas, so a sum over ranks assembles the whole tile's values.
+        idx = torch.from_numpy(sample_rows(T * T)).to(dev)
+        c = min(T, 512)
+        parts = [out.view(T * T, cout).index_select(0, idx), out[:c, :c].contiguous()]
+        if world > 1:
+            for t in parts:
+                dist.all_reduce(t)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"sr_pixel_sample": parts[0].cpu().numpy(), "sr_corner": parts[1].cpu().numpy()})
+        del parts
 
     # roofline of the dominant kernel (resblock convolutions), from the events recorded in the timed region
     pk = peaks()
@@ -473,10 +509,10 @@ def run_train(args):
             ms = float(t.item())
         return ms
 
-    losses = []
+    losses, last = [], [None]
 
     def step_dev():
-        tr.train_step(devb[:2], devb[2])
+        last[0] = tr.train_step(devb[:2], devb[2])
 
     def step_e2e():
         for d, h in zip(devb, host):
@@ -485,6 +521,14 @@ def run_train(args):
         losses.append(float(loss))                                      # device -> host read of the step's result
 
     ms = timed(step_dev)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the step receives after the last timed step: its loss / MSE and the updated fp32 master
+        # weights (a seeded sample of them when they exceed the dump budget, as VDSen2's 37.8 M do)
+        loss, mse = last[0]
+        idx = torch.from_numpy(sample_rows(tr.params.numel(), 4 * DUMP_SAMPLE)).to(dev)
+        dump_outputs(args.dump_outputs, {"loss": loss.double().cpu().numpy().reshape(1),
+                                         "mse": mse.double().cpu().numpy().reshape(1),
+                                         "params_sample": tr.params.index_select(0, idx).cpu().numpy()})
     ms_e2e = timed(step_e2e)
     # the one exchange step of the path: all-reduce of the flat fp32 gradient (1.79 M elements), timed on its own
     allreduce_us = None
@@ -553,8 +597,8 @@ def run_train(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=3)
-    ap.add_argument('--warmup', type=int, default=3)
+    ap.add_argument('--steps', type=int, default=None, help='timed steps (default 3; 50 for the GPU training step)')
+    ap.add_argument('--warmup', type=int, default=None, help='untimed steps first (default 3; 10 for the GPU training step)')
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--model', default='dsen2', choices=['dsen2', 'vdsen2'])
     ap.add_argument('--tile', type=int, default=10980)
@@ -565,10 +609,19 @@ def main():
     ap.add_argument('--workload', default='tile', choices=['tile', 'train'],
                     help="'tile' = the headline inference benchmark; 'train' = BASELINE.json configs[4] (training step)")
     ap.add_argument('--train-batch', type=int, default=0, help='patches per GPU and step (0 = the reference\'s: 128, or 8 with --model vdsen2)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed as DIR/<name>.npy (float32 / float64, at most 64 MB)')
     args = ap.parse_args()
-    if args.workload == 'train' and args.impl == 'ours':
-        if args.steps == 3:
-            args.steps, args.warmup = 50, 10
+    gpu_train = args.workload == 'train' and args.impl == 'ours'
+    if args.steps is None:
+        args.steps = 50 if gpu_train else 3
+    if args.warmup is None:
+        args.warmup = 10 if gpu_train else 3
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of the CUDA path (--impl ours)')
+    if gpu_train:
         run_train(args)
     elif args.impl == 'reference' and args.workload == 'train':
         run_reference_train(args)

@@ -154,12 +154,13 @@ def test_DSen2_60_synthetic_scenes_vs_oracle(env, seed):
 def test_rmse_gate_on_the_shipped_scenes_when_the_blobs_exist(env):
     """The north-star acceptance gate: DSen2 RMSE against the simulated ground truth within 0.5 % of the notebook's recorded
     values (Running_Demo_in_the_colab.ipynb:170,209,236).  The three ground-truth scenes and both weight files are listed
-    in the reference's .MISSING_LARGE_BLOBS, so this is skipped until they are supplied (DSEN2_DATA / DSEN2_MODELS, or
-    ../data and ../models relative to the test directory)."""
+    in the reference's .MISSING_LARGE_BLOBS and far larger than a test fixture, so this is skipped until they are supplied
+    (directories named by DSEN2_DATA and DSEN2_MODELS)."""
     import os
     from dsen2_b200 import demoDSen2, supres
-    data = os.environ.get('DSEN2_DATA', os.path.join(os.path.dirname(__file__), '..', '..', 'data'))
-    models = os.environ.get('DSEN2_MODELS', os.path.join(os.path.dirname(__file__), '..', '..', 'models'))
+    data, models = os.environ.get('DSEN2_DATA', ''), os.environ.get('DSEN2_MODELS', '')
+    if not data or not models:
+        pytest.skip("DSEN2_DATA / DSEN2_MODELS do not name the ground-truth scenes and shipped weights")
     cases = [('S2B_MSIL1C_20170725_T43WFQ.mat', False, 31.2404), ('S2A_MSIL1C_20171028_T34HCH.mat', True, 20.4089),
              ('S2B_MSIL1C_20170928_T18TWL.mat', False, 64.2276)]
     weights = [os.path.join(models, f) for f in ('s2_032_lr_1e-04.hdf5', 's2_030_lr_1e-05.hdf5')]

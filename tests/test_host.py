@@ -128,15 +128,71 @@ def test_load_full_model_file_layout(tmp_path):
     assert all(np.array_equal(a, b) for a, b in zip(ws, m2.get_weights()))
 
 
-def test_hdf5_reader_on_mat_fixture_if_reference_present(fingerprints):
-    path = '/root/reference/data/S2A_MSIL1C_20170527_T33UUB.mat'
-    if not os.path.exists(path):
-        pytest.skip("reference mount absent (GPU box)")
+def _write_mat73(path, arrays, chunk=(1, 128, 128)):
+    """A MATLAB v7.3 .mat file laid out the way the shipped scenes are: a 512-byte MATLAB header as HDF5 user block
+    (superblock base address 512), and each array a chunked dataset (v1 chunk B-tree) through the shuffle + deflate filters,
+    with MATLAB_class attributes.  dsen2_b200.hdf5.write_hdf5 only writes contiguous datasets, so the chunked path of the
+    reader is exercised with this file."""
+    import itertools
+    import struct
+    import zlib
+    from dsen2_b200 import hdf5 as h
+    w = h._Writer()
+    w.buf += b"\x00" * 96
+    members = {}
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a)
+        rank, cs = a.ndim, chunk[-a.ndim:]
+        keys = []
+        for offs in itertools.product(*[range(0, s, c) for s, c in zip(a.shape, cs)]):
+            block = np.zeros(cs, a.dtype)                          # edge chunks are stored whole, zero-padded
+            sub = a[tuple(slice(o, o + c) for o, c in zip(offs, cs))]
+            block[tuple(slice(0, n) for n in sub.shape)] = sub
+            shuffled = np.frombuffer(block.tobytes(), np.uint8).reshape(-1, a.itemsize).T.tobytes()
+            raw = zlib.compress(shuffled)
+            keys.append((len(raw), offs, w.alloc(raw)))
+        node = b"TREE" + struct.pack("<BBHQQ", 1, 0, len(keys), h._UNDEF, h._UNDEF)
+        for size, offs, addr in keys:
+            node += struct.pack("<II%dQQ" % (rank + 1), size, 0, *offs, 0, addr)
+        node += struct.pack("<II%dQ" % (rank + 1), 0, 0, *a.shape, 0)
+        btree = w.alloc(node)
+        filters = struct.pack("<BB6x", 1, 2) + struct.pack("<HHHHI4x", 2, 0, 1, 1, a.itemsize) + \
+            struct.pack("<HHHHI4x", 1, 0, 1, 1, 3)               # shuffle (element size), then deflate (level 3)
+        members[name] = w.object_header([
+            h._msg(0x01, h._ds_message(a.shape)),
+            h._msg(0x03, h._dt_message(a), flags=1),
+            h._msg(0x05, struct.pack("<BBBB", 2, 2, 0, 0)),
+            h._msg(0x08, struct.pack("<BBBQ%dI" % (rank + 1), 3, 2, rank + 1, btree, *cs, a.itemsize)),
+            h._msg(0x0B, filters),
+            h._attr_message("MATLAB_class", np.bytes_(b"single")),
+        ])
+    root = w.group(members, {})
+    sb = h._SIG + struct.pack("<BBBBBBBBHHI", 0, 0, 0, 0, 0, 8, 8, 0, 4, 16, 0)
+    sb += struct.pack("<QQQQ", 512, h._UNDEF, len(w.buf), h._UNDEF) + struct.pack("<QQII16x", 0, root, 0, 0)
+    w.buf[:96] = sb
+    header = b"MATLAB 7.3 MAT-file, Platform: GLNXA64, Created on: Sat May 27 12:00:00 2017 HDF5 schema 1.00 ."
+    with open(path, "wb") as fh:
+        fh.write(header.ljust(512, b" ") + bytes(w.buf))
+
+
+@pytest.fixture
+def malmo_mat(malmo, tmp_path):
+    """The Malmo scene (tests/golden/scene_malmo_u16.npz) as the reference's data/S2A_MSIL1C_20170527_T33UUB.mat stores it:
+    single-precision arrays, transposed to MATLAB's column-major order."""
+    path = tmp_path / 'S2A_MSIL1C_20170527_T33UUB.mat'
+    _write_mat73(str(path), {k: a.transpose() for k, a in zip(('im10', 'im20', 'im60'), malmo)})
+    return path
+
+
+def test_hdf5_reader_on_mat_fixture_if_reference_present(malmo_mat, fingerprints):
+    """The scene read back from a MATLAB v7.3 file has the sha1 of the arrays h5py read from the reference's .mat file."""
     import hashlib
     from dsen2_b200.hdf5 import File
-    f = File(path)
+    f = File(str(malmo_mat))
+    assert f['im10'].attrs['MATLAB_class'] == b'single'
     for k in ('im10', 'im20', 'im60'):
         a = f[k][()]
+        assert a.dtype == np.float32
         assert hashlib.sha1(np.ascontiguousarray(a).tobytes()).hexdigest()[:12] == fingerprints['malmo.' + k]
 
 
@@ -149,21 +205,20 @@ def test_weight_file_naming_convention():
     assert supres.weight_file(True, True).endswith('s2_034_lr_1e-04.hdf5')
 
 
-def test_demo_readh5_and_rmse(fingerprints, capsys):
-    """demoDSen2.py:14-35 mirrors: RMSE formula, readh5 on the shipped Malmoe scene when the reference tree is mounted."""
+def test_demo_readh5_and_rmse(malmo, malmo_mat, capsys):
+    """demoDSen2.py:14-35 mirrors: RMSE formula, readh5 on the Malmoe scene as a MATLAB v7.3 file."""
     from dsen2_b200 import demoDSen2
     a = np.arange(12, dtype=np.float32).reshape(3, 4)
     b = a + np.float32(2)
     assert demoDSen2.RMSE(a, b) == 2.0 and 'RMSE: 2.0000' in capsys.readouterr().out
-    path = '/root/reference/data/'
-    if not os.path.exists(path + 'S2A_MSIL1C_20170527_T33UUB.mat'):
-        pytest.skip('reference data not mounted')
+    path = str(malmo_mat.parent) + '/'
     old, demoDSen2.DATA_PATH = demoDSen2.DATA_PATH, path
     try:
         d10, d20, d60 = demoDSen2.readh5('S2A_MSIL1C_20170527_T33UUB.mat', im60=True)
     finally:
         demoDSen2.DATA_PATH = old
     assert d10.shape == (600, 600, 4) and d20.shape == (300, 300, 6) and d60.shape == (100, 100, 2) and d10.dtype == np.float32
+    assert all(np.array_equal(x, y) for x, y in zip((d10, d20, d60), malmo))
 
 
 def test_q_trunk_code_properties():

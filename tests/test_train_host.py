@@ -74,8 +74,10 @@ def test_gloo_world2_gradient_allreduce(tmp_path):
 
 def _worker_setup(rank, world, port, tmp):
     """What ``python -m torch.distributed.run -m dsen2_b200.supres_train`` does before training, on the gloo backend:
-    process group first, rank 0's weights everywhere, equal-length shards."""
-    os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank))
+    process group first, rank 0's weights everywhere, equal-length shards.  The ranks are CPU processes: with CUDA visible,
+    dist_setup would select device LOCAL_RANK, which a machine with fewer GPUs than ranks does not have."""
+    os.environ.update(MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank),
+                      CUDA_VISIBLE_DEVICES='')
     import torch.distributed as dist
     from dsen2_b200.DSen2Net import s2model
     assert train.dist_setup('gloo') == (rank, world)

@@ -249,9 +249,15 @@ class S2Model:
     def workspace_bytes(self, n, P):
         return int(_capi.lib().dsen2_s2model_workspace_bytes(n, P, sum(self.in_channels), self.feature_size))
 
-    def _buffers(self, dev, n, P):
+    def _buffers(self, dev, n, P, reuse_larger=False):
+        """Activation buffers for n patches of P x P.  ``reuse_larger``: views of the smallest cached set that holds n
+        patches, if there is one -- batches of active patches have arbitrary sizes, and a set per size would pile up."""
         torch = _capi.require_cuda()
         key = (dev.index, torch.cuda.current_stream().cuda_stream, n, P)
+        if reuse_larger and key not in self._workspace:
+            fits = [k for k in self._workspace if k[:2] == key[:2] and k[3] == P and k[2] >= n]
+            if fits:
+                return {name: t[:n] for name, t in self._workspace[min(fits, key=lambda k: k[2])].items()}
         buf = self._workspace.get(key)
         if buf is None:
             if len(self._workspace) > 8:
@@ -363,11 +369,12 @@ class S2Model:
                         "dsen2_s2model_forward")
         return out
 
-    def forward_images(self, d10, d20, d60, patch, border, first_patch, n, canvas, mul, timers=None):
+    def forward_images(self, d10, d20, d60, patch, border, first_patch, n, canvas, mul, timers=None, patch_ids=None):
         """Fused tile pipeline of the fast path: patches [first_patch, first_patch+n) are gathered straight
         from the HWC images (extract + bilinear + /mul), run through the network, and the pixels they own
         are written x mul into ``canvas`` (H, W, Cout).  No patch stack or prediction stack exists.  The images are
-        float32 or uint16 (digital numbers) HWC CUDA tensors."""
+        float32 or uint16 (digital numbers) HWC CUDA tensors.  ``patch_ids``: a CUDA int32 tensor of n patch indices to
+        run instead of the range (``first_patch`` is then ignored)."""
         torch = _capi.require_cuda()
         if not self.xin16:
             raise _capi.DSen2Error("forward_images needs a network with resblocks (num_layers > 0)")
@@ -376,21 +383,34 @@ class S2Model:
         imgs = [t for t in (d10, d20, d60) if t is not None]
         if any(t.dtype != d10.dtype for t in imgs) or d10.dtype not in (torch.float32, torch.uint16):
             raise ValueError("images must all be float32 or all be uint16")
+        if patch_ids is not None and not (patch_ids.is_cuda and patch_ids.dtype == torch.int32 and patch_ids.is_contiguous()
+                                          and tuple(patch_ids.shape) == (n,)):
+            raise ValueError("patch_ids must be a contiguous CUDA int32 tensor of %d ids" % n)
         img_dtype = _capi.IMG_U16 if d10.dtype == torch.uint16 else _capi.IMG_F32
         wts, biases, _wp, _bp = self._ensure_packed(dev)
         if n == 0:
             return canvas
         lib, ptr = _capi.lib(), _capi.ptr
-        buf = self._buffers(dev, n, patch)
+        buf = self._buffers(dev, n, patch, reuse_larger=patch_ids is not None)
         with torch.cuda.device(dev):
             st = _capi.stream_ptr()
-            self._timed(timers, 'prep', n, lambda: _capi.check(lib.dsen2_prep16_from_images(
-                ptr(d10), ptr(d20), ptr(d60), img_dtype, H, W, patch, border, first_patch, n, float(mul),
-                ptr(buf['xin_hi']), ptr(buf['xin_lo']), st), "dsen2_prep16_from_images"))
+            if patch_ids is None:
+                self._timed(timers, 'prep', n, lambda: _capi.check(lib.dsen2_prep16_from_images(
+                    ptr(d10), ptr(d20), ptr(d60), img_dtype, H, W, patch, border, first_patch, n, float(mul),
+                    ptr(buf['xin_hi']), ptr(buf['xin_lo']), st), "dsen2_prep16_from_images"))
+            else:
+                self._timed(timers, 'prep', n, lambda: _capi.check(lib.dsen2_prep16_from_images_ids(
+                    ptr(d10), ptr(d20), ptr(d60), img_dtype, H, W, patch, border, ptr(patch_ids), n, float(mul),
+                    ptr(buf['xin_hi']), ptr(buf['xin_lo']), st), "dsen2_prep16_from_images_ids"))
             self._trunk(buf, wts, biases, n, patch, st, timers)
-            self._timed(timers, 'conv_tail', n, lambda: _capi.check(lib.dsen2_conv_tail16_stitch(
-                *self._tail_args(buf, wts, biases), self.feature_size, n, patch, first_patch, border, H, W, float(mul),
-                ptr(canvas), st), "dsen2_conv_tail16_stitch"))
+            if patch_ids is None:
+                self._timed(timers, 'conv_tail', n, lambda: _capi.check(lib.dsen2_conv_tail16_stitch(
+                    *self._tail_args(buf, wts, biases), self.feature_size, n, patch, first_patch, border, H, W, float(mul),
+                    ptr(canvas), st), "dsen2_conv_tail16_stitch"))
+            else:
+                self._timed(timers, 'conv_tail', n, lambda: _capi.check(lib.dsen2_conv_tail16_stitch_ids(
+                    *self._tail_args(buf, wts, biases), self.feature_size, n, patch, ptr(patch_ids), border, H, W,
+                    float(mul), ptr(canvas), st), "dsen2_conv_tail16_stitch_ids"))
         return canvas
 
     def launches_per_forward(self):

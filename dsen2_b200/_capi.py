@@ -50,6 +50,14 @@ SIGNATURES = {
                                   c_int, c_int, c_void_p, c_void_p]),
     "dsen2_conv_tail16_stitch": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                          c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p]),
+    "dsen2_prep16_from_images_ids": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int,
+                                             c_float, c_void_p, c_void_p, c_void_p]),
+    "dsen2_conv_tail16_stitch_ids": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                             c_int, c_int, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p]),
+    "dsen2_nodata_patches": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float,
+                                     c_void_p, c_void_p, c_void_p]),
+    "dsen2_nodata_fill": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float,
+                                  c_int, c_void_p, c_void_p]),
     "dsen2_conv_resq256": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p,
                                    c_void_p, c_void_p]),
     "dsen2_conv_tail": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,

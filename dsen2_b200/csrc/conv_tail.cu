@@ -51,6 +51,7 @@ struct TailParams {
   float* out;
   int tail_mode;                      // 0: NCHW (n, cout, H, W) predictions; 1: stitched HWC canvas
   int first_patch, img_h, img_w, border, grid_ny, grid_nx;
+  const int* patch_ids;               // stitching form with IDS: batch entry b is patch patch_ids[b], not first_patch + b
 };
 
 template <int KPM>                     // 64-channel k-blocks per activation tensor: 2 (128 features) or 4 (256)
@@ -66,7 +67,7 @@ __device__ __forceinline__ int tail_stitch_tile_of(int y, int size, int S, int n
   return (size % S != 0 && y >= size - S) ? n - 1 : y / S;
 }
 
-template <int KPM>
+template <int KPM, bool IDS>
 __global__ void __launch_bounds__(kTThreads, 1)
 conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
                          const __grid_constant__ CUtensorMap tm_w, const TailParams p) {
@@ -184,11 +185,12 @@ conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid
           d.obase = (long long)b * p.cout * d.ostride + (long long)y * p.W + x;
         } else {
           const int S = p.H - 2 * p.border;
-          const int patch = p.first_patch + b;
+          const int patch = IDS ? __ldg(p.patch_ids + b) : p.first_patch + b;
           const int pty = patch / p.grid_nx, ptx = patch - pty * p.grid_nx;
           const int gy = min(pty * S, p.img_h - S) + y - p.border;
           const int gx = min(ptx * S, p.img_w - S) + x - p.border;
-          d.write = y >= p.border && y < p.H - p.border && x >= p.border && x < p.W - p.border &&
+          d.write = (!IDS || (patch >= 0 && patch < p.grid_ny * p.grid_nx)) &&
+                    y >= p.border && y < p.H - p.border && x >= p.border && x < p.W - p.border &&
                     tail_stitch_tile_of(gy, p.img_h, S, p.grid_ny) == pty && tail_stitch_tile_of(gx, p.img_w, S, p.grid_nx) == ptx;
           d.ostride = 1;
           d.obase = ((long long)gy * p.img_w + gx) * p.cout;
@@ -283,12 +285,12 @@ __global__ void pack_tail16_weights_kernel(const float* __restrict__ hwio, int F
   }
 }
 
-template <int KPM>
+template <int KPM, bool IDS>
 static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_lo, const void* d_w, int sms, cudaStream_t stream) {
   using Cfg = TailCfg<KPM>;
   static bool configured[64] = {};
   if (needs_config(configured)) {
-    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM, IDS>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   }
   const int F = KPM * 64;
   CUtensorMap hi, lo, w;
@@ -301,7 +303,7 @@ static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_
   const uint32_t wb[2] = {64, 128};
   if ((rc = make_tmap_f16_sw(&w, d_w, 2, wd, wb, 128)) != 0) return rc;
   const int grid = (int)(p.num_tiles < (uint32_t)sms ? p.num_tiles : (uint32_t)sms);
-  conv_tail_swapped_kernel<KPM><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
+  conv_tail_swapped_kernel<KPM, IDS><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
   return check_launch("conv_tail_swapped");
 }
 
@@ -335,8 +337,10 @@ static int tail16_common(TailParams& p, int features, const void* d_x_hi, const 
   p.bias = d_bias;
   p.skip_hi = (const __half*)d_xin_hi; p.skip_lo = (const __half*)d_xin_lo; p.skip_ch0 = skip_ch0;
   p.cout = cout; p.out = d_out;
-  return features == 256 ? launch_tail<4>(p, d_x_hi, d_x_lo, d_w, sms, (cudaStream_t)stream)
-                         : launch_tail<2>(p, d_x_hi, d_x_lo, d_w, sms, (cudaStream_t)stream);
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (p.patch_ids)
+    return features == 256 ? launch_tail<4, true>(p, d_x_hi, d_x_lo, d_w, sms, st) : launch_tail<2, true>(p, d_x_hi, d_x_lo, d_w, sms, st);
+  return features == 256 ? launch_tail<4, false>(p, d_x_hi, d_x_lo, d_w, sms, st) : launch_tail<2, false>(p, d_x_hi, d_x_lo, d_w, sms, st);
 }
 
 }  // namespace dsen2
@@ -364,10 +368,10 @@ extern "C" int dsen2_conv_tail16(const void* d_x_hi, const void* d_x_lo, const v
                        stream);
 }
 
-extern "C" int dsen2_conv_tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
-                                        const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
-                                        int n, int P, int first_patch, int border, int img_h, int img_w, float mul,
-                                        float* d_canvas, void* stream) {
+// the stitching form: patches first_patch + b, or d_patch_ids[b] when d_patch_ids is not null
+static int tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias, const void* d_xin_hi,
+                         const void* d_xin_lo, int skip_ch0, int cout, int feature_size, int n, int P, int first_patch,
+                         const int* d_patch_ids, int border, int img_h, int img_w, float mul, float* d_canvas, void* stream) {
   const int S = P - 2 * border;
   DSEN2_REQUIRE(P > 0 && border >= 0 && S > 0 && img_h >= S && img_w >= S && first_patch >= 0, DSEN2_E_BADARG,
                 "dsen2_conv_tail16_stitch: bad stitch geometry (P %d border %d image %dx%d)", P, border, img_h, img_w);
@@ -376,9 +380,27 @@ extern "C" int dsen2_conv_tail16_stitch(const void* d_x_hi, const void* d_x_lo, 
   p.out_mul = mul;
   p.first_patch = first_patch; p.img_h = img_h; p.img_w = img_w; p.border = border;
   p.grid_ny = ceil_div(img_h, S); p.grid_nx = ceil_div(img_w, S);
-  DSEN2_REQUIRE(first_patch + n <= p.grid_ny * p.grid_nx, DSEN2_E_BADARG,
+  p.patch_ids = d_patch_ids;
+  DSEN2_REQUIRE(d_patch_ids || first_patch + n <= p.grid_ny * p.grid_nx, DSEN2_E_BADARG,
                 "dsen2_conv_tail16_stitch: patch range [%d,%d) exceeds the %d tiles of the canvas", first_patch,
                 first_patch + n, p.grid_ny * p.grid_nx);
   return tail16_common(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, P, P, d_canvas,
                        stream);
+}
+
+extern "C" int dsen2_conv_tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                        const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
+                                        int n, int P, int first_patch, int border, int img_h, int img_w, float mul,
+                                        float* d_canvas, void* stream) {
+  return tail16_stitch(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P, first_patch,
+                       nullptr, border, img_h, img_w, mul, d_canvas, stream);
+}
+
+extern "C" int dsen2_conv_tail16_stitch_ids(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                            const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout,
+                                            int feature_size, int n, int P, const int* d_patch_ids, int border, int img_h,
+                                            int img_w, float mul, float* d_canvas, void* stream) {
+  DSEN2_REQUIRE(d_patch_ids, DSEN2_E_BADARG, "dsen2_conv_tail16_stitch_ids: null pointer");
+  return tail16_stitch(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P, 0, d_patch_ids,
+                       border, img_h, img_w, mul, d_canvas, stream);
 }

@@ -41,11 +41,6 @@ struct PrepSource {
   int s;              // upsampling factor to the 10 m patch (1 = none)
 };
 
-// image element -> float: exact for uint16 digital numbers (what GDAL hands s2_tiles_supres.py:311-315), so a
-// uint16 image and its float32 copy prepare bit-identical inputs
-__device__ __forceinline__ float ld_px(const float* p) { return __ldg(p); }
-__device__ __forceinline__ float ld_px(const uint16_t* p) { return (float)__ldg(p); }
-
 // value of band c of `src` at 10 m patch pixel (y, x): crop + symmetric pad (+ mirror bilinear) + /divisor
 template <typename T, int C, int OFF>
 __device__ __forceinline__ void prep_gather(const PrepSource& src, int si, int sj, int plr, int blr, int y, int x,
@@ -109,21 +104,23 @@ __global__ void prep16_from_patches_kernel(const float* __restrict__ x0, int c0,
   }
 }
 
-template <typename T>
+// IDS: batch entry b is patch ids[b] (a list of active patches) instead of first_patch + b
+template <typename T, bool IDS>
 __global__ void prep16_from_images_kernel(PrepSource s0, PrepSource s1, PrepSource s2, int nsrc, int plr, int blr, int P,
-                                          Tiling tl, int first_patch, long long total, float divisor,
-                                          __half* __restrict__ out_hi, __half* __restrict__ out_lo) {
+                                          Tiling tl, int first_patch, const int* __restrict__ ids, long long total,
+                                          float divisor, __half* __restrict__ out_hi, __half* __restrict__ out_lo) {
   const int PP = P * P;
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
     const int local = (int)(idx / PP);
     const int rem = (int)(idx - (long long)local * PP);
     const int y = rem / P, x = rem - y * P;
-    const int patch = first_patch + local;
+    const int patch = IDS ? __ldg(ids + local) : first_patch + local;
     float v[16];
 #pragma unroll
     for (int c = 0; c < 16; ++c) v[c] = 0.f;
-    if (patch < tl.n_i * tl.n_j) {               // surplus patches of the allocated stack stay zero (patches.py:32-39)
+    // surplus patches of the allocated stack stay zero (patches.py:32-39), and so do ids outside the tiling
+    if ((!IDS || patch >= 0) && patch < tl.n_i * tl.n_j) {
       const int ti = patch / tl.n_j, tj = patch - ti * tl.n_j;
       const int si = ti < tl.k_i ? ti * tl.stride : tl.last_i;
       const int sj = tj < tl.k_j ? tj * tl.stride : tl.last_j;
@@ -325,28 +322,29 @@ extern "C" int dsen2_prep16_from_patches(const float* d_x0, int c0, const float*
   return check_launch("prep16_from_patches");
 }
 
-extern "C" int dsen2_prep16_from_images(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H,
-                                        int W, int patch, int border, int first_patch, int num_patches, float divisor,
-                                        void* d_xin_hi, void* d_xin_lo, void* stream) {
-  DSEN2_REQUIRE(d_img10 && d_img20 && d_xin_hi && d_xin_lo, DSEN2_E_BADARG, "dsen2_prep16_from_images: null pointer");
+template <bool IDS>
+static int prep16_from_images(const char* name, const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype,
+                              int H, int W, int patch, int border, int first_patch, const int* d_patch_ids, int num_patches,
+                              float divisor, void* d_xin_hi, void* d_xin_lo, void* stream) {
+  DSEN2_REQUIRE(d_img10 && d_img20 && d_xin_hi && d_xin_lo && (!IDS || d_patch_ids), DSEN2_E_BADARG, "%s: null pointer", name);
   DSEN2_REQUIRE(img_dtype == DSEN2_IMG_F32 || img_dtype == DSEN2_IMG_U16, DSEN2_E_BADARG,
-                "dsen2_prep16_from_images: img_dtype must be DSEN2_IMG_F32 or DSEN2_IMG_U16 (got %d)", img_dtype);
+                "%s: img_dtype must be DSEN2_IMG_F32 or DSEN2_IMG_U16 (got %d)", name, img_dtype);
   const int r = d_img60 ? 6 : 2;                 // the tiling grid is the coarsest input (patches.py:45-53,114-122)
   DSEN2_REQUIRE(H > 0 && W > 0 && H % r == 0 && W % r == 0, DSEN2_E_BADARG,
-                "dsen2_prep16_from_images: 10 m size %dx%d must be a multiple of %d", H, W, r);
+                "%s: 10 m size %dx%d must be a multiple of %d", name, H, W, r);
   DSEN2_REQUIRE(patch > 0 && border >= 0 && patch % r == 0 && border % r == 0 && patch > 2 * border, DSEN2_E_BADARG,
-                "dsen2_prep16_from_images: patch %d / border %d must be multiples of %d", patch, border, r);
+                "%s: patch %d / border %d must be multiples of %d", name, patch, border, r);
   DSEN2_REQUIRE(first_patch >= 0 && num_patches >= 0 && divisor != 0.f, DSEN2_E_BADARG,
-                "dsen2_prep16_from_images: bad patch range / divisor");
+                "%s: bad patch range / divisor", name);
   DSEN2_REQUIRE(((uintptr_t)d_xin_hi % 16) == 0 && ((uintptr_t)d_xin_lo % 16) == 0, DSEN2_E_ALIGN,
-                "dsen2_prep16_from_images: outputs must be 16-byte aligned");
+                "%s: outputs must be 16-byte aligned", name);
   const int plr = patch / r, blr = border / r, gh = H / r, gw = W / r;
   DSEN2_REQUIRE(gh + 2 * blr >= plr && gw + 2 * blr >= plr, DSEN2_E_BADARG,
-                "dsen2_prep16_from_images: image %dx%d smaller than one patch (%d)", H, W, patch);
+                "%s: image %dx%d smaller than one patch (%d)", name, H, W, patch);
   if (num_patches == 0) return 0;
   const Tiling tl = make_tiling(gh, gw, plr, blr);
-  DSEN2_REQUIRE(first_patch + num_patches <= (tl.k_i + 1) * (tl.k_j + 1), DSEN2_E_BADARG,
-                "dsen2_prep16_from_images: patch range [%d,%d) exceeds the %d allocated patches", first_patch,
+  DSEN2_REQUIRE(IDS || first_patch + num_patches <= (tl.k_i + 1) * (tl.k_j + 1), DSEN2_E_BADARG,
+                "%s: patch range [%d,%d) exceeds the %d allocated patches", name, first_patch,
                 first_patch + num_patches, (tl.k_i + 1) * (tl.k_j + 1));
   PrepSource s0{d_img10, H, W, r, 1};
   PrepSource s1{d_img20, H / 2, W / 2, r / 2, 2};
@@ -354,12 +352,28 @@ extern "C" int dsen2_prep16_from_images(const void* d_img10, const void* d_img20
   const long long total = (long long)num_patches * patch * patch;
   const int block = 256;
   if (img_dtype == DSEN2_IMG_U16)
-    prep16_from_images_kernel<uint16_t><<<grid_for(total, block), block, 0, (cudaStream_t)stream>>>(
-        s0, s1, s2, d_img60 ? 3 : 2, plr, blr, patch, tl, first_patch, total, divisor, (__half*)d_xin_hi, (__half*)d_xin_lo);
+    prep16_from_images_kernel<uint16_t, IDS><<<grid_for(total, block), block, 0, (cudaStream_t)stream>>>(
+        s0, s1, s2, d_img60 ? 3 : 2, plr, blr, patch, tl, first_patch, d_patch_ids, total, divisor, (__half*)d_xin_hi,
+        (__half*)d_xin_lo);
   else
-    prep16_from_images_kernel<float><<<grid_for(total, block), block, 0, (cudaStream_t)stream>>>(
-        s0, s1, s2, d_img60 ? 3 : 2, plr, blr, patch, tl, first_patch, total, divisor, (__half*)d_xin_hi, (__half*)d_xin_lo);
-  return check_launch("prep16_from_images");
+    prep16_from_images_kernel<float, IDS><<<grid_for(total, block), block, 0, (cudaStream_t)stream>>>(
+        s0, s1, s2, d_img60 ? 3 : 2, plr, blr, patch, tl, first_patch, d_patch_ids, total, divisor, (__half*)d_xin_hi,
+        (__half*)d_xin_lo);
+  return check_launch(name);
+}
+
+extern "C" int dsen2_prep16_from_images(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H,
+                                        int W, int patch, int border, int first_patch, int num_patches, float divisor,
+                                        void* d_xin_hi, void* d_xin_lo, void* stream) {
+  return prep16_from_images<false>("dsen2_prep16_from_images", d_img10, d_img20, d_img60, img_dtype, H, W, patch, border,
+                                   first_patch, nullptr, num_patches, divisor, d_xin_hi, d_xin_lo, stream);
+}
+
+extern "C" int dsen2_prep16_from_images_ids(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype,
+                                            int H, int W, int patch, int border, const int* d_patch_ids, int num_patches,
+                                            float divisor, void* d_xin_hi, void* d_xin_lo, void* stream) {
+  return prep16_from_images<true>("dsen2_prep16_from_images_ids", d_img10, d_img20, d_img60, img_dtype, H, W, patch, border,
+                                  0, d_patch_ids, num_patches, divisor, d_xin_hi, d_xin_lo, stream);
 }
 
 extern "C" int dsen2_pack_head16_weights(const float* d_hwio, int cin, int feature_size, void* d_packed, void* stream) {

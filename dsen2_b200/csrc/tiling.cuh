@@ -65,5 +65,17 @@ __device__ __forceinline__ int tile_of(int y, int size, int S, int n) {
   return (size % S != 0 && y >= size - S) ? n - 1 : y / S;
 }
 
+// [lo, hi) of the output coordinates along one axis whose last writer is tile t (the set where tile_of(y) == t): tile t
+// starts at min(t * S, size - S), and the next tile's start ends it
+__host__ __device__ inline void owned_span(int t, int size, int S, int n, int& lo, int& hi) {
+  lo = t * S < size - S ? t * S : size - S;
+  hi = t + 1 < n ? ((t + 1) * S < size - S ? (t + 1) * S : size - S) : size;
+}
+
+// image element -> float: exact for uint16 digital numbers (what GDAL hands s2_tiles_supres.py:311-315), so a
+// uint16 image and its float32 copy prepare bit-identical inputs
+__device__ __forceinline__ float ld_px(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_px(const uint16_t* p) { return (float)__ldg(p); }
+
 
 }  // namespace dsen2

@@ -14,6 +14,10 @@ part of this image, so the script is split here into
 
     python -m dsen2_b200.s2_tiles_supres <data_file> [output_file] [--roi_x_y x1,y1,x2,y2] [--run_60]
                                          [--copy_original_bands] [--output_file_format npz|GTiff|ENVI ...]
+                                         [--nodata VALUE]
+
+``--nodata`` is an extension of the reference's options: pixels whose every input band holds VALUE (0 outside the footprint
+of a partly covered granule) stay VALUE in the output, which records VALUE as its nodata value.
 """
 import argparse
 import os
@@ -131,19 +135,21 @@ def read_windows(xmin, ymin, xmax, ymax):
 # ---------------------------------------------------------------------------------------------- #
 # super-resolution chaining and output assembly (s2_tiles_supres.py:332-342, 385-416)
 # ---------------------------------------------------------------------------------------------- #
-def super_resolve(data10, data20, data60, names10, names20, names60, deep=False, models=None):
+def super_resolve(data10, data20, data60, names10, names20, names60, deep=False, models=None, nodata=None):
     """The 60 m bands first, then the 20 m bands; returns (sr (H, W, n20 [+ n60]) or None, short names of its bands).
-    ``models`` (extension): {'20': S2Model, '60': S2Model} instead of the shipped weight files."""
+    ``models`` (extension): {'20': S2Model, '60': S2Model} instead of the shipped weight files; ``nodata`` (extension):
+    the nodata value of both calls (``supres.DSen2_20``)."""
     from . import supres
     models = models or {}
+    extra = {} if nodata is None else {'nodata': nodata}
     sr60 = None
     if names60 and names20 and names10:
         print("Super-resolving the 60m data into 10m bands")
-        sr60 = supres.DSen2_60(data10, data20, data60, deep=deep, model=models.get('60'))
+        sr60 = supres.DSen2_60(data10, data20, data60, deep=deep, model=models.get('60'), **extra)
     sr20 = None
     if names10 and names20:
         print("Super-resolving the 20m data into 10m bands")
-        sr20 = supres.DSen2_20(data10, data20, deep=deep, model=models.get('20'))
+        sr20 = supres.DSen2_20(data10, data20, deep=deep, model=models.get('20'), **extra)
     if sr20 is None:
         return None, []
     if sr60 is not None:
@@ -171,9 +177,13 @@ def shift_geotransform(geotransform, xmin, ymin):
     return tuple(geot)
 
 
-def save_npz(output_file, bands):
-    """``np.savez(output_file, bands=bands)`` with bands = {description: array} (:419-420)."""
-    np.savez(output_file, bands=dict(bands))
+def save_npz(output_file, bands, nodata=None):
+    """``np.savez(output_file, bands=bands)`` with bands = {description: array} (:419-420); with ``nodata`` also a
+    ``nodata`` entry holding the value."""
+    if nodata is None:
+        np.savez(output_file, bands=dict(bands))
+    else:
+        np.savez(output_file, bands=dict(bands), nodata=np.float64(nodata))
 
 
 # ---------------------------------------------------------------------------------------------- #
@@ -296,6 +306,9 @@ def build_parser():
     p.add_argument("--output_file_format", default="GTiff", help="GDAL driver name, or npz.")
     p.add_argument("--copy_original_bands", action="store_true", help="Also copy the original 10m bands into the output.")
     p.add_argument("--save_prefix", default="", help="Prefix for all output files.")
+    p.add_argument("--nodata", type=float, default=None,
+                   help="Extension: input value of pixels without data (e.g. 0).  Pixels whose every band holds it stay "
+                        "nodata in the output, which records the value; empty patches are not computed.")
     return p
 
 
@@ -347,7 +360,7 @@ def main(argv=None, models=None):
     data10 = ds.read(0, w10, i10) if i10 else None
     data20 = ds.read(1, w20, i20) if i20 else None
     data60 = ds.read(2, w60, i60) if i60 else None
-    sr, sr_names = super_resolve(data10, data20, data60, n10, n20, n60, models=models)
+    sr, sr_names = super_resolve(data10, data20, data60, n10, n20, n60, models=models, nodata=args.nodata)
     if sr is None:
         print("No super-resolution performed, exiting")
         return 0
@@ -370,7 +383,7 @@ def main(argv=None, models=None):
                                                           output_file))
     geot = shift_geotransform(ds.geotransform, xmin, ymin)
     if fmt == "npz":
-        save_npz(output_file, bands)
+        save_npz(output_file, bands, args.nodata)
     else:  # pragma: no cover - needs osgeo
         from osgeo import gdal
         result = driver.Create(output_file, data10.shape[1], data10.shape[0], len(bands), gdal.GDT_Float64)
@@ -379,6 +392,8 @@ def main(argv=None, models=None):
         for bidx, (desc, data) in enumerate(bands):
             result.GetRasterBand(bidx + 1).SetDescription(desc)
             result.GetRasterBand(bidx + 1).WriteArray(data)
+            if args.nodata is not None:
+                result.GetRasterBand(bidx + 1).SetNoDataValue(args.nodata)
     for desc, _ in bands:
         print(desc)
     return 0

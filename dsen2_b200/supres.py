@@ -5,13 +5,18 @@ The whole tile stays on the GPU between the upload of the inputs and the downloa
 image.  Per patch batch: one input-preparation kernel (extract + bilinear + /2000 fused, straight from the images),
 then the 14 (DSen2, 6 x 128) or 66 (VDSen2, 32 x 256) tcgen05 convolutions, the last one writing the stitched
 x2000 canvas.
+
+Nodata (an extension): with ``nodata=v``, an output pixel whose every input band (10 m, 20 m[, 60 m]) equals v is nodata
+and comes out as v; only the patches that own a pixel with data run the network.  Every other pixel is bit-identical to
+the output without ``nodata``.
 """
+import math
 import os
 
 import numpy as np
 
 from . import _capi, sharding
-from .DSen2Net import s2model
+from .DSen2Net import S2Model, s2model
 from .patches import bilinear_up_device, extract_patches_device, patch_counts, recompose_device
 
 SCALE = 2000
@@ -54,26 +59,106 @@ def default_device_batch(W, P, B):
     return nx * max(1, target // nx)
 
 
-def super_resolve_device(model, d10, d20, d60=None, first_patch=0, num_patches=None, out=None, device_batch=None,
-                         timers=None):
-    """Device-level pipeline.  d10/d20(/d60): CUDA HWC tensors, all float32 or all uint16.  Processes patches
-    [first_patch, first_patch+num_patches) of the FILLED patch list (surplus zero patches of
-    patches.py:32-39 are never read by recompose_images, so they are skipped) and writes the pixels those
-    patches own into ``out`` (H, W, Cout) float32 (allocated zero-filled if None)."""
+def check_nodata(nodata, model, uint16_images):
+    """The ``nodata`` argument as the float the kernels compare with (None stays None).  Rejected, not clamped: NaN, a
+    value that is not an integer in [0, 65535] for uint16 images, a network without resBlocks (``model`` None: no
+    network involved)."""
+    if nodata is None:
+        return None
+    v = float(nodata)
+    if math.isnan(v):
+        raise ValueError("nodata must not be NaN")
+    if uint16_images and not (v.is_integer() and 0 <= v <= 65535):
+        raise ValueError("nodata %r is not a uint16 value (an integer in [0, 65535])" % (nodata,))
+    if model is not None and not model.xin16:
+        raise ValueError("nodata needs a network with resBlocks (num_layers > 0)")
+    return v
+
+
+def _nodata_args(d10, d20, d60, nodata):
     torch = _capi.require_cuda()
-    run_60 = d60 is not None
+    g = _GEOM[d60 is not None]
+    H, W = int(d10.shape[0]), int(d10.shape[1])
+    img_dtype = _capi.IMG_U16 if d10.dtype == torch.uint16 else _capi.IMG_F32
+    ptr = _capi.ptr
+    return (ptr(d10), ptr(d20), ptr(d60), img_dtype, H, W, g['patch'], g['border']), float(nodata)
+
+
+def _scan_active(d10, d20, d60, first_patch, num_patches, nodata, ids, count, count_host, timers=None):
+    """Enqueue ``dsen2_nodata_patches`` for the range on the current stream (active ids -> ``ids``, their number ->
+    ``count``) and the copy of the count into the pinned ``count_host``; returns the event that follows the copy."""
+    torch = _capi.require_cuda()
+    imgs, v = _nodata_args(d10, d20, d60, nodata)
+    S2Model._timed(timers, 'nodata_patches', num_patches, lambda: _capi.check(_capi.lib().dsen2_nodata_patches(
+        *imgs, first_patch, num_patches, v, _capi.ptr(ids), _capi.ptr(count), _capi.stream_ptr()), "dsen2_nodata_patches"))
+    count_host.copy_(count, non_blocking=True)
+    ev = torch.cuda.Event()
+    ev.record()
+    return ev
+
+
+def _run_active(model, d10, d20, d60, first_patch, num_patches, nodata, ids, out, device_batch, timers=None):
+    """The network over the active patches ``ids`` (batches of at most ``device_batch``), then nodata into the nodata
+    pixels the range owns -- after the last layer, which also stitches active patches' values over their nodata pixels."""
+    g = _GEOM[d60 is not None]
+    for i in range(0, int(ids.shape[0]), device_batch):
+        batch = ids[i:i + device_batch]
+        model.forward_images(d10, d20, d60, g['patch'], g['border'], 0, int(batch.shape[0]), out, float(SCALE),
+                             timers=timers, patch_ids=batch)
+    imgs, v = _nodata_args(d10, d20, d60, nodata)
+    S2Model._timed(timers, 'nodata_fill', num_patches, lambda: _capi.check(_capi.lib().dsen2_nodata_fill(
+        *imgs, first_patch, num_patches, v, model.out_channels, _capi.ptr(out), _capi.stream_ptr()), "dsen2_nodata_fill"))
+
+
+def _active(d10, d20, d60, first_patch, num_patches, nodata, timers=None):
+    """Active patch ids of the range: a CUDA int32 tensor, after one device -> host read of their number."""
+    torch = _capi.require_cuda()
+    ids = torch.empty((max(1, num_patches),), dtype=torch.int32, device=d10.device)
+    count = torch.empty((1,), dtype=torch.int32, device=d10.device)
+    count_host = torch.empty((1,), dtype=torch.int32).pin_memory()
+    _scan_active(d10, d20, d60, first_patch, num_patches, nodata, ids, count, count_host, timers).synchronize()
+    return ids[:int(count_host[0])]
+
+
+def _filled_range(d10, run_60, first_patch, num_patches):
     g = _GEOM[run_60]
     r, P, B = g['ratio'], g['patch'], g['border']
     H, W = int(d10.shape[0]), int(d10.shape[1])
     if H % r or W % r:
         raise ValueError("10 m image size %dx%d must be a multiple of %d" % (H, W, r))
-    plr, blr = P // r, B // r
-    _, filled = patch_counts(H // r, W // r, plr, blr)
+    _, filled = patch_counts(H // r, W // r, P // r, B // r)
     if num_patches is None:
         num_patches = filled - first_patch
     if first_patch < 0 or first_patch + num_patches > filled:
         raise ValueError("patch range [%d, %d) outside the %d patches of this tile"
                          % (first_patch, first_patch + num_patches, filled))
+    return num_patches
+
+
+def active_patches(d10, d20, d60=None, nodata=0, first_patch=0, num_patches=None):
+    """Ascending indices (CUDA int32 tensor) of the patches of [first_patch, first_patch+num_patches) that own a pixel
+    with data: the patches ``super_resolve_device(..., nodata=nodata)`` runs through the network."""
+    torch = _capi.require_cuda()
+    nodata = check_nodata(nodata, None, d10.dtype == torch.uint16)
+    num_patches = _filled_range(d10, d60 is not None, first_patch, num_patches)
+    return _active(d10, d20, d60, first_patch, num_patches, nodata)
+
+
+def super_resolve_device(model, d10, d20, d60=None, first_patch=0, num_patches=None, out=None, device_batch=None,
+                         timers=None, nodata=None):
+    """Device-level pipeline.  d10/d20(/d60): CUDA HWC tensors, all float32 or all uint16.  Processes patches
+    [first_patch, first_patch+num_patches) of the FILLED patch list (surplus zero patches of
+    patches.py:32-39 are never read by recompose_images, so they are skipped) and writes the pixels those
+    patches own into ``out`` (H, W, Cout) float32 (allocated zero-filled if None).  ``nodata``: see the module
+    docstring; the active patches are found on the device, and their number is the one value read back."""
+    torch = _capi.require_cuda()
+    nodata = check_nodata(nodata, model, d10.dtype == torch.uint16)
+    run_60 = d60 is not None
+    g = _GEOM[run_60]
+    r, P, B = g['ratio'], g['patch'], g['border']
+    H, W = int(d10.shape[0]), int(d10.shape[1])
+    plr, blr = P // r, B // r
+    num_patches = _filled_range(d10, run_60, first_patch, num_patches)
     if out is None:
         out = torch.zeros((H, W, model.out_channels), dtype=torch.float32, device=d10.device)
     if device_batch is None:
@@ -81,6 +166,10 @@ def super_resolve_device(model, d10, d20, d60=None, first_patch=0, num_patches=N
     # recompose_images' "lone patch is returned uncropped" branch (patches.py:375-376) keys on the ALLOCATED patch count
     # (k_i+1)(k_j+1), which is 1 only for images smaller than one stride -- inputs get_test_patches itself cannot tile
     # (and dsen2_prep16_from_images rejects); every image that reaches this point is stitched and cropped.
+    if nodata is not None:
+        ids = _active(d10, d20, d60, first_patch, num_patches, nodata, timers)
+        _run_active(model, d10, d20, d60, first_patch, num_patches, nodata, ids, out, device_batch, timers)
+        return out
     for p0 in range(first_patch, first_patch + num_patches, device_batch):
         nb = min(device_batch, first_patch + num_patches - p0)
         if model.xin16:                          # fused: images -> x_in16 -> network -> stitched canvas
@@ -160,9 +249,34 @@ class HostPipeline:
             self.h2d_bytes += (b - a) * d.shape[1] * d.shape[2] * d.element_size()
         return b if done is None else max(done, b)
 
-    def run(self, h10, h20, h60=None, hout=None, first_patch=0, num_patches=None, timers=None):
+    def _nodata_buffers(self, nodata, first_patch, num_patches, chunks):
+        """Device id list of the range, device and pinned per-chunk counts: chunk k scans into its own slice / entry, so
+        the upload stream never overwrites what an earlier chunk's network still reads."""
+        torch = self.torch
+        nodata = check_nodata(nodata, self.model, self.dtype == torch.uint16)
+        if nodata is None:
+            return None, None, None, None
+        ids = torch.empty((max(1, num_patches),), dtype=torch.int32, device=self.dev)
+        count = torch.empty((chunks,), dtype=torch.int32, device=self.dev)
+        return nodata, ids, count, torch.empty((chunks,), dtype=torch.int32).pin_memory()
+
+    def _compute(self, k, p0, cnt, first_patch, nodata, ids, count_host, ev_scan, timers):
+        """Chunk k's network on the current stream (its inputs are resident): the whole range, or -- with ``nodata`` --
+        the active patches its scan found, then the nodata fill."""
+        if nodata is None:
+            super_resolve_device(self.model, self.d10, self.d20, self.d60, first_patch=p0, num_patches=cnt,
+                                 out=self.canvas, device_batch=self.device_batch, timers=timers)
+            return
+        ev_scan.synchronize()                        # this chunk's upload and scan only, never an earlier network
+        batch = self.device_batch or default_device_batch(self.W, self.P, self.B)
+        a = p0 - first_patch
+        _run_active(self.model, self.d10, self.d20, self.d60, p0, cnt, nodata, ids[a:a + int(count_host[k])], self.canvas,
+                    batch, timers)
+
+    def run(self, h10, h20, h60=None, hout=None, first_patch=0, num_patches=None, timers=None, nodata=None):
         """Pinned torch tensors in (dtype = the pipeline's), pinned float32 (H, W, Cout) tensor out.  Rows of ``hout`` that
-        the patch range owns only partly (the seam rows of a sharded range) are downloaded whole."""
+        the patch range owns only partly (the seam rows of a sharded range) are downloaded whole.  ``nodata``: see the
+        module docstring; each chunk's patch scan runs on the upload stream right behind its upload."""
         torch = self.torch
         filled = self.ny * self.nx
         if num_patches is None:
@@ -172,22 +286,28 @@ class HostPipeline:
         for h in (h10, h20) + ((h60,) if self.run_60 else ()):
             if h.dtype != self.dtype:
                 raise ValueError("host image dtype %s does not match the pipeline's %s" % (h.dtype, self.dtype))
+        plan = self._plan(first_patch, num_patches)
+        nodata, ids, count, count_host = self._nodata_buffers(nodata, first_patch, num_patches, len(plan))
         self.h2d_bytes = self.d2h_bytes = 0
         main = torch.cuda.current_stream(self.dev)
         self.up.wait_stream(main)
         self.down.wait_stream(main)
         done10 = done20 = done60 = None           # rows already resident on the device (per resolution)
-        for p0, cnt, (r0, r1), rects in self._plan(first_patch, num_patches):
+        for k, (p0, cnt, (r0, r1), rects) in enumerate(plan):
+            ev_scan = None
             with torch.cuda.stream(self.up):
                 done10 = self._upload(h10, self.d10, 1, r0, r1, done10)
                 done20 = self._upload(h20, self.d20, 2, r0, r1, done20)
                 if self.run_60:
                     done60 = self._upload(h60, self.d60, 6, r0, r1, done60)
+                if nodata is not None:
+                    a = p0 - first_patch
+                    ev_scan = _scan_active(self.d10, self.d20, self.d60, p0, cnt, nodata, ids[a:a + cnt],
+                                           count[k:k + 1], count_host[k:k + 1], timers)
                 ev_up = torch.cuda.Event()
                 ev_up.record(self.up)
             main.wait_event(ev_up)
-            super_resolve_device(self.model, self.d10, self.d20, self.d60, first_patch=p0, num_patches=cnt,
-                                 out=self.canvas, device_batch=self.device_batch, timers=timers)
+            self._compute(k, p0, cnt, first_patch, nodata, ids, count_host, ev_scan, timers)
             ev_c = torch.cuda.Event()
             ev_c.record(main)
             self.down.wait_event(ev_c)
@@ -229,9 +349,9 @@ class HostPipeline:
                                             initializer=torch.cuda.set_device, initargs=(self.dev,))
         return self._slots
 
-    def run_numpy(self, a10, a20, a60=None, out=None, first_patch=0, num_patches=None, timers=None):
+    def run_numpy(self, a10, a20, a60=None, out=None, first_patch=0, num_patches=None, timers=None, nodata=None):
         """Pageable numpy arrays in -> numpy (H, W, Cout) float32 out (allocated if None).  Arrays whose dtype is not
-        the pipeline's are cast while they are staged."""
+        the pipeline's are cast while they are staged.  ``nodata`` as in ``run``."""
         torch = self.torch
         filled = self.ny * self.nx
         if num_patches is None:
@@ -243,6 +363,7 @@ class HostPipeline:
         divs = (1, 2, 6) if self.run_60 else (1, 2)
         devs = [self.d10, self.d20] + ([self.d60] if self.run_60 else [])
         plan = self._plan(first_patch, num_patches)
+        nodata, ids, count, count_host = self._nodata_buffers(nodata, first_patch, num_patches, len(plan))
         slots = self._ring(plan)
         # rows of every resolution a chunk has to bring (those beyond what earlier chunks brought)
         need, done = [], [None] * len(divs)
@@ -288,11 +409,15 @@ class HostPipeline:
                         self.h2d_bytes += (b - a) * devs[i].shape[1] * devs[i].shape[2] * devs[i].element_size()
                 slot.ev_h2d.record(self.up)
                 slot.used_in = True
+                ev_scan = None
+                if nodata is not None:
+                    a = p0 - first_patch
+                    ev_scan = _scan_active(self.d10, self.d20, self.d60, p0, cnt, nodata, ids[a:a + cnt],
+                                           count[k:k + 1], count_host[k:k + 1], timers)
             main.wait_event(slot.ev_h2d)
             if k + self.RING < len(plan):
                 fin[k + self.RING] = self._pool.submit(stage_in, k + self.RING)
-            super_resolve_device(self.model, self.d10, self.d20, self.d60, first_patch=p0, num_patches=cnt,
-                                 out=self.canvas, device_batch=self.device_batch, timers=timers)
+            self._compute(k, p0, cnt, first_patch, nodata, ids, count_host, ev_scan, timers)
             ev_c = torch.cuda.Event()
             ev_c.record(main)
             self.down.wait_event(ev_c)
@@ -338,7 +463,9 @@ def _pipeline_for(model, H, W, run_60, dtype):
     return pipe
 
 
-def _run(model, arrays, out=None):
+def _run(model, arrays, out=None, nodata=None):
+    if nodata is not None:                   # rejected before the device is touched
+        nodata = check_nodata(nodata, model, model.xin16 and all(np.asarray(a).dtype == np.uint16 for a in arrays))
     torch = _capi.require_cuda()
     arrays = [np.asarray(a) for a in arrays]
     H, W = int(arrays[0].shape[0]), int(arrays[0].shape[1])
@@ -350,23 +477,24 @@ def _run(model, arrays, out=None):
     # else is staged as float32 (the reference divides by SCALE in floating point whatever the input type, supres.py:23-24)
     dtype = torch.uint16 if (model.xin16 and all(a.dtype == np.uint16 for a in arrays)) else torch.float32
     pipe = _pipeline_for(model, H, W, len(arrays) == 3, dtype)
-    res = pipe.run_numpy(*arrays, out=out)
+    res = pipe.run_numpy(*arrays, out=out, nodata=nodata)
     torch.cuda.current_stream().synchronize()
     return res
 
 
-def DSen2_20(d10, d20, deep=False, model=None, out=None):
+def DSen2_20(d10, d20, deep=False, model=None, out=None, nodata=None):
     """supres.py:15-30.  d10 (H,W,4), d20 (H/2,W/2,6) -> (H,W,6) float32.  Extensions: ``model`` supplies a preloaded
-    ``S2Model`` instead of the shipped hdf5 weights, ``out`` a preallocated (H,W,6) float32 array to fill."""
+    ``S2Model`` instead of the shipped hdf5 weights, ``out`` a preallocated (H,W,6) float32 array to fill, ``nodata`` the
+    input value of pixels without data (module docstring): they come out as ``nodata`` and empty patches are skipped."""
     input_shape = ((4, None, None), (6, None, None))
     if model is None:
         model = _load_model(input_shape, deep, run_60=False)
-    return _run(model, [d10, d20], out)
+    return _run(model, [d10, d20], out, nodata)
 
 
-def DSen2_60(d10, d20, d60, deep=False, model=None, out=None):
+def DSen2_60(d10, d20, d60, deep=False, model=None, out=None, nodata=None):
     """supres.py:33-50.  + d60 (H/6,W/6,2) -> (H,W,2) float32."""
     input_shape = ((4, None, None), (6, None, None), (2, None, None))
     if model is None:
         model = _load_model(input_shape, deep, run_60=True)
-    return _run(model, [d10, d20, d60], out)
+    return _run(model, [d10, d20, d60], out, nodata)

@@ -217,6 +217,37 @@ int dsen2_conv_tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void*
                              int n, int P, int first_patch, int border, int img_h, int img_w, float mul,
                              float* d_canvas, void* stream);
 
+/* The same two steps for an arbitrary list of patches (the active patches of dsen2_nodata_patches): the arguments of
+ * dsen2_prep16_from_images / dsen2_conv_tail16_stitch, with batch entry b = patch d_patch_ids[b] (absolute indices in the
+ * filled patch list, device int32 array of n = num_patches entries) instead of first_patch + b.  An id outside the tiling
+ * prepares a zero input and writes nothing.                                                                          */
+int dsen2_prep16_from_images_ids(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H, int W,
+                                 int patch, int border, const int* d_patch_ids, int num_patches, float divisor,
+                                 void* d_xin_hi, void* d_xin_lo, void* stream);
+int dsen2_conv_tail16_stitch_ids(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                 const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
+                                 int n, int P, const int* d_patch_ids, int border, int img_h, int img_w, float mul,
+                                 float* d_canvas, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Nodata (csrc/nodata.cu; an extension: the reference super-resolves nodata like data).  Images, img_dtype, H, W, patch
+ * and border as dsen2_prep16_from_images (d_img60 == NULL: 20 m path); `nodata` is the fill value v (not NaN).  Output pixel
+ * (y, x) is NODATA iff every band of img10[y, x], img20[y/2, x/2] and (60 m) img60[y/6, x/6] equals v in the images'
+ * element type; any other pixel is valid.
+ *   dsen2_nodata_patches: of the filled patches [first_patch, first_patch + num_patches), the ACTIVE ones -- those that
+ *       own (last writer wins, as dsen2_conv_tail16_stitch) at least one valid pixel -- as ascending absolute ids in
+ *       d_ids[0, *d_count).  d_ids holds num_patches ints (it is also the scan's scratch); d_count one int.
+ *   dsen2_nodata_fill: writes v into all cout bands of every nodata pixel of the (H, W, cout) float32 canvas that the
+ *       range owns.  Run it after the last layer: an active patch also stitches network values over its nodata pixels.
+ * Running only the active patches (dsen2_*_ids) and then the fill leaves every valid pixel bit-identical to the whole
+ * range run without nodata.                                                                                          */
+int dsen2_nodata_patches(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H, int W,
+                         int patch, int border, int first_patch, int num_patches, float nodata, int* d_ids, int* d_count,
+                         void* stream);
+int dsen2_nodata_fill(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H, int W,
+                      int patch, int border, int first_patch, int num_patches, float nodata, int cout, float* d_canvas,
+                      void* stream);
+
 /* Whole s2model forward (model.predict on one batch, supres.py:65) for n patches of (P, P).
  * d_weights[i] / d_bias[i] are the packed layers in Keras topological order (2*num_layers+2 entries):
  *   [0] dsen2_pack_head16_weights (dsen2_pack_head_weights when num_layers == 0, feature_size 128 only),

@@ -369,12 +369,16 @@ class S2Model:
                         "dsen2_s2model_forward")
         return out
 
-    def forward_images(self, d10, d20, d60, patch, border, first_patch, n, canvas, mul, timers=None, patch_ids=None):
+    def forward_images(self, d10, d20, d60, patch, border, first_patch, n, canvas, mul, timers=None, patch_ids=None,
+                       avoid=None):
         """Fused tile pipeline of the fast path: patches [first_patch, first_patch+n) are gathered straight
         from the HWC images (extract + bilinear + /mul), run through the network, and the pixels they own
         are written x mul into ``canvas`` (H, W, Cout).  No patch stack or prediction stack exists.  The images are
         float32 or uint16 (digital numbers) HWC CUDA tensors.  ``patch_ids``: a CUDA int32 tensor of n patch indices to
-        run instead of the range (``first_patch`` is then ignored)."""
+        run instead of the range (``first_patch`` is then ignored).  ``canvas`` is a contiguous float32 or uint16 tensor;
+        a uint16 canvas receives the float values rounded half to even and clipped to [0, 65535] (NaN: 0), and a value
+        equal to ``avoid`` (an int in [0, 65535], the nodata value) is written one step away from it
+        (``dsen2_conv_tail16_stitch_u16`` in include/dsen2_b200.h)."""
         torch = _capi.require_cuda()
         if not self.xin16:
             raise _capi.DSen2Error("forward_images needs a network with resblocks (num_layers > 0)")
@@ -386,6 +390,16 @@ class S2Model:
         if patch_ids is not None and not (patch_ids.is_cuda and patch_ids.dtype == torch.int32 and patch_ids.is_contiguous()
                                           and tuple(patch_ids.shape) == (n,)):
             raise ValueError("patch_ids must be a contiguous CUDA int32 tensor of %d ids" % n)
+        if not (canvas.is_cuda and canvas.dtype in (torch.float32, torch.uint16) and canvas.is_contiguous()
+                and tuple(canvas.shape) == (H, W, self.out_channels)):
+            raise ValueError("canvas must be a contiguous CUDA float32 or uint16 tensor of shape %s"
+                             % ((H, W, self.out_channels),))
+        u16 = canvas.dtype == torch.uint16
+        if avoid is not None and not u16:
+            raise ValueError("avoid applies to a uint16 canvas only")
+        avoid = -1 if avoid is None else int(avoid)
+        if not -1 <= avoid <= 65535:
+            raise ValueError("avoid %d is not a uint16 value" % avoid)
         img_dtype = _capi.IMG_U16 if d10.dtype == torch.uint16 else _capi.IMG_F32
         wts, biases, _wp, _bp = self._ensure_packed(dev)
         if n == 0:
@@ -403,14 +417,14 @@ class S2Model:
                     ptr(d10), ptr(d20), ptr(d60), img_dtype, H, W, patch, border, ptr(patch_ids), n, float(mul),
                     ptr(buf['xin_hi']), ptr(buf['xin_lo']), st), "dsen2_prep16_from_images_ids"))
             self._trunk(buf, wts, biases, n, patch, st, timers)
-            if patch_ids is None:
-                self._timed(timers, 'conv_tail', n, lambda: _capi.check(lib.dsen2_conv_tail16_stitch(
-                    *self._tail_args(buf, wts, biases), self.feature_size, n, patch, first_patch, border, H, W, float(mul),
-                    ptr(canvas), st), "dsen2_conv_tail16_stitch"))
-            else:
-                self._timed(timers, 'conv_tail', n, lambda: _capi.check(lib.dsen2_conv_tail16_stitch_ids(
-                    *self._tail_args(buf, wts, biases), self.feature_size, n, patch, ptr(patch_ids), border, H, W,
-                    float(mul), ptr(canvas), st), "dsen2_conv_tail16_stitch_ids"))
+            # the canvas type picks the entry point; the uint16 ones take the value to avoid after the scale
+            which = (ptr(patch_ids),) if patch_ids is not None else (first_patch,)
+            name = 'dsen2_conv_tail16_stitch' + ('_ids' if patch_ids is not None else '') + ('_u16' if u16 else '')
+            tail = getattr(lib, name)
+            extra = (float(mul), avoid) if u16 else (float(mul),)
+            self._timed(timers, 'conv_tail', n, lambda: _capi.check(tail(
+                *self._tail_args(buf, wts, biases), self.feature_size, n, patch, *which, border, H, W, *extra,
+                ptr(canvas), st), name))
         return canvas
 
     def launches_per_forward(self):

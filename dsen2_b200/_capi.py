@@ -58,6 +58,13 @@ SIGNATURES = {
                                      c_void_p, c_void_p, c_void_p]),
     "dsen2_nodata_fill": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float,
                                   c_int, c_void_p, c_void_p]),
+    "dsen2_conv_tail16_stitch_u16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                             c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_int, c_void_p, c_void_p]),
+    "dsen2_conv_tail16_stitch_ids_u16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                                 c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_float, c_int, c_void_p,
+                                                 c_void_p]),
+    "dsen2_nodata_fill_u16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                      c_float, c_int, c_void_p, c_void_p]),
     "dsen2_conv_resq256": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p,
                                    c_void_p, c_void_p]),
     "dsen2_conv_tail": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,

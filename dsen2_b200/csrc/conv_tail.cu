@@ -48,11 +48,24 @@ struct TailParams {
   const __half* skip_lo;
   int skip_ch0, cout;
   float out_mul;
-  float* out;
+  void* out;                          // float, or (stitched canvas only) uint16_t: the OutT of the kernel instance
   int tail_mode;                      // 0: NCHW (n, cout, H, W) predictions; 1: stitched HWC canvas
   int first_patch, img_h, img_w, border, grid_ny, grid_nx;
   const int* patch_ids;               // stitching form with IDS: batch entry b is patch patch_ids[b], not first_patch + b
+  int avoid;                          // uint16 canvas: a value the network must not write (the nodata value), -1 none
 };
+
+// The uint16 (digital number) canvas value of the float f the float canvas receives: NaN -> 0, else rint(clip(f, 0, 65535))
+// (round half to even; fmaxf returns 0 for a NaN f).  A value equal to `avoid` (>= 0) moves one step away from it, so a
+// dark or negative network output never reads as nodata.
+__device__ __forceinline__ uint16_t dn_of(float f, int avoid) {
+  int q = (int)__float2uint_rn(fminf(fmaxf(f, 0.f), 65535.f));
+  if (q == avoid) q = avoid == 65535 ? 65534 : q + 1;
+  return (uint16_t)q;
+}
+
+__device__ __forceinline__ void store_out(float* o, float f, int) { *o = f; }
+__device__ __forceinline__ void store_out(uint16_t* o, float f, int avoid) { *o = dn_of(f, avoid); }
 
 template <int KPM>                     // 64-channel k-blocks per activation tensor: 2 (128 features) or 4 (256)
 struct TailCfg {
@@ -67,7 +80,7 @@ __device__ __forceinline__ int tail_stitch_tile_of(int y, int size, int S, int n
   return (size % S != 0 && y >= size - S) ? n - 1 : y / S;
 }
 
-template <int KPM, bool IDS>
+template <int KPM, bool IDS, typename OutT>
 __global__ void __launch_bounds__(kTThreads, 1)
 conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
                          const __grid_constant__ CUtensorMap tm_w, const TailParams p) {
@@ -250,7 +263,8 @@ conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid
             }
             const float v = (vh + vl) + s_bias[c_lo + i];
             const float skip = __half2float(ch[i]) + __half2float(cl[i]);
-            p.out[obase + (c_lo + i) * ostride] = (v + skip) * p.out_mul;      // Add (DSen2Net.py:38), then x SCALE
+            store_out(static_cast<OutT*>(p.out) + obase + (c_lo + i) * ostride, (v + skip) * p.out_mul,   // Add
+                      p.avoid);                                                                       // (DSen2Net.py:38), x SCALE
           }
         }
       }
@@ -285,12 +299,12 @@ __global__ void pack_tail16_weights_kernel(const float* __restrict__ hwio, int F
   }
 }
 
-template <int KPM, bool IDS>
+template <int KPM, bool IDS, typename OutT>
 static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_lo, const void* d_w, int sms, cudaStream_t stream) {
   using Cfg = TailCfg<KPM>;
   static bool configured[64] = {};
   if (needs_config(configured)) {
-    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM, IDS>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM, IDS, OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   }
   const int F = KPM * 64;
   CUtensorMap hi, lo, w;
@@ -303,12 +317,13 @@ static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_
   const uint32_t wb[2] = {64, 128};
   if ((rc = make_tmap_f16_sw(&w, d_w, 2, wd, wb, 128)) != 0) return rc;
   const int grid = (int)(p.num_tiles < (uint32_t)sms ? p.num_tiles : (uint32_t)sms);
-  conv_tail_swapped_kernel<KPM, IDS><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
+  conv_tail_swapped_kernel<KPM, IDS, OutT><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
   return check_launch("conv_tail_swapped");
 }
 
+template <typename OutT>
 static int tail16_common(TailParams& p, int features, const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
-                         const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int n, int H, int W, float* d_out,
+                         const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int n, int H, int W, OutT* d_out,
                          void* stream) {
   DSEN2_REQUIRE(d_x_hi && d_x_lo && d_w && d_bias && d_xin_hi && d_xin_lo && d_out, DSEN2_E_BADARG, "dsen2_conv_tail16: null pointer");
   DSEN2_REQUIRE(features == 128 || features == 256, DSEN2_E_BADARG, "dsen2_conv_tail16: feature_size must be 128 or 256 (got %d)",
@@ -339,8 +354,10 @@ static int tail16_common(TailParams& p, int features, const void* d_x_hi, const 
   p.cout = cout; p.out = d_out;
   const cudaStream_t st = (cudaStream_t)stream;
   if (p.patch_ids)
-    return features == 256 ? launch_tail<4, true>(p, d_x_hi, d_x_lo, d_w, sms, st) : launch_tail<2, true>(p, d_x_hi, d_x_lo, d_w, sms, st);
-  return features == 256 ? launch_tail<4, false>(p, d_x_hi, d_x_lo, d_w, sms, st) : launch_tail<2, false>(p, d_x_hi, d_x_lo, d_w, sms, st);
+    return features == 256 ? launch_tail<4, true, OutT>(p, d_x_hi, d_x_lo, d_w, sms, st)
+                           : launch_tail<2, true, OutT>(p, d_x_hi, d_x_lo, d_w, sms, st);
+  return features == 256 ? launch_tail<4, false, OutT>(p, d_x_hi, d_x_lo, d_w, sms, st)
+                         : launch_tail<2, false, OutT>(p, d_x_hi, d_x_lo, d_w, sms, st);
 }
 
 }  // namespace dsen2
@@ -364,36 +381,41 @@ extern "C" int dsen2_conv_tail16(const void* d_x_hi, const void* d_x_lo, const v
   TailParams p{};
   p.tail_mode = 0;
   p.out_mul = 1.0f;
-  return tail16_common(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, H, W, d_pred_nchw,
+  p.avoid = -1;
+  return tail16_common<float>(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, H, W, d_pred_nchw,
                        stream);
 }
 
-// the stitching form: patches first_patch + b, or d_patch_ids[b] when d_patch_ids is not null
+// the stitching form: patches first_patch + b, or d_patch_ids[b] when d_patch_ids is not null; float or uint16 canvas
+template <typename OutT>
 static int tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias, const void* d_xin_hi,
                          const void* d_xin_lo, int skip_ch0, int cout, int feature_size, int n, int P, int first_patch,
-                         const int* d_patch_ids, int border, int img_h, int img_w, float mul, float* d_canvas, void* stream) {
+                         const int* d_patch_ids, int border, int img_h, int img_w, float mul, int avoid, OutT* d_canvas,
+                         void* stream) {
   const int S = P - 2 * border;
   DSEN2_REQUIRE(P > 0 && border >= 0 && S > 0 && img_h >= S && img_w >= S && first_patch >= 0, DSEN2_E_BADARG,
                 "dsen2_conv_tail16_stitch: bad stitch geometry (P %d border %d image %dx%d)", P, border, img_h, img_w);
+  DSEN2_REQUIRE(avoid >= -1 && avoid <= 65535, DSEN2_E_BADARG, "dsen2_conv_tail16_stitch: avoid %d outside [-1, 65535]", avoid);
   TailParams p{};
   p.tail_mode = 1;
   p.out_mul = mul;
+  p.avoid = avoid;
   p.first_patch = first_patch; p.img_h = img_h; p.img_w = img_w; p.border = border;
   p.grid_ny = ceil_div(img_h, S); p.grid_nx = ceil_div(img_w, S);
   p.patch_ids = d_patch_ids;
   DSEN2_REQUIRE(d_patch_ids || first_patch + n <= p.grid_ny * p.grid_nx, DSEN2_E_BADARG,
                 "dsen2_conv_tail16_stitch: patch range [%d,%d) exceeds the %d tiles of the canvas", first_patch,
                 first_patch + n, p.grid_ny * p.grid_nx);
-  return tail16_common(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, P, P, d_canvas,
-                       stream);
+  return tail16_common<OutT>(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, P, P,
+                             d_canvas, stream);
 }
 
 extern "C" int dsen2_conv_tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
                                         const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
                                         int n, int P, int first_patch, int border, int img_h, int img_w, float mul,
                                         float* d_canvas, void* stream) {
-  return tail16_stitch(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P, first_patch,
-                       nullptr, border, img_h, img_w, mul, d_canvas, stream);
+  return tail16_stitch<float>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P,
+                              first_patch, nullptr, border, img_h, img_w, mul, -1, d_canvas, stream);
 }
 
 extern "C" int dsen2_conv_tail16_stitch_ids(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
@@ -401,6 +423,24 @@ extern "C" int dsen2_conv_tail16_stitch_ids(const void* d_x_hi, const void* d_x_
                                             int feature_size, int n, int P, const int* d_patch_ids, int border, int img_h,
                                             int img_w, float mul, float* d_canvas, void* stream) {
   DSEN2_REQUIRE(d_patch_ids, DSEN2_E_BADARG, "dsen2_conv_tail16_stitch_ids: null pointer");
-  return tail16_stitch(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P, 0, d_patch_ids,
-                       border, img_h, img_w, mul, d_canvas, stream);
+  return tail16_stitch<float>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P, 0,
+                              d_patch_ids, border, img_h, img_w, mul, -1, d_canvas, stream);
+}
+
+extern "C" int dsen2_conv_tail16_stitch_u16(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                            const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout,
+                                            int feature_size, int n, int P, int first_patch, int border, int img_h,
+                                            int img_w, float mul, int avoid, uint16_t* d_canvas, void* stream) {
+  return tail16_stitch<uint16_t>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P,
+                                 first_patch, nullptr, border, img_h, img_w, mul, avoid, d_canvas, stream);
+}
+
+extern "C" int dsen2_conv_tail16_stitch_ids_u16(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                                const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout,
+                                                int feature_size, int n, int P, const int* d_patch_ids, int border,
+                                                int img_h, int img_w, float mul, int avoid, uint16_t* d_canvas,
+                                                void* stream) {
+  DSEN2_REQUIRE(d_patch_ids, DSEN2_E_BADARG, "dsen2_conv_tail16_stitch_ids_u16: null pointer");
+  return tail16_stitch<uint16_t>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P, 0,
+                                 d_patch_ids, border, img_h, img_w, mul, avoid, d_canvas, stream);
 }

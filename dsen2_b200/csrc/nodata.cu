@@ -6,7 +6,8 @@
 //   dsen2_nodata_patches: the ACTIVE patches of a range -- those that own (last writer wins, patches.py:394-403) at least one
 //                         valid pixel -- as an ascending id list.  One block per patch reads the patch's owned rectangle
 //                         and stops at the first valid pixel; a single-block scan then compacts the flags in place.
-//   dsen2_nodata_fill:    v into every nodata pixel the range owns, after the last layer has stitched the active patches.
+//   dsen2_nodata_fill:    v into every nodata pixel the range owns, after the last layer has stitched the active patches
+//                         (dsen2_nodata_fill_u16: the same into a uint16 canvas).
 // Together they read the inputs about once (1.3 GB of uint16 for a full 10980^2 tile, all of it only where it is empty).
 #include "common.cuh"
 #include "tiling.cuh"
@@ -92,18 +93,19 @@ __global__ void __launch_bounds__(1024) nodata_compact_kernel(int* __restrict__ 
   if (threadIdx.x == 0) *count = base;
 }
 
-// v into the nodata pixels of rows [y0, y0 + total / W) whose owner lies in [first_patch, end_patch)
-template <typename T>
+// v into the nodata pixels of rows [y0, y0 + total / W) whose owner lies in [first_patch, end_patch); OutT: the canvas
+// element type, float or uint16_t (v is then an integer in [0, 65535])
+template <typename T, typename OutT>
 __global__ void nodata_fill_kernel(NodataImages m, int S, int ny, int nx, int first_patch, int end_patch, int y0,
-                                   long long total, int cout, float* __restrict__ canvas) {
+                                   long long total, int cout, OutT* __restrict__ canvas) {
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
     const int dy = (int)(idx / m.W);
     const int y = y0 + dy, x = (int)(idx - (long long)dy * m.W);
     const int owner = tile_of(y, m.H, S, ny) * nx + tile_of(x, m.W, S, nx);
     if (owner >= first_patch && owner < end_patch && is_nodata<T>(m, y, x)) {
-      float* o = canvas + ((long long)y * m.W + x) * cout;
-      for (int c = 0; c < cout; ++c) o[c] = m.v;
+      OutT* o = canvas + ((long long)y * m.W + x) * cout;
+      for (int c = 0; c < cout; ++c) o[c] = (OutT)m.v;
     }
   }
 }
@@ -159,15 +161,16 @@ extern "C" int dsen2_nodata_patches(const void* d_img10, const void* d_img20, co
   return check_launch("nodata_compact");
 }
 
-extern "C" int dsen2_nodata_fill(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H, int W,
-                                 int patch, int border, int first_patch, int num_patches, float nodata, int cout,
-                                 float* d_canvas, void* stream) {
+template <typename OutT>
+static int nodata_fill(const char* name, const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H,
+                       int W, int patch, int border, int first_patch, int num_patches, float nodata, int cout,
+                       OutT* d_canvas, void* stream) {
   Tiling tl;
   int S = 0;
-  int rc = nodata_args("dsen2_nodata_fill", d_img10, d_img20, d_img60, img_dtype, H, W, patch, border, first_patch,
-                       num_patches, nodata, tl, S);
+  int rc = nodata_args(name, d_img10, d_img20, d_img60, img_dtype, H, W, patch, border, first_patch, num_patches, nodata,
+                       tl, S);
   if (rc) return rc;
-  DSEN2_REQUIRE(d_canvas && cout > 0, DSEN2_E_BADARG, "dsen2_nodata_fill: null canvas or cout %d", cout);
+  DSEN2_REQUIRE(d_canvas && cout > 0, DSEN2_E_BADARG, "%s: null canvas or cout %d", name, cout);
   if (num_patches == 0) return 0;
   // rows owned by the range: from the first patch's patch row to the last one's
   int y0, y1, unused;
@@ -178,10 +181,28 @@ extern "C" int dsen2_nodata_fill(const void* d_img10, const void* d_img20, const
   const int block = 256;
   const cudaStream_t st = (cudaStream_t)stream;
   if (img_dtype == DSEN2_IMG_U16)
-    nodata_fill_kernel<uint16_t><<<grid_for(total, block), block, 0, st>>>(m, S, tl.n_i, tl.n_j, first_patch,
-                                                                          first_patch + num_patches, y0, total, cout, d_canvas);
+    nodata_fill_kernel<uint16_t, OutT><<<grid_for(total, block), block, 0, st>>>(m, S, tl.n_i, tl.n_j, first_patch,
+                                                                                first_patch + num_patches, y0, total, cout,
+                                                                                d_canvas);
   else
-    nodata_fill_kernel<float><<<grid_for(total, block), block, 0, st>>>(m, S, tl.n_i, tl.n_j, first_patch,
-                                                                       first_patch + num_patches, y0, total, cout, d_canvas);
+    nodata_fill_kernel<float, OutT><<<grid_for(total, block), block, 0, st>>>(m, S, tl.n_i, tl.n_j, first_patch,
+                                                                             first_patch + num_patches, y0, total, cout,
+                                                                             d_canvas);
   return check_launch("nodata_fill");
+}
+
+extern "C" int dsen2_nodata_fill(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H, int W,
+                                 int patch, int border, int first_patch, int num_patches, float nodata, int cout,
+                                 float* d_canvas, void* stream) {
+  return nodata_fill<float>("dsen2_nodata_fill", d_img10, d_img20, d_img60, img_dtype, H, W, patch, border, first_patch,
+                            num_patches, nodata, cout, d_canvas, stream);
+}
+
+extern "C" int dsen2_nodata_fill_u16(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H,
+                                     int W, int patch, int border, int first_patch, int num_patches, float nodata, int cout,
+                                     uint16_t* d_canvas, void* stream) {
+  DSEN2_REQUIRE(nodata >= 0.f && nodata <= 65535.f && nodata == (float)(int)nodata, DSEN2_E_BADARG,
+                "dsen2_nodata_fill_u16: nodata %g is not a uint16 value", (double)nodata);
+  return nodata_fill<uint16_t>("dsen2_nodata_fill_u16", d_img10, d_img20, d_img60, img_dtype, H, W, patch, border,
+                               first_patch, num_patches, nodata, cout, d_canvas, stream);
 }

@@ -14,10 +14,13 @@ part of this image, so the script is split here into
 
     python -m dsen2_b200.s2_tiles_supres <data_file> [output_file] [--roi_x_y x1,y1,x2,y2] [--run_60]
                                          [--copy_original_bands] [--output_file_format npz|GTiff|ENVI ...]
-                                         [--nodata VALUE]
+                                         [--nodata VALUE] [--output_dtype float64|uint16]
 
 ``--nodata`` is an extension of the reference's options: pixels whose every input band holds VALUE (0 outside the footprint
-of a partly covered granule) stay VALUE in the output, which records VALUE as its nodata value.
+of a partly covered granule) stay VALUE in the output, which records VALUE as its nodata value.  ``--output_dtype uint16``
+(another extension) writes the super-resolved bands as uint16 digital numbers, the input's own format, rounded and saturated
+on the GPU (``supres.DSen2_20(out_dtype=)``); VALUE must then be a uint16 value.  The default ``float64`` is the reference's
+output.
 """
 import argparse
 import os
@@ -135,13 +138,17 @@ def read_windows(xmin, ymin, xmax, ymax):
 # ---------------------------------------------------------------------------------------------- #
 # super-resolution chaining and output assembly (s2_tiles_supres.py:332-342, 385-416)
 # ---------------------------------------------------------------------------------------------- #
-def super_resolve(data10, data20, data60, names10, names20, names60, deep=False, models=None, nodata=None):
+def super_resolve(data10, data20, data60, names10, names20, names60, deep=False, models=None, nodata=None,
+                  out_dtype=None):
     """The 60 m bands first, then the 20 m bands; returns (sr (H, W, n20 [+ n60]) or None, short names of its bands).
     ``models`` (extension): {'20': S2Model, '60': S2Model} instead of the shipped weight files; ``nodata`` (extension):
-    the nodata value of both calls (``supres.DSen2_20``)."""
+    the nodata value of both calls (``supres.DSen2_20``); ``out_dtype`` (extension): their output type (float32 if None,
+    or np.uint16)."""
     from . import supres
     models = models or {}
     extra = {} if nodata is None else {'nodata': nodata}
+    if out_dtype is not None:
+        extra['out_dtype'] = out_dtype
     sr60 = None
     if names60 and names20 and names10:
         print("Super-resolving the 60m data into 10m bands")
@@ -309,11 +316,24 @@ def build_parser():
     p.add_argument("--nodata", type=float, default=None,
                    help="Extension: input value of pixels without data (e.g. 0).  Pixels whose every band holds it stay "
                         "nodata in the output, which records the value; empty patches are not computed.")
+    p.add_argument("--output_dtype", choices=("float64", "uint16"), default="float64",
+                   help="Extension: data type of the written bands.  uint16: digital numbers like the input, rounded and "
+                        "clipped to [0, 65535] on the GPU; a computed value equal to --nodata is moved one step off it.")
     return p
 
 
+def parse_args(argv=None):
+    parser = build_parser()
+    args = parser.parse_args(argv)
+    if args.output_dtype == "uint16" and args.nodata is not None and \
+            not (args.nodata.is_integer() and 0 <= args.nodata <= 65535):
+        parser.error("--nodata %r is not a uint16 value (an integer in [0, 65535]), as --output_dtype uint16 needs"
+                     % args.nodata)
+    return args
+
+
 def main(argv=None, models=None):
-    args = build_parser().parse_args(argv)
+    args = parse_args(argv)
     if args.list_output_file_formats:                # before the input is opened, as in the reference (:64-79)
         for line in output_file_formats():
             print(line)
@@ -360,7 +380,9 @@ def main(argv=None, models=None):
     data10 = ds.read(0, w10, i10) if i10 else None
     data20 = ds.read(1, w20, i20) if i20 else None
     data60 = ds.read(2, w60, i60) if i60 else None
-    sr, sr_names = super_resolve(data10, data20, data60, n10, n20, n60, models=models, nodata=args.nodata)
+    u16 = args.output_dtype == "uint16"
+    sr, sr_names = super_resolve(data10, data20, data60, n10, n20, n60, models=models, nodata=args.nodata,
+                                 out_dtype=np.uint16 if u16 else None)
     if sr is None:
         print("No super-resolution performed, exiting")
         return 0
@@ -386,7 +408,8 @@ def main(argv=None, models=None):
         save_npz(output_file, bands, args.nodata)
     else:  # pragma: no cover - needs osgeo
         from osgeo import gdal
-        result = driver.Create(output_file, data10.shape[1], data10.shape[0], len(bands), gdal.GDT_Float64)
+        result = driver.Create(output_file, data10.shape[1], data10.shape[0], len(bands),
+                               gdal.GDT_UInt16 if u16 else gdal.GDT_Float64)
         result.SetGeoTransform(geot)
         result.SetProjection(ds.projection)
         for bidx, (desc, data) in enumerate(bands):

@@ -9,6 +9,11 @@ x2000 canvas.
 Nodata (an extension): with ``nodata=v``, an output pixel whose every input band (10 m, 20 m[, 60 m]) equals v is nodata
 and comes out as v; only the patches that own a pixel with data run the network.  Every other pixel is bit-identical to
 the output without ``nodata``.
+
+Digital-number output (an extension): with ``out_dtype=uint16`` the last layer rounds and saturates its values on the
+device and writes a uint16 canvas: NaN becomes 0, every other value is rint(clip(f, 0, 65535)) (half to even) of the float f
+the float32 output holds.  With ``nodata=v`` as well, nodata pixels are v, and a valid value that would round to v is
+written as v + 1 (65534 for v = 65535), so no computed value reads as nodata.
 """
 import math
 import os
@@ -75,6 +80,46 @@ def check_nodata(nodata, model, uint16_images):
     return v
 
 
+_OUT_DTYPES = {'float32': False, 'uint16': True}
+
+
+def check_out_dtype(out_dtype, model):
+    """True when ``out_dtype`` (a numpy or torch dtype; None = float32) asks for uint16 digital numbers, False for float32.
+    Rejected with ``ValueError``: any other type, and uint16 with a network without resBlocks (it runs the separate
+    extract / network / recompose kernels, which write float32; ``model`` None: not checked)."""
+    if out_dtype is None:
+        return False
+    name = str(out_dtype)
+    if name.startswith('torch.'):
+        name = name[len('torch.'):]
+    else:
+        try:
+            name = np.dtype(out_dtype).name
+        except TypeError:
+            name = None
+    if name not in _OUT_DTYPES:
+        raise ValueError("out_dtype must be float32 or uint16, got %r" % (out_dtype,))
+    u16 = _OUT_DTYPES[name]
+    if u16 and model is not None and not model.xin16:
+        raise ValueError("uint16 output needs a network with resBlocks (num_layers > 0)")
+    return u16
+
+
+def _check_out(out, shape, dtype, what):
+    if out is not None and (out.dtype != dtype or tuple(out.shape) != tuple(shape)):
+        raise ValueError("%s must be %s of shape %s, got %s of shape %s"
+                         % (what, dtype, tuple(shape), out.dtype, tuple(out.shape)))
+
+
+def _zeros_canvas(torch, shape, u16, device):
+    """Zero-filled device canvas: float32, or uint16 (zeroed through an int16 view: no CUDA fill of uint16 is needed)."""
+    if not u16:
+        return torch.zeros(shape, dtype=torch.float32, device=device)
+    out = torch.empty(shape, dtype=torch.uint16, device=device)
+    out.view(torch.int16).zero_()
+    return out
+
+
 def _nodata_args(d10, d20, d60, nodata):
     torch = _capi.require_cuda()
     g = _GEOM[d60 is not None]
@@ -99,15 +144,21 @@ def _scan_active(d10, d20, d60, first_patch, num_patches, nodata, ids, count, co
 
 def _run_active(model, d10, d20, d60, first_patch, num_patches, nodata, ids, out, device_batch, timers=None):
     """The network over the active patches ``ids`` (batches of at most ``device_batch``), then nodata into the nodata
-    pixels the range owns -- after the last layer, which also stitches active patches' values over their nodata pixels."""
+    pixels the range owns -- after the last layer, which also stitches active patches' values over their nodata pixels.
+    A uint16 ``out`` gets network values moved off v (``avoid``) and the uint16 fill."""
+    torch = _capi.require_cuda()
     g = _GEOM[d60 is not None]
+    u16 = out.dtype == torch.uint16
+    avoid = int(nodata) if u16 else None
     for i in range(0, int(ids.shape[0]), device_batch):
         batch = ids[i:i + device_batch]
         model.forward_images(d10, d20, d60, g['patch'], g['border'], 0, int(batch.shape[0]), out, float(SCALE),
-                             timers=timers, patch_ids=batch)
+                             timers=timers, patch_ids=batch, avoid=avoid)
     imgs, v = _nodata_args(d10, d20, d60, nodata)
-    S2Model._timed(timers, 'nodata_fill', num_patches, lambda: _capi.check(_capi.lib().dsen2_nodata_fill(
-        *imgs, first_patch, num_patches, v, model.out_channels, _capi.ptr(out), _capi.stream_ptr()), "dsen2_nodata_fill"))
+    name = 'dsen2_nodata_fill_u16' if u16 else 'dsen2_nodata_fill'
+    fill = getattr(_capi.lib(), name)
+    S2Model._timed(timers, 'nodata_fill', num_patches, lambda: _capi.check(fill(
+        *imgs, first_patch, num_patches, v, model.out_channels, _capi.ptr(out), _capi.stream_ptr()), name))
 
 
 def _active(d10, d20, d60, first_patch, num_patches, nodata, timers=None):
@@ -145,22 +196,26 @@ def active_patches(d10, d20, d60=None, nodata=0, first_patch=0, num_patches=None
 
 
 def super_resolve_device(model, d10, d20, d60=None, first_patch=0, num_patches=None, out=None, device_batch=None,
-                         timers=None, nodata=None):
+                         timers=None, nodata=None, out_dtype=None):
     """Device-level pipeline.  d10/d20(/d60): CUDA HWC tensors, all float32 or all uint16.  Processes patches
     [first_patch, first_patch+num_patches) of the FILLED patch list (surplus zero patches of
     patches.py:32-39 are never read by recompose_images, so they are skipped) and writes the pixels those
-    patches own into ``out`` (H, W, Cout) float32 (allocated zero-filled if None).  ``nodata``: see the module
-    docstring; the active patches are found on the device, and their number is the one value read back."""
+    patches own into ``out`` (H, W, Cout) of ``out_dtype`` (torch.float32 when None, or torch.uint16: see the module
+    docstring; allocated zero-filled if None).  ``nodata``: see the module docstring; the active patches are found on
+    the device, and their number is the one value read back."""
     torch = _capi.require_cuda()
-    nodata = check_nodata(nodata, model, d10.dtype == torch.uint16)
+    u16 = check_out_dtype(out_dtype, model)
+    nodata = check_nodata(nodata, model, d10.dtype == torch.uint16 or u16)
     run_60 = d60 is not None
     g = _GEOM[run_60]
     r, P, B = g['ratio'], g['patch'], g['border']
     H, W = int(d10.shape[0]), int(d10.shape[1])
     plr, blr = P // r, B // r
+    shape = (H, W, model.out_channels)
+    _check_out(out, shape, torch.uint16 if u16 else torch.float32, "out")
     num_patches = _filled_range(d10, run_60, first_patch, num_patches)
     if out is None:
-        out = torch.zeros((H, W, model.out_channels), dtype=torch.float32, device=d10.device)
+        out = _zeros_canvas(torch, shape, u16, d10.device)
     if device_batch is None:
         device_batch = default_device_batch(W, P, B)
     # recompose_images' "lone patch is returned uncropped" branch (patches.py:375-376) keys on the ALLOCATED patch count
@@ -195,9 +250,9 @@ def _np_dtype_of(torch, dt):
 class _Slot:
     """One slot of the pinned staging ring: input rows of a chunk per resolution + the output rectangles it owns."""
 
-    def __init__(self, torch, shapes_in, dtype, out_elems):
+    def __init__(self, torch, shapes_in, dtype, out_elems, out_dtype):
         self.inp = [torch.empty(s, dtype=dtype).pin_memory() for s in shapes_in]
-        self.out = torch.empty((out_elems,), dtype=torch.float32).pin_memory()
+        self.out = torch.empty((out_elems,), dtype=out_dtype).pin_memory()
         self.ev_h2d, self.ev_d2h = torch.cuda.Event(), torch.cuda.Event()
         self.used_in = self.used_out = False
 
@@ -212,11 +267,14 @@ class HostPipeline:
     by worker threads (numpy releases the GIL for the copies), so neither the page-locked upload nor the first-touch
     page faults of a freshly allocated output serialise with the GPU.  ``dtype``: element type of the device-resident
     images, float32 or uint16 (Sentinel-2 digital numbers as GDAL delivers them, s2_tiles_supres.py:311-315: half the
-    bytes over PCIe; ``dsen2_prep16_from_images`` converts exactly, results are bit-identical)."""
+    bytes over PCIe; ``dsen2_prep16_from_images`` converts exactly, results are bit-identical).  ``out_dtype``: element
+    type of the output canvas and of the host output, float32 (None) or uint16 (module docstring: half the bytes back)."""
 
     RING = 3
 
-    def __init__(self, model, H, W, run_60=False, device=None, chunk_patch_rows=None, device_batch=None, dtype=None):
+    def __init__(self, model, H, W, run_60=False, device=None, chunk_patch_rows=None, device_batch=None, dtype=None,
+                 out_dtype=None):
+        u16 = check_out_dtype(out_dtype, model)
         torch = _capi.require_cuda()
         self.torch, self.model, self.run_60 = torch, model, run_60
         self.H, self.W = int(H), int(W)
@@ -233,7 +291,8 @@ class HostPipeline:
         mk = lambda h, w, c: torch.empty((h, w, c), dtype=self.dtype, device=self.dev)
         self.d10, self.d20 = mk(self.H, self.W, 4), mk(self.H // 2, self.W // 2, 6)
         self.d60 = mk(self.H // 6, self.W // 6, 2) if run_60 else None
-        self.canvas = torch.zeros((self.H, self.W, model.out_channels), dtype=torch.float32, device=self.dev)
+        self.out_dtype = torch.uint16 if u16 else torch.float32
+        self.canvas = _zeros_canvas(torch, (self.H, self.W, model.out_channels), u16, self.dev)
         self.up, self.down = torch.cuda.Stream(self.dev), torch.cuda.Stream(self.dev)
         self.h2d_bytes = self.d2h_bytes = 0
         self._slots, self._pool = None, None
@@ -253,7 +312,7 @@ class HostPipeline:
         """Device id list of the range, device and pinned per-chunk counts: chunk k scans into its own slice / entry, so
         the upload stream never overwrites what an earlier chunk's network still reads."""
         torch = self.torch
-        nodata = check_nodata(nodata, self.model, self.dtype == torch.uint16)
+        nodata = check_nodata(nodata, self.model, self.dtype == torch.uint16 or self.out_dtype == torch.uint16)
         if nodata is None:
             return None, None, None, None
         ids = torch.empty((max(1, num_patches),), dtype=torch.int32, device=self.dev)
@@ -265,7 +324,7 @@ class HostPipeline:
         the active patches its scan found, then the nodata fill."""
         if nodata is None:
             super_resolve_device(self.model, self.d10, self.d20, self.d60, first_patch=p0, num_patches=cnt,
-                                 out=self.canvas, device_batch=self.device_batch, timers=timers)
+                                 out=self.canvas, device_batch=self.device_batch, timers=timers, out_dtype=self.out_dtype)
             return
         ev_scan.synchronize()                        # this chunk's upload and scan only, never an earlier network
         batch = self.device_batch or default_device_batch(self.W, self.P, self.B)
@@ -274,15 +333,16 @@ class HostPipeline:
                     batch, timers)
 
     def run(self, h10, h20, h60=None, hout=None, first_patch=0, num_patches=None, timers=None, nodata=None):
-        """Pinned torch tensors in (dtype = the pipeline's), pinned float32 (H, W, Cout) tensor out.  Rows of ``hout`` that
-        the patch range owns only partly (the seam rows of a sharded range) are downloaded whole.  ``nodata``: see the
+        """Pinned torch tensors in (dtype = the pipeline's), pinned (H, W, Cout) tensor of ``out_dtype`` out.  Rows of
+        ``hout`` that the patch range owns only partly (the seam rows of a sharded range) are downloaded whole.  ``nodata``: see the
         module docstring; each chunk's patch scan runs on the upload stream right behind its upload."""
         torch = self.torch
         filled = self.ny * self.nx
         if num_patches is None:
             num_patches = filled - first_patch
         if hout is None:
-            hout = torch.empty((self.H, self.W, self.model.out_channels), dtype=torch.float32).pin_memory()
+            hout = torch.empty((self.H, self.W, self.model.out_channels), dtype=self.out_dtype).pin_memory()
+        _check_out(hout, self.canvas.shape, self.out_dtype, "hout")
         for h in (h10, h20) + ((h60,) if self.run_60 else ()):
             if h.dtype != self.dtype:
                 raise ValueError("host image dtype %s does not match the pipeline's %s" % (h.dtype, self.dtype))
@@ -318,7 +378,7 @@ class HostPipeline:
                     # of those rows that another rank owns come along as they are on this device (never computed here);
                     # `sharding.assemble` / `owned_rects` say which part of a row is this rank's.
                     hout[y0:y1].copy_(self.canvas[y0:y1], non_blocking=True)
-                    self.d2h_bytes += (y1 - y0) * self.W * self.canvas.shape[2] * 4
+                    self.d2h_bytes += (y1 - y0) * self.W * self.canvas.shape[2] * self.canvas.element_size()
         main.wait_stream(self.down)
         return hout
 
@@ -342,7 +402,7 @@ class HostPipeline:
             * self.canvas.shape[2]
         if self._slots is None or any(a.shape[0] < s[0] for a, s in zip(self._slots[0].inp, shapes)) \
                 or self._slots[0].out.numel() < out_elems:
-            self._slots = [_Slot(torch, shapes, self.dtype, out_elems) for _ in range(self.RING)]
+            self._slots = [_Slot(torch, shapes, self.dtype, out_elems, self.out_dtype) for _ in range(self.RING)]
         if self._pool is None:
             from concurrent.futures import ThreadPoolExecutor
             self._pool = ThreadPoolExecutor(max_workers=4, thread_name_prefix='dsen2-stage',
@@ -350,15 +410,17 @@ class HostPipeline:
         return self._slots
 
     def run_numpy(self, a10, a20, a60=None, out=None, first_patch=0, num_patches=None, timers=None, nodata=None):
-        """Pageable numpy arrays in -> numpy (H, W, Cout) float32 out (allocated if None).  Arrays whose dtype is not
-        the pipeline's are cast while they are staged.  ``nodata`` as in ``run``."""
+        """Pageable numpy arrays in -> numpy (H, W, Cout) array of ``out_dtype`` out (allocated if None).  Arrays whose
+        dtype is not the pipeline's are cast while they are staged.  ``nodata`` as in ``run``."""
         torch = self.torch
         filled = self.ny * self.nx
         if num_patches is None:
             num_patches = filled - first_patch
         C = self.model.out_channels
+        np_out = _np_dtype_of(torch, self.out_dtype)
         if out is None:
-            out = np.empty((self.H, self.W, C), np.float32)
+            out = np.empty((self.H, self.W, C), np_out)
+        _check_out(out, (self.H, self.W, C), np.dtype(np_out), "out")
         srcs = [a10, a20] + ([a60] if self.run_60 else [])
         divs = (1, 2, 6) if self.run_60 else (1, 2)
         devs = [self.d10, self.d20] + ([self.d60] if self.run_60 else [])
@@ -432,7 +494,7 @@ class HostPipeline:
                               non_blocking=True)
                     offs.append(o)
                     o += nel
-                    self.d2h_bytes += nel * 4
+                    self.d2h_bytes += nel * self.canvas.element_size()
                 slot.ev_d2h.record(self.down)
             src = slot.out.numpy()
 
@@ -450,22 +512,29 @@ class HostPipeline:
 _pipe_cache = {}
 
 
-def _pipeline_for(model, H, W, run_60, dtype):
+def _pipeline_for(model, H, W, run_60, dtype, out_dtype):
     """HostPipeline objects (device-resident tile + pinned staging ring) are kept for the last shapes used, so a caller
     that super-resolves scene after scene pays the allocations once."""
     torch = _capi.require_cuda()
-    key = (id(model), H, W, run_60, dtype, torch.cuda.current_device())
+    key = (id(model), H, W, run_60, dtype, out_dtype, torch.cuda.current_device())
     pipe = _pipe_cache.get(key)
     if pipe is None or pipe.model is not model:
         if len(_pipe_cache) >= 2:
             _pipe_cache.clear()
-        pipe = _pipe_cache[key] = HostPipeline(model, H, W, run_60=run_60, dtype=dtype)
+        pipe = _pipe_cache[key] = HostPipeline(model, H, W, run_60=run_60, dtype=dtype, out_dtype=out_dtype)
     return pipe
 
 
-def _run(model, arrays, out=None, nodata=None):
-    if nodata is not None:                   # rejected before the device is touched
-        nodata = check_nodata(nodata, model, model.xin16 and all(np.asarray(a).dtype == np.uint16 for a in arrays))
+def _run(model, arrays, out=None, nodata=None, out_dtype=np.float32):
+    # rejected before the device is touched
+    u16 = check_out_dtype(out_dtype, model)
+    if nodata is not None:
+        nodata = check_nodata(nodata, model,
+                              u16 or (model.xin16 and all(np.asarray(a).dtype == np.uint16 for a in arrays)))
+    a10 = np.asarray(arrays[0])
+    if out is not None and a10.ndim >= 2:
+        _check_out(out, (a10.shape[0], a10.shape[1], model.out_channels), np.dtype(np.uint16 if u16 else np.float32),
+                   "out")
     torch = _capi.require_cuda()
     arrays = [np.asarray(a) for a in arrays]
     H, W = int(arrays[0].shape[0]), int(arrays[0].shape[1])
@@ -476,25 +545,26 @@ def _run(model, arrays, out=None, nodata=None):
     # uint16 digital numbers (GDAL, s2_tiles_supres.py:311-315) stay uint16 up to the input-preparation kernel; everything
     # else is staged as float32 (the reference divides by SCALE in floating point whatever the input type, supres.py:23-24)
     dtype = torch.uint16 if (model.xin16 and all(a.dtype == np.uint16 for a in arrays)) else torch.float32
-    pipe = _pipeline_for(model, H, W, len(arrays) == 3, dtype)
+    pipe = _pipeline_for(model, H, W, len(arrays) == 3, dtype, torch.uint16 if u16 else torch.float32)
     res = pipe.run_numpy(*arrays, out=out, nodata=nodata)
     torch.cuda.current_stream().synchronize()
     return res
 
 
-def DSen2_20(d10, d20, deep=False, model=None, out=None, nodata=None):
+def DSen2_20(d10, d20, deep=False, model=None, out=None, nodata=None, out_dtype=np.float32):
     """supres.py:15-30.  d10 (H,W,4), d20 (H/2,W/2,6) -> (H,W,6) float32.  Extensions: ``model`` supplies a preloaded
-    ``S2Model`` instead of the shipped hdf5 weights, ``out`` a preallocated (H,W,6) float32 array to fill, ``nodata`` the
-    input value of pixels without data (module docstring): they come out as ``nodata`` and empty patches are skipped."""
+    ``S2Model`` instead of the shipped hdf5 weights, ``out`` a preallocated (H,W,6) array of ``out_dtype`` to fill,
+    ``nodata`` the input value of pixels without data (module docstring): they come out as ``nodata`` and empty patches are
+    skipped; ``out_dtype`` np.uint16: digital numbers, rounded and saturated on the device (module docstring)."""
     input_shape = ((4, None, None), (6, None, None))
     if model is None:
         model = _load_model(input_shape, deep, run_60=False)
-    return _run(model, [d10, d20], out, nodata)
+    return _run(model, [d10, d20], out, nodata, out_dtype)
 
 
-def DSen2_60(d10, d20, d60, deep=False, model=None, out=None, nodata=None):
-    """supres.py:33-50.  + d60 (H/6,W/6,2) -> (H,W,2) float32."""
+def DSen2_60(d10, d20, d60, deep=False, model=None, out=None, nodata=None, out_dtype=np.float32):
+    """supres.py:33-50.  + d60 (H/6,W/6,2) -> (H,W,2) float32 (or ``out_dtype``)."""
     input_shape = ((4, None, None), (6, None, None), (2, None, None))
     if model is None:
         model = _load_model(input_shape, deep, run_60=True)
-    return _run(model, [d10, d20, d60], out, nodata)
+    return _run(model, [d10, d20, d60], out, nodata, out_dtype)

@@ -216,6 +216,14 @@ int dsen2_conv_tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void*
                              const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
                              int n, int P, int first_patch, int border, int img_h, int img_w, float mul,
                              float* d_canvas, void* stream);
+/* The same into a (img_h, img_w, cout) uint16 canvas of digital numbers: with f the float the entry above writes, the
+ * value is 0 for NaN and otherwise rint(clip(f, 0, 65535)) (round half to even).  A value equal to `avoid` (the nodata
+ * value of the run, -1 = none, otherwise in [0, 65535]) is written as avoid + 1 (65534 for 65535): a network output never
+ * reads as nodata.                                                                                                  */
+int dsen2_conv_tail16_stitch_u16(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                 const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
+                                 int n, int P, int first_patch, int border, int img_h, int img_w, float mul, int avoid,
+                                 uint16_t* d_canvas, void* stream);
 
 /* The same two steps for an arbitrary list of patches (the active patches of dsen2_nodata_patches): the arguments of
  * dsen2_prep16_from_images / dsen2_conv_tail16_stitch, with batch entry b = patch d_patch_ids[b] (absolute indices in the
@@ -228,6 +236,11 @@ int dsen2_conv_tail16_stitch_ids(const void* d_x_hi, const void* d_x_lo, const v
                                  const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
                                  int n, int P, const int* d_patch_ids, int border, int img_h, int img_w, float mul,
                                  float* d_canvas, void* stream);
+/* dsen2_conv_tail16_stitch_u16 for a list of patches. */
+int dsen2_conv_tail16_stitch_ids_u16(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                     const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
+                                     int n, int P, const int* d_patch_ids, int border, int img_h, int img_w, float mul,
+                                     int avoid, uint16_t* d_canvas, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Nodata (csrc/nodata.cu; an extension: the reference super-resolves nodata like data).  Images, img_dtype, H, W, patch
@@ -239,6 +252,8 @@ int dsen2_conv_tail16_stitch_ids(const void* d_x_hi, const void* d_x_lo, const v
  *       d_ids[0, *d_count).  d_ids holds num_patches ints (it is also the scan's scratch); d_count one int.
  *   dsen2_nodata_fill: writes v into all cout bands of every nodata pixel of the (H, W, cout) float32 canvas that the
  *       range owns.  Run it after the last layer: an active patch also stitches network values over its nodata pixels.
+ *   dsen2_nodata_fill_u16: the same for the uint16 canvas of dsen2_conv_tail16_stitch[_ids]_u16; v must be an integer in
+ *       [0, 65535].  With avoid = v there, nodata pixels are exactly those that hold v.
  * Running only the active patches (dsen2_*_ids) and then the fill leaves every valid pixel bit-identical to the whole
  * range run without nodata.                                                                                          */
 int dsen2_nodata_patches(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H, int W,
@@ -247,6 +262,9 @@ int dsen2_nodata_patches(const void* d_img10, const void* d_img20, const void* d
 int dsen2_nodata_fill(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H, int W,
                       int patch, int border, int first_patch, int num_patches, float nodata, int cout, float* d_canvas,
                       void* stream);
+int dsen2_nodata_fill_u16(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H, int W,
+                          int patch, int border, int first_patch, int num_patches, float nodata, int cout,
+                          uint16_t* d_canvas, void* stream);
 
 /* Whole s2model forward (model.predict on one batch, supres.py:65) for n patches of (P, P).
  * d_weights[i] / d_bias[i] are the packed layers in Keras topological order (2*num_layers+2 entries):

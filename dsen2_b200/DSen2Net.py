@@ -370,7 +370,7 @@ class S2Model:
         return out
 
     def forward_images(self, d10, d20, d60, patch, border, first_patch, n, canvas, mul, timers=None, patch_ids=None,
-                       avoid=None):
+                       avoid=None, add_offset=None):
         """Fused tile pipeline of the fast path: patches [first_patch, first_patch+n) are gathered straight
         from the HWC images (extract + bilinear + /mul), run through the network, and the pixels they own
         are written x mul into ``canvas`` (H, W, Cout).  No patch stack or prediction stack exists.  The images are
@@ -378,7 +378,9 @@ class S2Model:
         run instead of the range (``first_patch`` is then ignored).  ``canvas`` is a contiguous float32 or uint16 tensor;
         a uint16 canvas receives the float values rounded half to even and clipped to [0, 65535] (NaN: 0), and a value
         equal to ``avoid`` (an int in [0, 65535], the nodata value) is written one step away from it
-        (``dsen2_conv_tail16_stitch_u16`` in include/dsen2_b200.h)."""
+        (``dsen2_conv_tail16_stitch_u16`` in include/dsen2_b200.h).  ``add_offset``: a finite float (None: none) added to
+        every band value before the preparation and subtracted from every output value before it is stored
+        (``dsen2_prep16_from_images_offset``, ``dsen2_conv_tail16_stitch_offset``)."""
         torch = _capi.require_cuda()
         if not self.xin16:
             raise _capi.DSen2Error("forward_images needs a network with resblocks (num_layers > 0)")
@@ -408,7 +410,12 @@ class S2Model:
         buf = self._buffers(dev, n, patch, reuse_larger=patch_ids is not None)
         with torch.cuda.device(dev):
             st = _capi.stream_ptr()
-            if patch_ids is None:
+            if add_offset is not None:
+                self._timed(timers, 'prep', n, lambda: _capi.check(lib.dsen2_prep16_from_images_offset(
+                    ptr(d10), ptr(d20), ptr(d60), img_dtype, H, W, patch, border, first_patch, ptr(patch_ids), n,
+                    float(mul), float(add_offset), ptr(buf['xin_hi']), ptr(buf['xin_lo']), st),
+                    "dsen2_prep16_from_images_offset"))
+            elif patch_ids is None:
                 self._timed(timers, 'prep', n, lambda: _capi.check(lib.dsen2_prep16_from_images(
                     ptr(d10), ptr(d20), ptr(d60), img_dtype, H, W, patch, border, first_patch, n, float(mul),
                     ptr(buf['xin_hi']), ptr(buf['xin_lo']), st), "dsen2_prep16_from_images"))
@@ -417,6 +424,12 @@ class S2Model:
                     ptr(d10), ptr(d20), ptr(d60), img_dtype, H, W, patch, border, ptr(patch_ids), n, float(mul),
                     ptr(buf['xin_hi']), ptr(buf['xin_lo']), st), "dsen2_prep16_from_images_ids"))
             self._trunk(buf, wts, biases, n, patch, st, timers)
+            if add_offset is not None:
+                self._timed(timers, 'conv_tail', n, lambda: _capi.check(lib.dsen2_conv_tail16_stitch_offset(
+                    *self._tail_args(buf, wts, biases), self.feature_size, n, patch, first_patch, ptr(patch_ids), border,
+                    H, W, float(mul), float(add_offset), _capi.IMG_U16 if u16 else _capi.IMG_F32, avoid, ptr(canvas), st),
+                    "dsen2_conv_tail16_stitch_offset"))
+                return canvas
             # the canvas type picks the entry point; the uint16 ones take the value to avoid after the scale
             which = (ptr(patch_ids),) if patch_ids is not None else (first_patch,)
             name = 'dsen2_conv_tail16_stitch' + ('_ids' if patch_ids is not None else '') + ('_u16' if u16 else '')

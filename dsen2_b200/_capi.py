@@ -65,6 +65,11 @@ SIGNATURES = {
                                                  c_void_p]),
     "dsen2_nodata_fill_u16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                       c_float, c_int, c_void_p, c_void_p]),
+    "dsen2_prep16_from_images_offset": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
+                                                c_void_p, c_int, c_float, c_float, c_void_p, c_void_p, c_void_p]),
+    "dsen2_conv_tail16_stitch_offset": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                                c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_float, c_float,
+                                                c_int, c_int, c_void_p, c_void_p]),
     "dsen2_conv_resq256": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p,
                                    c_void_p, c_void_p]),
     "dsen2_conv_tail": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,

@@ -53,6 +53,7 @@ struct TailParams {
   int first_patch, img_h, img_w, border, grid_ny, grid_nx;
   const int* patch_ids;               // stitching form with IDS: batch entry b is patch patch_ids[b], not first_patch + b
   int avoid;                          // uint16 canvas: a value the network must not write (the nodata value), -1 none
+  float add_offset;                   // instances with ADD: subtracted from every stitched value (the product's radiometric offset)
 };
 
 // The uint16 (digital number) canvas value of the float f the float canvas receives: NaN -> 0, else rint(clip(f, 0, 65535))
@@ -80,7 +81,7 @@ __device__ __forceinline__ int tail_stitch_tile_of(int y, int size, int S, int n
   return (size % S != 0 && y >= size - S) ? n - 1 : y / S;
 }
 
-template <int KPM, bool IDS, typename OutT>
+template <int KPM, bool IDS, typename OutT, bool ADD>
 __global__ void __launch_bounds__(kTThreads, 1)
 conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
                          const __grid_constant__ CUtensorMap tm_w, const TailParams p) {
@@ -263,8 +264,10 @@ conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid
             }
             const float v = (vh + vl) + s_bias[c_lo + i];
             const float skip = __half2float(ch[i]) + __half2float(cl[i]);
-            store_out(static_cast<OutT*>(p.out) + obase + (c_lo + i) * ostride, (v + skip) * p.out_mul,   // Add
-                      p.avoid);                                                                       // (DSen2Net.py:38), x SCALE
+            // Add (DSen2Net.py:38), x SCALE; ADD: - add_offset, back to the product's convention (__fsub_rn is never
+            // contracted into an FMA with the multiply)
+            store_out(static_cast<OutT*>(p.out) + obase + (c_lo + i) * ostride,
+                      ADD ? __fsub_rn((v + skip) * p.out_mul, p.add_offset) : (v + skip) * p.out_mul, p.avoid);
           }
         }
       }
@@ -299,12 +302,12 @@ __global__ void pack_tail16_weights_kernel(const float* __restrict__ hwio, int F
   }
 }
 
-template <int KPM, bool IDS, typename OutT>
+template <int KPM, bool IDS, typename OutT, bool ADD>
 static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_lo, const void* d_w, int sms, cudaStream_t stream) {
   using Cfg = TailCfg<KPM>;
   static bool configured[64] = {};
   if (needs_config(configured)) {
-    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM, IDS, OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM, IDS, OutT, ADD>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   }
   const int F = KPM * 64;
   CUtensorMap hi, lo, w;
@@ -317,14 +320,22 @@ static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_
   const uint32_t wb[2] = {64, 128};
   if ((rc = make_tmap_f16_sw(&w, d_w, 2, wd, wb, 128)) != 0) return rc;
   const int grid = (int)(p.num_tiles < (uint32_t)sms ? p.num_tiles : (uint32_t)sms);
-  conv_tail_swapped_kernel<KPM, IDS, OutT><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
+  conv_tail_swapped_kernel<KPM, IDS, OutT, ADD><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
   return check_launch("conv_tail_swapped");
 }
 
+template <bool IDS, typename OutT, bool ADD>
+static int launch_tail_f(const TailParams& p, int features, const void* d_x_hi, const void* d_x_lo, const void* d_w, int sms,
+                         cudaStream_t stream) {
+  return features == 256 ? launch_tail<4, IDS, OutT, ADD>(p, d_x_hi, d_x_lo, d_w, sms, stream)
+                         : launch_tail<2, IDS, OutT, ADD>(p, d_x_hi, d_x_lo, d_w, sms, stream);
+}
+
+// add: run the ADD instances, which subtract p.add_offset from every stitched value
 template <typename OutT>
 static int tail16_common(TailParams& p, int features, const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
                          const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int n, int H, int W, OutT* d_out,
-                         void* stream) {
+                         bool add, void* stream) {
   DSEN2_REQUIRE(d_x_hi && d_x_lo && d_w && d_bias && d_xin_hi && d_xin_lo && d_out, DSEN2_E_BADARG, "dsen2_conv_tail16: null pointer");
   DSEN2_REQUIRE(features == 128 || features == 256, DSEN2_E_BADARG, "dsen2_conv_tail16: feature_size must be 128 or 256 (got %d)",
                 features);
@@ -354,10 +365,10 @@ static int tail16_common(TailParams& p, int features, const void* d_x_hi, const 
   p.cout = cout; p.out = d_out;
   const cudaStream_t st = (cudaStream_t)stream;
   if (p.patch_ids)
-    return features == 256 ? launch_tail<4, true, OutT>(p, d_x_hi, d_x_lo, d_w, sms, st)
-                           : launch_tail<2, true, OutT>(p, d_x_hi, d_x_lo, d_w, sms, st);
-  return features == 256 ? launch_tail<4, false, OutT>(p, d_x_hi, d_x_lo, d_w, sms, st)
-                         : launch_tail<2, false, OutT>(p, d_x_hi, d_x_lo, d_w, sms, st);
+    return add ? launch_tail_f<true, OutT, true>(p, features, d_x_hi, d_x_lo, d_w, sms, st)
+               : launch_tail_f<true, OutT, false>(p, features, d_x_hi, d_x_lo, d_w, sms, st);
+  return add ? launch_tail_f<false, OutT, true>(p, features, d_x_hi, d_x_lo, d_w, sms, st)
+             : launch_tail_f<false, OutT, false>(p, features, d_x_hi, d_x_lo, d_w, sms, st);
 }
 
 }  // namespace dsen2
@@ -383,15 +394,16 @@ extern "C" int dsen2_conv_tail16(const void* d_x_hi, const void* d_x_lo, const v
   p.out_mul = 1.0f;
   p.avoid = -1;
   return tail16_common<float>(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, H, W, d_pred_nchw,
-                       stream);
+                       false, stream);
 }
 
-// the stitching form: patches first_patch + b, or d_patch_ids[b] when d_patch_ids is not null; float or uint16 canvas
+// the stitching form: patches first_patch + b, or d_patch_ids[b] when d_patch_ids is not null; float or uint16 canvas;
+// with add, add_offset is subtracted from every value after the scale
 template <typename OutT>
 static int tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias, const void* d_xin_hi,
                          const void* d_xin_lo, int skip_ch0, int cout, int feature_size, int n, int P, int first_patch,
                          const int* d_patch_ids, int border, int img_h, int img_w, float mul, int avoid, OutT* d_canvas,
-                         void* stream) {
+                         void* stream, bool add = false, float add_offset = 0.f) {
   const int S = P - 2 * border;
   DSEN2_REQUIRE(P > 0 && border >= 0 && S > 0 && img_h >= S && img_w >= S && first_patch >= 0, DSEN2_E_BADARG,
                 "dsen2_conv_tail16_stitch: bad stitch geometry (P %d border %d image %dx%d)", P, border, img_h, img_w);
@@ -400,6 +412,7 @@ static int tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w
   p.tail_mode = 1;
   p.out_mul = mul;
   p.avoid = avoid;
+  p.add_offset = add_offset;
   p.first_patch = first_patch; p.img_h = img_h; p.img_w = img_w; p.border = border;
   p.grid_ny = ceil_div(img_h, S); p.grid_nx = ceil_div(img_w, S);
   p.patch_ids = d_patch_ids;
@@ -407,7 +420,7 @@ static int tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w
                 "dsen2_conv_tail16_stitch: patch range [%d,%d) exceeds the %d tiles of the canvas", first_patch,
                 first_patch + n, p.grid_ny * p.grid_nx);
   return tail16_common<OutT>(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, P, P,
-                             d_canvas, stream);
+                             d_canvas, add, stream);
 }
 
 extern "C" int dsen2_conv_tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
@@ -443,4 +456,23 @@ extern "C" int dsen2_conv_tail16_stitch_ids_u16(const void* d_x_hi, const void* 
   DSEN2_REQUIRE(d_patch_ids, DSEN2_E_BADARG, "dsen2_conv_tail16_stitch_ids_u16: null pointer");
   return tail16_stitch<uint16_t>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P, 0,
                                  d_patch_ids, border, img_h, img_w, mul, avoid, d_canvas, stream);
+}
+
+extern "C" int dsen2_conv_tail16_stitch_offset(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                               const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout,
+                                               int feature_size, int n, int P, int first_patch, const int* d_patch_ids,
+                                               int border, int img_h, int img_w, float mul, float add_offset,
+                                               int canvas_dtype, int avoid, void* d_canvas, void* stream) {
+  DSEN2_REQUIRE(isfinite(add_offset), DSEN2_E_BADARG, "dsen2_conv_tail16_stitch_offset: add_offset must be finite");
+  DSEN2_REQUIRE(canvas_dtype == DSEN2_IMG_F32 || canvas_dtype == DSEN2_IMG_U16, DSEN2_E_BADARG,
+                "dsen2_conv_tail16_stitch_offset: canvas_dtype must be DSEN2_IMG_F32 or DSEN2_IMG_U16 (got %d)", canvas_dtype);
+  DSEN2_REQUIRE(canvas_dtype == DSEN2_IMG_U16 || avoid == -1, DSEN2_E_BADARG,
+                "dsen2_conv_tail16_stitch_offset: avoid must be -1 for a float canvas (got %d)", avoid);
+  const int first = d_patch_ids ? 0 : first_patch;
+  if (canvas_dtype == DSEN2_IMG_U16)
+    return tail16_stitch<uint16_t>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P,
+                                   first, d_patch_ids, border, img_h, img_w, mul, avoid, (uint16_t*)d_canvas, stream, true,
+                                   add_offset);
+  return tail16_stitch<float>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P, first,
+                              d_patch_ids, border, img_h, img_w, mul, -1, (float*)d_canvas, stream, true, add_offset);
 }

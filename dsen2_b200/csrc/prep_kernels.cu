@@ -7,6 +7,7 @@
 //                               get_test_patches60 (patches.py:19-156: symmetric pad, crop), interp_patches
 //                               (patches.py:11-16: per-patch bilinear with mirror boundary) and the /2000 scaling
 //                               (supres.py:23-24,42-44) with the arithmetic of the standalone kernels.
+//   dsen2_prep16_from_images_offset : the same with a radiometric offset added to every loaded band value first
 // Training step (and networks without resblocks): "x_in", 64 channels per pixel = the three HORIZONTAL taps of the first
 // 3x3 convolution pre-gathered, x_in[n][y][x][t*16 + c] = X[n][c][y][x + t - 1] (zero outside the patch), because the
 // first layer's weight-gradient GEMM wants 128-byte pixel rows (dsen2_prep_from_patches).
@@ -41,17 +42,24 @@ struct PrepSource {
   int s;              // upsampling factor to the 10 m patch (1 = none)
 };
 
+// A band value as the arithmetic below takes it: the stored element, or with ADD fl32(x + add_offset) (the radiometric
+// offset of Sentinel-2 products since processing baseline 04.00).  ADD is a template switch, not an add of 0: -0 + 0 is +0.
+template <bool ADD, typename T>
+__device__ __forceinline__ float ld_band(const T* p, float add_offset) {
+  return ADD ? __fadd_rn(ld_px(p), add_offset) : ld_px(p);
+}
+
 // value of band c of `src` at 10 m patch pixel (y, x): crop + symmetric pad (+ mirror bilinear) + /divisor
-template <typename T, int C, int OFF>
+template <typename T, int C, int OFF, bool ADD>
 __device__ __forceinline__ void prep_gather(const PrepSource& src, int si, int sj, int plr, int blr, int y, int x,
-                                            float divisor, float (&v)[16]) {
+                                            float divisor, float add_offset, float (&v)[16]) {
   const T* img = reinterpret_cast<const T*>(src.img);
   const int p = plr * src.ratio, b = blr * src.ratio;
   const int oi = si * src.ratio - b, oj = sj * src.ratio - b;
   if (src.s == 1) {
     const T* q = img + ((long long)sym_index(oi + y, src.H) * src.W + sym_index(oj + x, src.W)) * C;
 #pragma unroll
-    for (int c = 0; c < C; ++c) v[OFF + c] = __fdiv_rn(ld_px(q + c), divisor);
+    for (int c = 0; c < C; ++c) v[OFF + c] = __fdiv_rn(ld_band<ADD>(q + c, add_offset), divisor);
     return;
   }
   int y0, y1, x0, x1;
@@ -67,8 +75,8 @@ __device__ __forceinline__ void prep_gather(const PrepSource& src, int si, int s
   const float k = 30000.0f;                  // the reference scales by 1/30000 around the resize (patches.py:15)
 #pragma unroll
   for (int c = 0; c < C; ++c) {
-    const float v00 = __fdiv_rn(ld_px(p00 + c), k), v01 = __fdiv_rn(ld_px(p01 + c), k);
-    const float v10 = __fdiv_rn(ld_px(p10 + c), k), v11 = __fdiv_rn(ld_px(p11 + c), k);
+    const float v00 = __fdiv_rn(ld_band<ADD>(p00 + c, add_offset), k), v01 = __fdiv_rn(ld_band<ADD>(p01 + c, add_offset), k);
+    const float v10 = __fdiv_rn(ld_band<ADD>(p10 + c, add_offset), k), v11 = __fdiv_rn(ld_band<ADD>(p11 + c, add_offset), k);
     const float c0 = v00 * (1.0f - fy) + v10 * fy;   // rows first, then columns (as bilinear_mirror_kernel)
     const float c1 = v01 * (1.0f - fy) + v11 * fy;
     const float r = (c0 * (1.0f - fx) + c1 * fx) * k;
@@ -104,11 +112,13 @@ __global__ void prep16_from_patches_kernel(const float* __restrict__ x0, int c0,
   }
 }
 
-// IDS: batch entry b is patch ids[b] (a list of active patches) instead of first_patch + b
-template <typename T, bool IDS>
+// IDS: batch entry b is patch ids[b] (a list of active patches) instead of first_patch + b.  ADD: add_offset is added to
+// every loaded band value (ld_band); it is the last parameter, so the other instances keep their parameter layout.
+template <typename T, bool IDS, bool ADD>
 __global__ void prep16_from_images_kernel(PrepSource s0, PrepSource s1, PrepSource s2, int nsrc, int plr, int blr, int P,
                                           Tiling tl, int first_patch, const int* __restrict__ ids, long long total,
-                                          float divisor, __half* __restrict__ out_hi, __half* __restrict__ out_lo) {
+                                          float divisor, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
+                                          float add_offset) {
   const int PP = P * P;
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
@@ -124,9 +134,9 @@ __global__ void prep16_from_images_kernel(PrepSource s0, PrepSource s1, PrepSour
       const int ti = patch / tl.n_j, tj = patch - ti * tl.n_j;
       const int si = ti < tl.k_i ? ti * tl.stride : tl.last_i;
       const int sj = tj < tl.k_j ? tj * tl.stride : tl.last_j;
-      prep_gather<T, 4, 0>(s0, si, sj, plr, blr, y, x, divisor, v);     // 10 m bands   (DSen2Net.py:24,26 order)
-      prep_gather<T, 6, 4>(s1, si, sj, plr, blr, y, x, divisor, v);     // 20 m bands
-      if (nsrc == 3) prep_gather<T, 2, 10>(s2, si, sj, plr, blr, y, x, divisor, v);   // 60 m bands
+      prep_gather<T, 4, 0, ADD>(s0, si, sj, plr, blr, y, x, divisor, add_offset, v);     // 10 m bands   (DSen2Net.py:24,26 order)
+      prep_gather<T, 6, 4, ADD>(s1, si, sj, plr, blr, y, x, divisor, add_offset, v);     // 20 m bands
+      if (nsrc == 3) prep_gather<T, 2, 10, ADD>(s2, si, sj, plr, blr, y, x, divisor, add_offset, v);   // 60 m bands
     }
     Half16 hi, lo;
     split16(v, hi, lo);
@@ -322,10 +332,21 @@ extern "C" int dsen2_prep16_from_patches(const float* d_x0, int c0, const float*
   return check_launch("prep16_from_patches");
 }
 
+template <typename T, bool IDS, bool ADD>
+static void launch_prep16(PrepSource s0, PrepSource s1, PrepSource s2, int nsrc, int plr, int blr, int P, Tiling tl,
+                          int first_patch, const int* d_patch_ids, long long total, float divisor, float add_offset,
+                          void* d_xin_hi, void* d_xin_lo, cudaStream_t stream) {
+  const int block = 256;
+  prep16_from_images_kernel<T, IDS, ADD><<<grid_for(total, block), block, 0, stream>>>(
+      s0, s1, s2, nsrc, plr, blr, P, tl, first_patch, d_patch_ids, total, divisor, (__half*)d_xin_hi, (__half*)d_xin_lo,
+      add_offset);
+}
+
+// add: run the ADD instances with add_offset (finite; checked by the caller)
 template <bool IDS>
 static int prep16_from_images(const char* name, const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype,
                               int H, int W, int patch, int border, int first_patch, const int* d_patch_ids, int num_patches,
-                              float divisor, void* d_xin_hi, void* d_xin_lo, void* stream) {
+                              float divisor, bool add, float add_offset, void* d_xin_hi, void* d_xin_lo, void* stream) {
   DSEN2_REQUIRE(d_img10 && d_img20 && d_xin_hi && d_xin_lo && (!IDS || d_patch_ids), DSEN2_E_BADARG, "%s: null pointer", name);
   DSEN2_REQUIRE(img_dtype == DSEN2_IMG_F32 || img_dtype == DSEN2_IMG_U16, DSEN2_E_BADARG,
                 "%s: img_dtype must be DSEN2_IMG_F32 or DSEN2_IMG_U16 (got %d)", name, img_dtype);
@@ -350,15 +371,19 @@ static int prep16_from_images(const char* name, const void* d_img10, const void*
   PrepSource s1{d_img20, H / 2, W / 2, r / 2, 2};
   PrepSource s2{d_img60, H / 6, W / 6, 1, 6};
   const long long total = (long long)num_patches * patch * patch;
-  const int block = 256;
-  if (img_dtype == DSEN2_IMG_U16)
-    prep16_from_images_kernel<uint16_t, IDS><<<grid_for(total, block), block, 0, (cudaStream_t)stream>>>(
-        s0, s1, s2, d_img60 ? 3 : 2, plr, blr, patch, tl, first_patch, d_patch_ids, total, divisor, (__half*)d_xin_hi,
-        (__half*)d_xin_lo);
-  else
-    prep16_from_images_kernel<float, IDS><<<grid_for(total, block), block, 0, (cudaStream_t)stream>>>(
-        s0, s1, s2, d_img60 ? 3 : 2, plr, blr, patch, tl, first_patch, d_patch_ids, total, divisor, (__half*)d_xin_hi,
-        (__half*)d_xin_lo);
+  const int nsrc = d_img60 ? 3 : 2;
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (img_dtype == DSEN2_IMG_U16) {
+    if (add) launch_prep16<uint16_t, IDS, true>(s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
+                                                divisor, add_offset, d_xin_hi, d_xin_lo, st);
+    else launch_prep16<uint16_t, IDS, false>(s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
+                                             divisor, 0.f, d_xin_hi, d_xin_lo, st);
+  } else {
+    if (add) launch_prep16<float, IDS, true>(s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
+                                             divisor, add_offset, d_xin_hi, d_xin_lo, st);
+    else launch_prep16<float, IDS, false>(s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
+                                          divisor, 0.f, d_xin_hi, d_xin_lo, st);
+  }
   return check_launch(name);
 }
 
@@ -366,14 +391,27 @@ extern "C" int dsen2_prep16_from_images(const void* d_img10, const void* d_img20
                                         int W, int patch, int border, int first_patch, int num_patches, float divisor,
                                         void* d_xin_hi, void* d_xin_lo, void* stream) {
   return prep16_from_images<false>("dsen2_prep16_from_images", d_img10, d_img20, d_img60, img_dtype, H, W, patch, border,
-                                   first_patch, nullptr, num_patches, divisor, d_xin_hi, d_xin_lo, stream);
+                                   first_patch, nullptr, num_patches, divisor, false, 0.f, d_xin_hi, d_xin_lo, stream);
 }
 
 extern "C" int dsen2_prep16_from_images_ids(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype,
                                             int H, int W, int patch, int border, const int* d_patch_ids, int num_patches,
                                             float divisor, void* d_xin_hi, void* d_xin_lo, void* stream) {
   return prep16_from_images<true>("dsen2_prep16_from_images_ids", d_img10, d_img20, d_img60, img_dtype, H, W, patch, border,
-                                  0, d_patch_ids, num_patches, divisor, d_xin_hi, d_xin_lo, stream);
+                                  0, d_patch_ids, num_patches, divisor, false, 0.f, d_xin_hi, d_xin_lo, stream);
+}
+
+extern "C" int dsen2_prep16_from_images_offset(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype,
+                                               int H, int W, int patch, int border, int first_patch, const int* d_patch_ids,
+                                               int num_patches, float divisor, float add_offset, void* d_xin_hi,
+                                               void* d_xin_lo, void* stream) {
+  const char* name = "dsen2_prep16_from_images_offset";
+  DSEN2_REQUIRE(isfinite(add_offset), DSEN2_E_BADARG, "%s: add_offset must be finite", name);
+  if (d_patch_ids)
+    return prep16_from_images<true>(name, d_img10, d_img20, d_img60, img_dtype, H, W, patch, border, 0, d_patch_ids,
+                                    num_patches, divisor, true, add_offset, d_xin_hi, d_xin_lo, stream);
+  return prep16_from_images<false>(name, d_img10, d_img20, d_img60, img_dtype, H, W, patch, border, first_patch, nullptr,
+                                   num_patches, divisor, true, add_offset, d_xin_hi, d_xin_lo, stream);
 }
 
 extern "C" int dsen2_pack_head16_weights(const float* d_hwio, int cin, int feature_size, void* d_packed, void* stream) {

@@ -14,15 +14,19 @@ part of this image, so the script is split here into
 
     python -m dsen2_b200.s2_tiles_supres <data_file> [output_file] [--roi_x_y x1,y1,x2,y2] [--run_60]
                                          [--copy_original_bands] [--output_file_format npz|GTiff|ENVI ...]
-                                         [--nodata VALUE] [--output_dtype float64|uint16]
+                                         [--nodata VALUE] [--output_dtype float64|uint16] [--add_offset VALUE]
 
 ``--nodata`` is an extension of the reference's options: pixels whose every input band holds VALUE (0 outside the footprint
 of a partly covered granule) stay VALUE in the output, which records VALUE as its nodata value.  ``--output_dtype uint16``
 (another extension) writes the super-resolved bands as uint16 digital numbers, the input's own format, rounded and saturated
 on the GPU (``supres.DSen2_20(out_dtype=)``); VALUE must then be a uint16 value.  The default ``float64`` is the reference's
-output.
+output.  ``--add_offset VALUE`` (an extension) is the radiometric offset of the product, as its metadata states it
+(RADIO_ADD_OFFSET / BOA_ADD_OFFSET: -1000 for processing baseline 04.00 and later): it is added to the inputs before the
+network and subtracted from its output on the GPU (``supres.DSen2_20(add_offset=)``), so the super-resolved bands are in the
+product's own convention, like the bands ``--copy_original_bands`` copies.  ``--nodata`` stays the value the product stores.
 """
 import argparse
+import math
 import os
 import re
 import sys
@@ -139,16 +143,18 @@ def read_windows(xmin, ymin, xmax, ymax):
 # super-resolution chaining and output assembly (s2_tiles_supres.py:332-342, 385-416)
 # ---------------------------------------------------------------------------------------------- #
 def super_resolve(data10, data20, data60, names10, names20, names60, deep=False, models=None, nodata=None,
-                  out_dtype=None):
+                  out_dtype=None, add_offset=None):
     """The 60 m bands first, then the 20 m bands; returns (sr (H, W, n20 [+ n60]) or None, short names of its bands).
     ``models`` (extension): {'20': S2Model, '60': S2Model} instead of the shipped weight files; ``nodata`` (extension):
     the nodata value of both calls (``supres.DSen2_20``); ``out_dtype`` (extension): their output type (float32 if None,
-    or np.uint16)."""
+    or np.uint16); ``add_offset`` (extension): the product's radiometric offset, for both calls."""
     from . import supres
     models = models or {}
     extra = {} if nodata is None else {'nodata': nodata}
     if out_dtype is not None:
         extra['out_dtype'] = out_dtype
+    if add_offset is not None:
+        extra['add_offset'] = add_offset
     sr60 = None
     if names60 and names20 and names10:
         print("Super-resolving the 60m data into 10m bands")
@@ -184,13 +190,11 @@ def shift_geotransform(geotransform, xmin, ymin):
     return tuple(geot)
 
 
-def save_npz(output_file, bands, nodata=None):
-    """``np.savez(output_file, bands=bands)`` with bands = {description: array} (:419-420); with ``nodata`` also a
-    ``nodata`` entry holding the value."""
-    if nodata is None:
-        np.savez(output_file, bands=dict(bands))
-    else:
-        np.savez(output_file, bands=dict(bands), nodata=np.float64(nodata))
+def save_npz(output_file, bands, nodata=None, add_offset=None):
+    """``np.savez(output_file, bands=bands)`` with bands = {description: array} (:419-420); with ``nodata`` / ``add_offset``
+    also a ``nodata`` / ``add_offset`` entry holding the value."""
+    extra = {name: np.float64(v) for name, v in (('nodata', nodata), ('add_offset', add_offset)) if v is not None}
+    np.savez(output_file, bands=dict(bands), **extra)
 
 
 # ---------------------------------------------------------------------------------------------- #
@@ -319,6 +323,11 @@ def build_parser():
     p.add_argument("--output_dtype", choices=("float64", "uint16"), default="float64",
                    help="Extension: data type of the written bands.  uint16: digital numbers like the input, rounded and "
                         "clipped to [0, 65535] on the GPU; a computed value equal to --nodata is moved one step off it.")
+    p.add_argument("--add_offset", type=float, default=None, metavar="VALUE",
+                   help="Extension: radiometric offset of the product, as RADIO_ADD_OFFSET (L1C) / BOA_ADD_OFFSET (L2A) in "
+                        "its metadata.  Products of processing baseline 04.00 and later (from 25 January 2022, and the "
+                        "reprocessed archive) want --add_offset -1000.  It is added to the inputs before the network and "
+                        "subtracted from the output on the GPU; the output stays in the product's convention.")
     return p
 
 
@@ -329,6 +338,8 @@ def parse_args(argv=None):
             not (args.nodata.is_integer() and 0 <= args.nodata <= 65535):
         parser.error("--nodata %r is not a uint16 value (an integer in [0, 65535]), as --output_dtype uint16 needs"
                      % args.nodata)
+    if args.add_offset is not None and not math.isfinite(args.add_offset):
+        parser.error("--add_offset %r is not a finite number" % args.add_offset)
     return args
 
 
@@ -382,7 +393,7 @@ def main(argv=None, models=None):
     data60 = ds.read(2, w60, i60) if i60 else None
     u16 = args.output_dtype == "uint16"
     sr, sr_names = super_resolve(data10, data20, data60, n10, n20, n60, models=models, nodata=args.nodata,
-                                 out_dtype=np.uint16 if u16 else None)
+                                 out_dtype=np.uint16 if u16 else None, add_offset=args.add_offset)
     if sr is None:
         print("No super-resolution performed, exiting")
         return 0
@@ -405,7 +416,7 @@ def main(argv=None, models=None):
                                                           output_file))
     geot = shift_geotransform(ds.geotransform, xmin, ymin)
     if fmt == "npz":
-        save_npz(output_file, bands, args.nodata)
+        save_npz(output_file, bands, args.nodata, args.add_offset)
     else:  # pragma: no cover - needs osgeo
         from osgeo import gdal
         result = driver.Create(output_file, data10.shape[1], data10.shape[0], len(bands),

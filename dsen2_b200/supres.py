@@ -14,7 +14,15 @@ Digital-number output (an extension): with ``out_dtype=uint16`` the last layer r
 device and writes a uint16 canvas: NaN becomes 0, every other value is rint(clip(f, 0, 65535)) (half to even) of the float f
 the float32 output holds.  With ``nodata=v`` as well, nodata pixels are v, and a valid value that would round to v is
 written as v + 1 (65534 for v = 65535), so no computed value reads as nodata.
+
+Radiometric offset (an extension): in Sentinel-2 products of processing baseline 04.00 and later, reflectance is
+(DN + add_offset) / 10000, with the add_offset of their metadata (RADIO_ADD_OFFSET / BOA_ADD_OFFSET, -1000); the network
+expects DN = 10000 x reflectance.  With ``add_offset=a`` every band value x of the input images, as held on the device
+(uint16, or float32 as staged), becomes fl32(x + a) before the preparation, and every output value f becomes fl32(f - a):
+the output is in the product's own convention (quantised after that for uint16 output).  Nodata is still decided on the
+stored values, and nodata pixels are written as the stored v.
 """
+
 import math
 import os
 
@@ -80,6 +88,24 @@ def check_nodata(nodata, model, uint16_images):
     return v
 
 
+def check_add_offset(add_offset, model):
+    """The ``add_offset`` argument as the float32 value the kernels use, as a Python float (None stays None).  Rejected with
+    ``ValueError``: anything but a real number, a value that is not finite in float32, and a network without resBlocks (its
+    separate extract / network / recompose kernels take no offset; ``model`` None: not checked)."""
+    if add_offset is None:
+        return None
+    a = np.asarray(add_offset)
+    if a.ndim != 0 or a.dtype.kind not in 'iuf':
+        raise ValueError("add_offset must be a number, got %r" % (add_offset,))
+    with np.errstate(over='ignore'):
+        v = np.float32(a)
+    if not np.isfinite(v):
+        raise ValueError("add_offset %r is not a finite float32 value" % (add_offset,))
+    if model is not None and not model.xin16:
+        raise ValueError("add_offset needs a network with resBlocks (num_layers > 0)")
+    return float(v)
+
+
 _OUT_DTYPES = {'float32': False, 'uint16': True}
 
 
@@ -142,10 +168,12 @@ def _scan_active(d10, d20, d60, first_patch, num_patches, nodata, ids, count, co
     return ev
 
 
-def _run_active(model, d10, d20, d60, first_patch, num_patches, nodata, ids, out, device_batch, timers=None):
+def _run_active(model, d10, d20, d60, first_patch, num_patches, nodata, ids, out, device_batch, timers=None,
+                add_offset=None):
     """The network over the active patches ``ids`` (batches of at most ``device_batch``), then nodata into the nodata
     pixels the range owns -- after the last layer, which also stitches active patches' values over their nodata pixels.
-    A uint16 ``out`` gets network values moved off v (``avoid``) and the uint16 fill."""
+    A uint16 ``out`` gets network values moved off v (``avoid``) and the uint16 fill.  The fill writes v as it is: the
+    offset applies to network values only."""
     torch = _capi.require_cuda()
     g = _GEOM[d60 is not None]
     u16 = out.dtype == torch.uint16
@@ -153,7 +181,7 @@ def _run_active(model, d10, d20, d60, first_patch, num_patches, nodata, ids, out
     for i in range(0, int(ids.shape[0]), device_batch):
         batch = ids[i:i + device_batch]
         model.forward_images(d10, d20, d60, g['patch'], g['border'], 0, int(batch.shape[0]), out, float(SCALE),
-                             timers=timers, patch_ids=batch, avoid=avoid)
+                             timers=timers, patch_ids=batch, avoid=avoid, add_offset=add_offset)
     imgs, v = _nodata_args(d10, d20, d60, nodata)
     name = 'dsen2_nodata_fill_u16' if u16 else 'dsen2_nodata_fill'
     fill = getattr(_capi.lib(), name)
@@ -196,13 +224,14 @@ def active_patches(d10, d20, d60=None, nodata=0, first_patch=0, num_patches=None
 
 
 def super_resolve_device(model, d10, d20, d60=None, first_patch=0, num_patches=None, out=None, device_batch=None,
-                         timers=None, nodata=None, out_dtype=None):
+                         timers=None, nodata=None, out_dtype=None, add_offset=None):
     """Device-level pipeline.  d10/d20(/d60): CUDA HWC tensors, all float32 or all uint16.  Processes patches
     [first_patch, first_patch+num_patches) of the FILLED patch list (surplus zero patches of
     patches.py:32-39 are never read by recompose_images, so they are skipped) and writes the pixels those
     patches own into ``out`` (H, W, Cout) of ``out_dtype`` (torch.float32 when None, or torch.uint16: see the module
     docstring; allocated zero-filled if None).  ``nodata``: see the module docstring; the active patches are found on
-    the device, and their number is the one value read back."""
+    the device, and their number is the one value read back.  ``add_offset``: see the module docstring."""
+    add_offset = check_add_offset(add_offset, model)
     torch = _capi.require_cuda()
     u16 = check_out_dtype(out_dtype, model)
     nodata = check_nodata(nodata, model, d10.dtype == torch.uint16 or u16)
@@ -223,12 +252,12 @@ def super_resolve_device(model, d10, d20, d60=None, first_patch=0, num_patches=N
     # (and dsen2_prep16_from_images rejects); every image that reaches this point is stitched and cropped.
     if nodata is not None:
         ids = _active(d10, d20, d60, first_patch, num_patches, nodata, timers)
-        _run_active(model, d10, d20, d60, first_patch, num_patches, nodata, ids, out, device_batch, timers)
+        _run_active(model, d10, d20, d60, first_patch, num_patches, nodata, ids, out, device_batch, timers, add_offset)
         return out
     for p0 in range(first_patch, first_patch + num_patches, device_batch):
         nb = min(device_batch, first_patch + num_patches - p0)
         if model.xin16:                          # fused: images -> x_in16 -> network -> stitched canvas
-            model.forward_images(d10, d20, d60, P, B, p0, nb, out, float(SCALE), timers=timers)
+            model.forward_images(d10, d20, d60, P, B, p0, nb, out, float(SCALE), timers=timers, add_offset=add_offset)
             continue
         # a network without resblocks: separate extract / bilinear / network / stitch kernels
         if run_60:
@@ -319,23 +348,27 @@ class HostPipeline:
         count = torch.empty((chunks,), dtype=torch.int32, device=self.dev)
         return nodata, ids, count, torch.empty((chunks,), dtype=torch.int32).pin_memory()
 
-    def _compute(self, k, p0, cnt, first_patch, nodata, ids, count_host, ev_scan, timers):
+    def _compute(self, k, p0, cnt, first_patch, nodata, ids, count_host, ev_scan, timers, add_offset):
         """Chunk k's network on the current stream (its inputs are resident): the whole range, or -- with ``nodata`` --
         the active patches its scan found, then the nodata fill."""
         if nodata is None:
             super_resolve_device(self.model, self.d10, self.d20, self.d60, first_patch=p0, num_patches=cnt,
-                                 out=self.canvas, device_batch=self.device_batch, timers=timers, out_dtype=self.out_dtype)
+                                 out=self.canvas, device_batch=self.device_batch, timers=timers, out_dtype=self.out_dtype,
+                                 add_offset=add_offset)
             return
         ev_scan.synchronize()                        # this chunk's upload and scan only, never an earlier network
         batch = self.device_batch or default_device_batch(self.W, self.P, self.B)
         a = p0 - first_patch
         _run_active(self.model, self.d10, self.d20, self.d60, p0, cnt, nodata, ids[a:a + int(count_host[k])], self.canvas,
-                    batch, timers)
+                    batch, timers, add_offset)
 
-    def run(self, h10, h20, h60=None, hout=None, first_patch=0, num_patches=None, timers=None, nodata=None):
+    def run(self, h10, h20, h60=None, hout=None, first_patch=0, num_patches=None, timers=None, nodata=None,
+            add_offset=None):
         """Pinned torch tensors in (dtype = the pipeline's), pinned (H, W, Cout) tensor of ``out_dtype`` out.  Rows of
         ``hout`` that the patch range owns only partly (the seam rows of a sharded range) are downloaded whole.  ``nodata``: see the
-        module docstring; each chunk's patch scan runs on the upload stream right behind its upload."""
+        module docstring; each chunk's patch scan runs on the upload stream right behind its upload.  ``add_offset``: see
+        the module docstring."""
+        add_offset = check_add_offset(add_offset, self.model)
         torch = self.torch
         filled = self.ny * self.nx
         if num_patches is None:
@@ -367,7 +400,7 @@ class HostPipeline:
                 ev_up = torch.cuda.Event()
                 ev_up.record(self.up)
             main.wait_event(ev_up)
-            self._compute(k, p0, cnt, first_patch, nodata, ids, count_host, ev_scan, timers)
+            self._compute(k, p0, cnt, first_patch, nodata, ids, count_host, ev_scan, timers, add_offset)
             ev_c = torch.cuda.Event()
             ev_c.record(main)
             self.down.wait_event(ev_c)
@@ -409,9 +442,12 @@ class HostPipeline:
                                             initializer=torch.cuda.set_device, initargs=(self.dev,))
         return self._slots
 
-    def run_numpy(self, a10, a20, a60=None, out=None, first_patch=0, num_patches=None, timers=None, nodata=None):
+    def run_numpy(self, a10, a20, a60=None, out=None, first_patch=0, num_patches=None, timers=None, nodata=None,
+                  add_offset=None):
         """Pageable numpy arrays in -> numpy (H, W, Cout) array of ``out_dtype`` out (allocated if None).  Arrays whose
-        dtype is not the pipeline's are cast while they are staged.  ``nodata`` as in ``run``."""
+        dtype is not the pipeline's are cast while they are staged (the offset applies to the staged values).  ``nodata``
+        and ``add_offset`` as in ``run``."""
+        add_offset = check_add_offset(add_offset, self.model)
         torch = self.torch
         filled = self.ny * self.nx
         if num_patches is None:
@@ -479,7 +515,7 @@ class HostPipeline:
             main.wait_event(slot.ev_h2d)
             if k + self.RING < len(plan):
                 fin[k + self.RING] = self._pool.submit(stage_in, k + self.RING)
-            self._compute(k, p0, cnt, first_patch, nodata, ids, count_host, ev_scan, timers)
+            self._compute(k, p0, cnt, first_patch, nodata, ids, count_host, ev_scan, timers, add_offset)
             ev_c = torch.cuda.Event()
             ev_c.record(main)
             self.down.wait_event(ev_c)
@@ -525,9 +561,10 @@ def _pipeline_for(model, H, W, run_60, dtype, out_dtype):
     return pipe
 
 
-def _run(model, arrays, out=None, nodata=None, out_dtype=np.float32):
+def _run(model, arrays, out=None, nodata=None, out_dtype=np.float32, add_offset=None):
     # rejected before the device is touched
     u16 = check_out_dtype(out_dtype, model)
+    add_offset = check_add_offset(add_offset, model)
     if nodata is not None:
         nodata = check_nodata(nodata, model,
                               u16 or (model.xin16 and all(np.asarray(a).dtype == np.uint16 for a in arrays)))
@@ -546,25 +583,27 @@ def _run(model, arrays, out=None, nodata=None, out_dtype=np.float32):
     # else is staged as float32 (the reference divides by SCALE in floating point whatever the input type, supres.py:23-24)
     dtype = torch.uint16 if (model.xin16 and all(a.dtype == np.uint16 for a in arrays)) else torch.float32
     pipe = _pipeline_for(model, H, W, len(arrays) == 3, dtype, torch.uint16 if u16 else torch.float32)
-    res = pipe.run_numpy(*arrays, out=out, nodata=nodata)
+    res = pipe.run_numpy(*arrays, out=out, nodata=nodata, add_offset=add_offset)
     torch.cuda.current_stream().synchronize()
     return res
 
 
-def DSen2_20(d10, d20, deep=False, model=None, out=None, nodata=None, out_dtype=np.float32):
+def DSen2_20(d10, d20, deep=False, model=None, out=None, nodata=None, out_dtype=np.float32, add_offset=None):
     """supres.py:15-30.  d10 (H,W,4), d20 (H/2,W/2,6) -> (H,W,6) float32.  Extensions: ``model`` supplies a preloaded
     ``S2Model`` instead of the shipped hdf5 weights, ``out`` a preallocated (H,W,6) array of ``out_dtype`` to fill,
     ``nodata`` the input value of pixels without data (module docstring): they come out as ``nodata`` and empty patches are
-    skipped; ``out_dtype`` np.uint16: digital numbers, rounded and saturated on the device (module docstring)."""
+    skipped; ``out_dtype`` np.uint16: digital numbers, rounded and saturated on the device (module docstring);
+    ``add_offset`` the radiometric offset of the product (-1000 for processing baseline 04.00 and later; module docstring):
+    removed from the inputs and restored on the output, on the device."""
     input_shape = ((4, None, None), (6, None, None))
     if model is None:
         model = _load_model(input_shape, deep, run_60=False)
-    return _run(model, [d10, d20], out, nodata, out_dtype)
+    return _run(model, [d10, d20], out, nodata, out_dtype, add_offset)
 
 
-def DSen2_60(d10, d20, d60, deep=False, model=None, out=None, nodata=None, out_dtype=np.float32):
+def DSen2_60(d10, d20, d60, deep=False, model=None, out=None, nodata=None, out_dtype=np.float32, add_offset=None):
     """supres.py:33-50.  + d60 (H/6,W/6,2) -> (H,W,2) float32 (or ``out_dtype``)."""
     input_shape = ((4, None, None), (6, None, None), (2, None, None))
     if model is None:
         model = _load_model(input_shape, deep, run_60=True)
-    return _run(model, [d10, d20, d60], out, nodata, out_dtype)
+    return _run(model, [d10, d20, d60], out, nodata, out_dtype, add_offset)

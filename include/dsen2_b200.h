@@ -242,6 +242,26 @@ int dsen2_conv_tail16_stitch_ids_u16(const void* d_x_hi, const void* d_x_lo, con
                                      int n, int P, const int* d_patch_ids, int border, int img_h, int img_w, float mul,
                                      int avoid, uint16_t* d_canvas, void* stream);
 
+/* Radiometric offset (an extension: Sentinel-2 products of processing baseline 04.00 and later store
+ * DN = 10000 * reflectance - add_offset, with add_offset = RADIO_ADD_OFFSET / BOA_ADD_OFFSET = -1000 in their metadata, while
+ * the network expects DN = 10000 * reflectance).  The two steps above with a finite `add_offset` (anything else:
+ * DSEN2_E_BADARG):
+ *   dsen2_prep16_from_images_offset: every band value x of the images, as stored (uint16 or float32), becomes
+ *       fl32(x + add_offset) before any other arithmetic of the preparation (the bilinear round trip, the / divisor).
+ *   dsen2_conv_tail16_stitch_offset: with f the float the stitching entry writes for those inputs, the canvas receives
+ *       fl32(f - add_offset) -- the output is in the convention of the input product -- or, for a uint16 canvas, the
+ *       digital number of that value as dsen2_conv_tail16_stitch_u16 computes it.
+ * Both take the range form and the list form: d_patch_ids == NULL: patches [first_patch, first_patch + num_patches); else
+ * the listed ids (first_patch ignored).  The nodata entry points take the stored values: v is the value the product holds. */
+int dsen2_prep16_from_images_offset(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int H, int W,
+                                    int patch, int border, int first_patch, const int* d_patch_ids, int num_patches,
+                                    float divisor, float add_offset, void* d_xin_hi, void* d_xin_lo, void* stream);
+/* canvas_dtype DSEN2_IMG_F32 / DSEN2_IMG_U16; avoid as dsen2_conv_tail16_stitch_u16 (-1 for a float canvas). */
+int dsen2_conv_tail16_stitch_offset(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                    const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
+                                    int n, int P, int first_patch, const int* d_patch_ids, int border, int img_h, int img_w,
+                                    float mul, float add_offset, int canvas_dtype, int avoid, void* d_canvas, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Nodata (csrc/nodata.cu; an extension: the reference super-resolves nodata like data).  Images, img_dtype, H, W, patch
  * and border as dsen2_prep16_from_images (d_img60 == NULL: 20 m path); `nodata` is the fill value v (not NaN).  Output pixel

@@ -91,6 +91,11 @@ __global__ void extract_patches_generic_kernel(const float* __restrict__ img, in
 // ------------------------------------------------------------------------------------------ //
 // bilinear, mirror boundary, integer scale s (patches.py:11-16): u = (o + .5)/s - .5
 // ------------------------------------------------------------------------------------------ //
+// a * (1 - f) + b * f as every bilinear kernel here (and prep_gather) evaluates it: the first product fused into the sum,
+// the second rounded.  Spelled out so that the compiler cannot contract the expression differently in each kernel: the
+// kernels below must give the same bits for the same plane.
+__device__ __forceinline__ float lerp_rn(float a, float b, float f) { return __fmaf_rn(a, 1.0f - f, __fmul_rn(b, f)); }
+
 __global__ void bilinear_mirror_kernel(const float* __restrict__ in, int p, int s, long long total, float post_div,
                                        float* __restrict__ out) {
   const int P = p * s;
@@ -104,13 +109,14 @@ __global__ void bilinear_mirror_kernel(const float* __restrict__ in, int p, int 
     float fy, fx;
     bilin_tap(oy, s, p, y0, y1, fy);
     bilin_tap(ox, s, p, x0, x1, fx);
+    if (p == 1) y0 = x0 = 0;                 // bilin_tap mirrors the tap -1 to 1, which a one-pixel plane does not have
     const float* src = in + plane * (long long)p * p;
     const float k = 30000.0f;                // the reference scales by 1/30000 around the resize
     const float v00 = __fdiv_rn(__ldg(src + y0 * p + x0), k), v01 = __fdiv_rn(__ldg(src + y0 * p + x1), k);
     const float v10 = __fdiv_rn(__ldg(src + y1 * p + x0), k), v11 = __fdiv_rn(__ldg(src + y1 * p + x1), k);
-    const float c0 = v00 * (1.0f - fy) + v10 * fy;   // rows first, then columns (as the oracle)
-    const float c1 = v01 * (1.0f - fy) + v11 * fy;
-    const float r = (c0 * (1.0f - fx) + c1 * fx) * k;
+    const float c0 = lerp_rn(v00, v10, fy);  // rows first, then columns (as the oracle)
+    const float c1 = lerp_rn(v01, v11, fy);
+    const float r = __fmul_rn(lerp_rn(c0, c1, fx), k);
     out[idx] = (post_div == 1.0f) ? r : __fdiv_rn(r, post_div);
   }
 }
@@ -119,7 +125,7 @@ __global__ void bilinear_mirror_kernel(const float* __restrict__ in, int p, int 
 // on each side), divides every input value by 30000 ONCE into shared memory (the direct kernel does it four times per
 // output) and produces the s * kBilRows output rows from there.  A thread owns FOUR consecutive output columns (their x
 // taps are computed once, the row is written with 16-byte stores; blockDim.x = P / 4) and walks the band's output rows.
-// Same operations per output as bilinear_mirror_kernel => same bits.
+// Same operations per output as bilinear_mirror_kernel (lerp_rn) => same bits.
 constexpr int kBilRows = 16, kBilThreads = 256, kBilMaxP = 1024;
 
 __device__ __forceinline__ int mirror_index(int g, int n) {
@@ -174,9 +180,9 @@ __global__ void __launch_bounds__(kBilThreads) bilinear_mirror_band_kernel(const
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const float v00 = row0[xl[j]], v01 = row0[xl[j] + 1], v10 = row1[xl[j]], v11 = row1[xl[j] + 1];
-      const float c0 = v00 * (1.0f - fy) + v10 * fy;   // rows first, then columns (as the oracle)
-      const float c1 = v01 * (1.0f - fy) + v11 * fy;
-      const float v = (c0 * (1.0f - fx[j]) + c1 * fx[j]) * k;
+      const float c0 = lerp_rn(v00, v10, fy);          // rows first, then columns (as the oracle)
+      const float c1 = lerp_rn(v01, v11, fy);
+      const float v = __fmul_rn(lerp_rn(c0, c1, fx[j]), k);
       r[j] = (post_div == 1.0f) ? v : __fdiv_rn(v, post_div);
     }
     *reinterpret_cast<float4*>(dst + (long long)oy * P) = make_float4(r[0], r[1], r[2], r[3]);
@@ -218,11 +224,11 @@ __global__ void __launch_bounds__(256) bilinear_mirror_x2_p64_kernel(const float
       const float fy = h ? 0.75f : 0.25f;
       float c[4], o[4];
 #pragma unroll
-      for (int j = 0; j < 4; ++j) c[j] = top[j] * (1.0f - fy) + bot[j] * fy;      // rows first, then columns
-      o[0] = (c[0] * (1.0f - 0.75f) + c[1] * 0.75f) * k;
-      o[1] = (c[1] * (1.0f - 0.25f) + c[2] * 0.25f) * k;
-      o[2] = (c[1] * (1.0f - 0.75f) + c[2] * 0.75f) * k;
-      o[3] = (c[2] * (1.0f - 0.25f) + c[3] * 0.25f) * k;
+      for (int j = 0; j < 4; ++j) c[j] = lerp_rn(top[j], bot[j], fy);      // rows first, then columns
+      o[0] = __fmul_rn(lerp_rn(c[0], c[1], 0.75f), k);
+      o[1] = __fmul_rn(lerp_rn(c[1], c[2], 0.25f), k);
+      o[2] = __fmul_rn(lerp_rn(c[1], c[2], 0.75f), k);
+      o[3] = __fmul_rn(lerp_rn(c[2], c[3], 0.25f), k);
       if (post_div != 1.0f) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) o[j] = __fdiv_rn(o[j], post_div);

@@ -13,6 +13,7 @@ power-of-two loss scale so that the MAE gradient sign(pred-y)/N enters the fp16 
 Master weights, gradients and the Nadam moments are fp32.  DSen2 (feature_size 128) and VDSen2 (256; ``--deep``,
 ``supres_train.py:129-131``: the 256-channel layers stream their weights, weight gradients run per 128 x 128 block).
 """
+import gc
 import math
 import os
 
@@ -285,21 +286,31 @@ class Trainer:
             overlap = multi and self._overlap_allreduce(n, P)
             if key not in self._graphs:
                 # one graph on a single GPU; with several ranks the NCCL all-reduce stays an eager call between
-                # "gradient" graphs and an "update" graph (a collective inside the capture deadlocked in testing)
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g):
-                    loss, mse = self._step_body(b['in_x'], b['in_y'], not multi, dev_hp=True, part='a' if overlap else None)
-                    self.loss_out[0].copy_(loss)
-                    self.loss_out[1].copy_(mse)
-                gb = g2 = None
-                if overlap:
-                    gb = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(gb):
-                        self._step_body(b['in_x'], b['in_y'], False, part='b')
-                if multi:
-                    g2 = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g2):
-                        self._update_dev()
+                # "gradient" graphs and an "update" graph (a collective inside the capture deadlocked in testing).
+                # The cyclic garbage collector stays off while capturing: a dropped model and its trainer form a cycle, and
+                # collecting it there would destroy that trainer's graphs, which a capturing stream does not permit (it
+                # invalidates this capture).
+                gc_was_enabled = gc.isenabled()
+                gc.disable()
+                try:
+                    g = torch.cuda.CUDAGraph()
+                    with torch.cuda.graph(g):
+                        loss, mse = self._step_body(b['in_x'], b['in_y'], not multi, dev_hp=True,
+                                                    part='a' if overlap else None)
+                        self.loss_out[0].copy_(loss)
+                        self.loss_out[1].copy_(mse)
+                    gb = g2 = None
+                    if overlap:
+                        gb = torch.cuda.CUDAGraph()
+                        with torch.cuda.graph(gb):
+                            self._step_body(b['in_x'], b['in_y'], False, part='b')
+                    if multi:
+                        g2 = torch.cuda.CUDAGraph()
+                        with torch.cuda.graph(g2):
+                            self._update_dev()
+                finally:
+                    if gc_was_enabled:
+                        gc.enable()
                 self._graphs[key] = (g, gb, g2)
             g, gb, g2 = self._graphs[key]
             g.replay()

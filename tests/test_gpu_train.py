@@ -333,6 +333,41 @@ def test_back_to_back_graph_steps_use_their_own_nadam_scalars(env):
     assert np.median(d) < 1e-3 and np.mean(d > 0.25) < 0.01     # fp32 atomics in the weight gradients: last-bit noise only
 
 
+def test_capture_while_a_dropped_trainer_awaits_collection(env):
+    """A dropped model and its trainer form a reference cycle that keeps the trainer's CUDA graph until the cyclic collector
+    runs.  Destroying a graph while another stream captures invalidates that capture, so the collector must not run
+    during a capture: with collections due on every allocation, another model still captures and replays its steps, the
+    collector is off inside the capture and on again afterwards, and the dropped trainer is collected after it."""
+    import gc
+    import weakref
+    torch, _capi, lib = env
+    from dsen2_b200.train import Nadam
+    model, ws, xs, y = _setup(L=1, n=4, P=32)
+    model.compile(optimizer=Nadam(lr=1e-3), loss='mean_absolute_error')
+    for _ in range(3):
+        model.train_on_batch(xs, y)                             # the second step captures the graph
+    assert model._trainer._graphs
+    dropped = weakref.ref(model._trainer)
+    del model
+    again = _setup(L=1, n=4, P=32)[0]
+    again.compile(optimizer=Nadam(lr=1e-3), loss='mean_absolute_error')
+    tr = again._trainer
+    collector_on = []
+    repack = tr.repack
+    tr.repack = lambda: (collector_on.append(gc.isenabled()), repack())[1]
+    threshold = gc.get_threshold()
+    gc.set_threshold(1, 1, 1)
+    try:
+        losses = [float(np.asarray(again.train_on_batch(xs, y)).ravel()[0]) for _ in range(3)]
+    finally:
+        gc.set_threshold(*threshold)
+    torch.cuda.synchronize()
+    assert tr._graphs and np.isfinite(losses).all()
+    assert collector_on[:2] == [True, False] and gc.isenabled()  # eager first step, then the capture
+    gc.collect()
+    assert dropped() is None
+
+
 def test_full_model_checkpoint_resumes_training(env, tmp_path):
     """model.save (ModelCheckpoint(save_weights_only=False), supres_train.py:195-201) carries the Nadam state: a model rebuilt
     from the file continues exactly like the one that kept training."""

@@ -9,6 +9,8 @@ import ctypes
 import numpy as np
 import pytest
 
+import tile_schedule as ts
+
 pytestmark = pytest.mark.gpu
 
 GATE = 5e-3
@@ -40,10 +42,12 @@ def _pack(torch, _capi, lib, w_hwio, cin_pad, cout_pad):
     return dst
 
 
-@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (1, 192, 192), (3, 40, 24), (1, 8, 200), (5, 16, 8)])
+@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (1, 192, 192), (3, 40, 24), (1, 8, 200), (5, 16, 8), ts.PATCH,
+                                   ts.RAGGED])
 @pytest.mark.parametrize('F', [128, 256])
 def test_conv_relu_layer(env, shape, F):
-    """First convolution of a resBlock (DSen2Net.py:10-11) for F = 128 (resident weights) and 256 (streamed weights)."""
+    """First convolution of a resBlock (DSen2Net.py:10-11) for F = 128 (resident weights) and 256 (streamed weights); the
+    ts.PATCH / ts.RAGGED cases run several tiles per CTA pair, as real runs do."""
     torch, _capi, lib = env
     n, H, W = shape
     rng = np.random.RandomState(H * 7 + W + F)
@@ -59,7 +63,9 @@ def test_conv_relu_layer(env, shape, F):
                                     _capi.stream_ptr()), 'conv relu')
     torch.cuda.synchronize()
     ref = np.maximum(_conv_ref(torch, x, w, bias), 0)
-    np.testing.assert_allclose(out.cpu().numpy().astype(np.float32), ref, rtol=2e-3, atol=2e-3)
+    got = out.cpu().numpy().astype(np.float32)
+    ts.check(ts.pair_schedule(n, H, W), 'conv_relu F=%d' % F, np.abs(got - ref).max())
+    np.testing.assert_allclose(got, ref, rtol=2e-3, atol=2e-3)
     assert lib.dsen2_conv_relu(_capi.ptr(tx), _capi.ptr(tw), _capi.ptr(tb), n, H, W, 192, _capi.ptr(out),
                                _capi.stream_ptr()) == -1                              # unsupported feature size is refused
 

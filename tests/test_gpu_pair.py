@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from cases import CASES20, CASES60, synth
+import tile_schedule as ts
 from qtrunk import NORMAL, q_decode as _q_decode, q_encode as _q_encode, q_from_tiles as _q_from_tiles, q_to_tiles as _q_to_tiles
 
 pytestmark = pytest.mark.gpu
@@ -126,7 +127,7 @@ def _conv64(x_nhwc, w_hwio, bias):
     return y.permute(0, 2, 3, 1).contiguous().numpy()
 
 
-@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (3, 40, 24), (1, 8, 200), (5, 16, 8)])
+@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (3, 40, 24), (1, 8, 200), (5, 16, 8), ts.PATCH])
 def test_conv_head_fp32_equivalent(env, shape):
     torch, _capi, lib = env
     n, H, W = shape
@@ -157,6 +158,7 @@ def test_conv_head_fp32_equivalent(env, shape):
     w_eff = w_hi.astype(np.float64) + (w - w_hi.astype(np.float32)).astype(np.float16).astype(np.float64)
     ref = np.maximum(_conv64(xin, w_eff, bias), 0)
     got = ohi.cpu().numpy().astype(np.float64) + olo.cpu().numpy().astype(np.float64)
+    ts.check(ts.pair_schedule(n, H, W), 'conv_head', np.abs(got - ref).max())
     np.testing.assert_allclose(got, ref, rtol=2e-5, atol=2e-5)
     assert np.abs(got - np.maximum(_conv64(xcat.transpose(0, 2, 3, 1), w, bias), 0)).max() < 5e-5   # vs true fp32 layer
     # fp32 trunk seed, tile-row-major (n, H, W/8, F/4, 8, 4): the same values before the hi/lo split
@@ -166,7 +168,7 @@ def test_conv_head_fp32_equivalent(env, shape):
 
 
 @pytest.mark.parametrize('shape,cout,ch0', [((2, 32, 32), 6, 4), ((1, 128, 128), 6, 4), ((1, 48, 48), 2, 10),
-                                            ((3, 40, 24), 6, 4)])
+                                            ((3, 40, 24), 6, 4), (ts.PATCH, 6, 4)])
 def test_conv_tail_nchw_fp32_equivalent(env, shape, cout, ch0):
     torch, _capi, lib = env
     n, H, W = shape
@@ -185,23 +187,38 @@ def test_conv_tail_nchw_fp32_equivalent(env, shape, cout, ch0):
     _capi.check(lib.dsen2_pack_tail_weights(_capi.ptr(torch.from_numpy(w).cuda()), F, cout, _capi.ptr(tw),
                                             _capi.stream_ptr()), 'pack tail')
     dev = [torch.from_numpy(a).cuda() for a in (x_hi, x_lo, xin_hi, xin_lo, bias)]
-    out = torch.full((n, cout, H, W), -5.0, device='cuda')
-    _capi.check(lib.dsen2_conv_tail(_capi.ptr(dev[0]), _capi.ptr(dev[1]), _capi.ptr(tw), _capi.ptr(dev[4]),
-                                    _capi.ptr(dev[2]), _capi.ptr(dev[3]), ch0, cout, n, H, W, _capi.ptr(out),
-                                    _capi.stream_ptr()), 'conv tail')
-    torch.cuda.synchronize()
+
+    def tail(b0, m):
+        out = torch.full((m, cout, H, W), -5.0, device='cuda')
+        _capi.check(lib.dsen2_conv_tail(_capi.ptr(dev[0][b0:]), _capi.ptr(dev[1][b0:]), _capi.ptr(tw), _capi.ptr(dev[4]),
+                                        _capi.ptr(dev[2][b0:]), _capi.ptr(dev[3][b0:]), ch0, cout, m, H, W, _capi.ptr(out),
+                                        _capi.stream_ptr()), 'conv tail')
+        torch.cuda.synchronize()
+        return out.cpu().numpy()
+    got = tail(0, n)
+    # a tile's result does not depend on which CTA computes it, or after which tiles: the batch equals one launch per
+    # patch (at most one tile per CTA) bit for bit
+    alone = np.concatenate([tail(b, 1) for b in range(n)])
+    assert np.array_equal(got.view(np.uint32), alone.view(np.uint32))
     xe = x_hi.astype(np.float64) + x_lo.astype(np.float64)
     w_hi = w.astype(np.float16)
     w_eff = w_hi.astype(np.float64) + (w - w_hi.astype(np.float32)).astype(np.float16).astype(np.float64)
     skip = (xin_hi.astype(np.float64) + xin_lo.astype(np.float64))[..., 16 + ch0:16 + ch0 + cout]
-    ref = (_conv64(xe, w_eff, bias[:cout]) + skip).transpose(0, 3, 1, 2)
-    np.testing.assert_allclose(out.cpu().numpy(), ref, rtol=2e-5, atol=2e-5)
+    conv = _conv64(xe, w_eff, bias[:cout])
+    ref = (conv + skip).transpose(0, 3, 1, 2)
+    ts.check(ts.pair_schedule(n, H, W), 'conv_tail cout=%d' % cout, np.abs(got - ref).max())
+    # relative to the magnitudes the fp32 arithmetic carries: where the skip cancels the convolution (|conv| ~ 4, sum ~ 0.05)
+    # the accumulation error of the convolution (~3e-5 at most) is all that is left
+    scale = (np.abs(conv) + np.abs(skip)).transpose(0, 3, 1, 2)
+    assert (np.abs(got - ref) <= 2e-5 + 2e-5 * scale).all(), np.abs(got - ref).max()
 
 
 @pytest.mark.parametrize('shape,cout,ch0,F', [((2, 32, 32), 6, 4, 128), ((1, 128, 128), 6, 4, 256), ((1, 48, 48), 2, 10, 256),
-                                              ((3, 40, 24), 6, 4, 256), ((1, 192, 192), 2, 10, 128)])
+                                              ((3, 40, 24), 6, 4, 256), ((1, 192, 192), 2, 10, 128), (ts.PATCH, 6, 4, 128),
+                                              (ts.PATCH, 6, 4, 256), (ts.PATCH, 7, 9, 128), (ts.RAGGED, 1, 15, 256)])
 def test_conv_tail16_nchw_fp32_equivalent(env, shape, cout, ch0, F):
-    """Last layer (F -> cout, split hi + lo operands) + global skip from the 16-channel prepared input, F = 128 / 256."""
+    """Last layer (F -> cout, split hi + lo operands) + global skip from the 16-channel prepared input, F = 128 / 256.
+    cout 7 (kTMaxCout: 126 of the 128 weight rows) with the skip reaching channel 15, and cout 1."""
     torch, _capi, lib = env
     n, H, W = shape
     rng = np.random.RandomState(H * 3 + cout + F)
@@ -226,7 +243,9 @@ def test_conv_tail16_nchw_fp32_equivalent(env, shape, cout, ch0, F):
     skip = (xin_hi.astype(np.float64) + xin_lo.astype(np.float64))[..., ch0:ch0 + cout]
     ref = (_conv64(xe, w_eff, bias[:cout]) + skip).transpose(0, 3, 1, 2)
     tol = 2e-5 if F == 128 else 6e-5          # fp32 accumulation order over K = 4 * 9 * F products
-    np.testing.assert_allclose(out.cpu().numpy(), ref, rtol=tol, atol=tol)
+    got = out.cpu().numpy()
+    ts.check(ts.tail_schedule(n, H, W), 'conv_tail16 F=%d cout=%d' % (F, cout), np.abs(got - ref).max())
+    np.testing.assert_allclose(got, ref, rtol=tol, atol=tol)
 
 
 @pytest.mark.parametrize('tag,F', [('a', 128), ('b', 128), ('c', 128), ('d', 128), ('b', 256)])
@@ -256,6 +275,7 @@ def test_conv_tail_stitch_matches_recompose(env, tag, F):
     _capi.check(lib.dsen2_conv_tail16(_capi.ptr(dev[0]), _capi.ptr(dev[1]), _capi.ptr(tw), _capi.ptr(dev[4]),
                                       _capi.ptr(dev[2]), _capi.ptr(dev[3]), 4, cout, F, n, P, P, _capi.ptr(pred),
                                       _capi.stream_ptr()), 'conv tail16')
+    ts.report(ts.tail_schedule(n - n // 2, P, P, border=B), 'conv_tail16_stitch F=%d, larger shard' % F, float('nan'))
     canvas = torch.full((H, W, cout), -1.0, device='cuda')
     # two shards, second first: ownership (not launch order) decides every pixel
     half = n // 2
@@ -277,7 +297,7 @@ def test_conv_tail_stitch_matches_recompose(env, tag, F):
 
 
 @pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (3, 40, 24), (1, 8, 200), (2, 192, 192), (2, 32, 32, 256),
-                                   (1, 24, 72, 256)])
+                                   (1, 24, 72, 256), ts.PATCH, ts.RAGGED, ts.PATCH + (256,), ts.RAGGED + (256,)])
 @pytest.mark.parametrize('want_lo', [False, True])
 def test_conv_res32_fp32_trunk_update(env, shape, want_lo):
     """trunk32 <- trunk32 + 0.1 * (conv(t) + b) in place on the tile-row-major fp32 trunk; fp16 hi (and lo) copies.
@@ -303,6 +323,7 @@ def test_conv_res32_fp32_trunk_update(env, shape, want_lo):
     ref = x.astype(np.float64) + 0.1 * _conv64(t.astype(np.float64), w.astype(np.float16).astype(np.float64), bias)
     got = tx.cpu().numpy().transpose(0, 1, 2, 4, 3, 5).reshape(n, H, W, F)
     tol = 2e-5 if F == 128 else 4e-5                  # fp32 accumulation over K = 9 F
+    ts.check(ts.pair_schedule(n, H, W), 'conv_res32 F=%d lo=%s' % (F, want_lo), np.abs(got - ref).max())
     np.testing.assert_allclose(got, ref, rtol=tol, atol=tol)
     assert np.array_equal(hi.cpu().numpy().view(np.uint16), got.astype(np.float16).view(np.uint16))
     if want_lo:
@@ -311,7 +332,7 @@ def test_conv_res32_fp32_trunk_update(env, shape, want_lo):
 
 
 # ---- fp16 + 8 bit trunk (include/dsen2_b200.h: dsen2_conv_head16_q / dsen2_conv_resq) -------------------------------
-@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (3, 40, 24), (1, 8, 200), (2, 192, 192)])
+@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (3, 40, 24), (1, 8, 200), (2, 192, 192), ts.PATCH, ts.RAGGED])
 @pytest.mark.parametrize('last', [False, True])
 def test_conv_resq_trunk_update(env, shape, last):
     """x <- x + 0.1 * (conv(t) + b) on the fp16 + 8 bit trunk, in place; the last block emits x_hi, x_lo for the tail."""
@@ -337,8 +358,10 @@ def test_conv_resq_trunk_update(env, shape, last):
     torch.cuda.synchronize()
     ref = x_seen.astype(np.float64) + 0.1 * _conv64(t.astype(np.float64), w.astype(np.float16).astype(np.float64), bias)
     h = thi.cpu().numpy()
+    sched = ts.pair_schedule(n, H, W)
     if last:
         got = h.astype(np.float64) + lo.cpu().numpy().astype(np.float64)
+        ts.check(sched, 'conv_resq last', np.abs(got - ref).max())
         np.testing.assert_allclose(got, ref, rtol=2e-5, atol=2e-5)
         # x_hi = fp16(x): re-rounding hi + lo differs only where x sits within 2^-22 of a rounding tie (~2^-11 of the elements)
         assert np.mean(got.astype(np.float32).astype(np.float16).view(np.uint16) == h.view(np.uint16)) > 0.999
@@ -346,6 +369,7 @@ def test_conv_resq_trunk_update(env, shape, last):
     else:
         q = _q_from_tiles(tq.cpu().numpy())
         got = _q_decode(h, q)
+        ts.check(sched, 'conv_resq', np.abs(got - ref).max())
         np.testing.assert_allclose(got, ref, rtol=2e-5, atol=2e-5)
         ok = np.abs(got) >= 2 * NORMAL
         h2, q2 = _q_encode(got[ok])
@@ -374,7 +398,8 @@ def test_prep16_from_patches_layout_bit_exact(env, chan):
     assert np.array_equal(lo.cpu().numpy().view(np.uint16), elo.view(np.uint16))
 
 
-@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (3, 40, 24), (1, 8, 200), (5, 16, 8), (1, 192, 192)])
+@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (3, 40, 24), (1, 8, 200), (5, 16, 8), (1, 192, 192), ts.PATCH,
+                                   ts.RAGGED])
 @pytest.mark.parametrize('F', [128, 256])
 def test_conv_head16_q_nine_taps(env, shape, F):
     """First layer on the 16-channel input: nine shifted 32-byte-row descriptors, three products (hi*W_hi + hi*W_lo +
@@ -403,11 +428,45 @@ def test_conv_head16_q_nine_taps(env, shape, F):
     w_eff = w_hi.astype(np.float64) + (w - w_hi.astype(np.float32)).astype(np.float16).astype(np.float64)
     ref = np.maximum(_conv64(xin, w_eff, bias), 0)         # (the kernel drops lo * W_lo: ~2^-22 of a product)
     got = _q_decode(ohi.cpu().numpy(), _q_from_tiles(oq.cpu().numpy()))
+    ts.check(ts.pair_schedule(n, H, W), 'conv_head16_q F=%d' % F, np.abs(got - ref).max())
     np.testing.assert_allclose(got, ref, rtol=2e-5, atol=2e-5)
     assert np.abs(got - np.maximum(_conv64(xcat.transpose(0, 2, 3, 1), w, bias), 0)).max() < 5e-5   # vs the true fp32 layer
 
 
-@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (3, 40, 24)])
+@pytest.mark.parametrize('shape', [ts.PATCH, ts.RAGGED])
+def test_conv_head16_relu(env, shape):
+    """The first layer of the 256-feature training step (dsen2_conv_head16_relu): the nine-tap three-product convolution of
+    dsen2_conv_head16_q, relu -> NHWC fp16 and the seed of the fp32 trunk, tile-row-major (n, H, W/8, F/4, 8, 4)."""
+    torch, _capi, lib = env
+    n, H, W = shape
+    C, F = 12, 256
+    rng = np.random.RandomState(H + 3 * W + F)
+    x = rng.uniform(0, 5, size=(n, H, W, C)).astype(np.float32)
+    hi, lo = _split(np.concatenate([x, np.zeros((n, H, W, 16 - C), np.float32)], axis=-1))
+    lim = np.sqrt(6.0 / (9 * C))
+    w = rng.uniform(-lim, lim, size=(3, 3, C, F)).astype(np.float32)
+    bias = (rng.randn(F) * 0.1).astype(np.float32)
+    tw = torch.empty((9, 2 * F, 16), dtype=torch.float16, device='cuda')
+    _capi.check(lib.dsen2_pack_head16_weights(_capi.ptr(torch.from_numpy(w).cuda()), C, F, _capi.ptr(tw),
+                                              _capi.stream_ptr()), 'pack head16')
+    thi, tlo, tb = torch.from_numpy(hi).cuda(), torch.from_numpy(lo).cuda(), torch.from_numpy(bias).cuda()
+    ohi = torch.zeros((n, H, W, F), dtype=torch.float16, device='cuda')
+    x32 = torch.full((n, H, W // 8, F // 4, 8, 4), -3.0, device='cuda')
+    _capi.check(lib.dsen2_conv_head16_relu(_capi.ptr(thi), _capi.ptr(tlo), _capi.ptr(tw), _capi.ptr(tb), n, H, W, F,
+                                           _capi.ptr(ohi), _capi.ptr(x32), _capi.stream_ptr()), 'conv head16 relu')
+    torch.cuda.synchronize()
+    xin = (hi.astype(np.float64) + lo.astype(np.float64))[..., :C]
+    w_hi = w.astype(np.float16)
+    w_eff = w_hi.astype(np.float64) + (w - w_hi.astype(np.float32)).astype(np.float16).astype(np.float64)
+    ref = np.maximum(_conv64(xin, w_eff, bias), 0)         # (the kernel drops lo * W_lo: ~2^-22 of a product)
+    trunk = x32.cpu().numpy().transpose(0, 1, 2, 4, 3, 5).reshape(n, H, W, F)
+    ts.check(ts.pair_schedule(n, H, W), 'conv_head16_relu', np.abs(trunk - ref).max())
+    np.testing.assert_allclose(trunk, ref, rtol=2e-5, atol=2e-5)
+    assert np.abs(trunk - np.maximum(_conv64(x, w, bias), 0)).max() < 5e-5                       # vs the true fp32 layer
+    assert np.array_equal(trunk.astype(np.float16).view(np.uint16), ohi.cpu().numpy().view(np.uint16))
+
+
+@pytest.mark.parametrize('shape', [(2, 32, 32), (1, 128, 128), (3, 40, 24), ts.PATCH, ts.RAGGED])
 @pytest.mark.parametrize('last', [False, True])
 def test_conv_resq256_trunk_update(env, shape, last):
     """The 256-feature (VDSen2) resblock update on the fp16 + 8 bit trunk: two 64-channel passes per thread; the last
@@ -432,12 +491,15 @@ def test_conv_resq256_trunk_update(env, shape, last):
                                        _capi.ptr(tq), _capi.ptr(lo), _capi.stream_ptr()), 'conv resq256')
     torch.cuda.synchronize()
     ref = x_seen.astype(np.float64) + 0.1 * _conv64(t.astype(np.float64), w.astype(np.float16).astype(np.float64), bias)
+    sched = ts.pair_schedule(n, H, W)
     if last:
         got = thi.cpu().numpy().astype(np.float64) + lo.cpu().numpy().astype(np.float64)
+        ts.check(sched, 'conv_resq256 last', np.abs(got - ref).max())
         np.testing.assert_allclose(got, ref, rtol=3e-5, atol=3e-5)
         return
     h, q = thi.cpu().numpy(), _q_from_tiles(tq.cpu().numpy())
     got = _q_decode(h, q)
+    ts.check(sched, 'conv_resq256', np.abs(got - ref).max())
     np.testing.assert_allclose(got, ref, rtol=3e-5, atol=3e-5)
     ok = np.abs(got) >= 2 * NORMAL
     h2, q2 = _q_encode(got[ok])

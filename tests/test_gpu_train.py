@@ -8,6 +8,8 @@ with float64 restatements on the SAME fp16-rounded operands (rtol/atol 1e-3 or t
 import numpy as np
 import pytest
 
+import tile_schedule as ts
+
 pytestmark = pytest.mark.gpu
 
 
@@ -71,11 +73,14 @@ def test_relu_mask(env, C):
     assert np.array_equal(out.cpu().numpy().view(np.uint16), np.where(a.astype(np.float32) > 0, g, np.float16(0)).view(np.uint16))
 
 
-@pytest.mark.parametrize('C', [128, 256])
-def test_conv_relu_bwd_is_the_transposed_convolution(env, C):
+@pytest.mark.parametrize('C,shape', [pytest.param(C, (2, 32, 32), id=str(C)) for C in (128, 256)] +
+                         [pytest.param(C, s, id='%d-%s' % (C, name)) for name, s in (('patch', ts.PATCH), ('batch128', ts.BATCH128))
+                          for C in (128, 256)])
+def test_conv_relu_bwd_is_the_transposed_convolution(env, C, shape):
+    """ts.BATCH128 is DSen2's training batch: seven tiles on the busiest CTA pair."""
     torch, _capi, lib = env
     import torch.nn.functional as F
-    n, H, W = 2, 32, 32
+    n, H, W = shape
     rng = np.random.RandomState(3)
     dy = (rng.randn(n, H, W, C) * 0.1).astype(np.float16)
     act = np.maximum(rng.randn(n, H, W, C), 0).astype(np.float16)
@@ -95,7 +100,9 @@ def test_conv_relu_bwd_is_the_transposed_convolution(env, C):
     wt = torch.from_numpy(wq).permute(3, 2, 0, 1).contiguous()                     # (Cout, Cin, 3, 3)
     g = F.conv_transpose2d(torch.from_numpy(dy.astype(np.float64)).permute(0, 3, 1, 2), wt, padding=1)
     ref = np.where(act.astype(np.float32) > 0, g.permute(0, 2, 3, 1).numpy(), 0)
-    np.testing.assert_allclose(out.cpu().numpy().astype(np.float64), ref, rtol=2e-3, atol=2e-3 * np.abs(ref).max())
+    got = out.cpu().numpy().astype(np.float64)
+    ts.check(ts.pair_schedule(n, H, W), 'conv_relu_bwd C=%d' % C, np.abs(got - ref).max() / np.abs(ref).max())
+    np.testing.assert_allclose(got, ref, rtol=2e-3, atol=2e-3 * np.abs(ref).max())
 
 
 @pytest.mark.parametrize('F', [128, 256])
@@ -136,8 +143,11 @@ def _setup(L=2, n=4, P=32, run_60=False, seed=0, F=128):
 
 @pytest.mark.parametrize('cfg', [dict(L=2, n=4, P=32), dict(L=6, n=8, P=32), dict(L=1, n=2, P=32, run_60=True),
                                  dict(L=0, n=2, P=16), dict(L=2, n=4, P=32, F=256), dict(L=1, n=2, P=32, run_60=True, F=256),
-                                 dict(L=4, n=8, P=32, F=256), dict(L=32, n=2, P=32, F=256)])
+                                 dict(L=4, n=8, P=32, F=256), dict(L=32, n=2, P=32, F=256), dict(L=2, n=128, P=32),
+                                 dict(L=1, n=64, P=32, F=256)])
 def test_gradients_vs_autograd(env, cfg):
+    """n = 128 is DSen2's training batch (supres_train.py), n = 64 at F = 256 the benchmark's VDSen2 training step: there
+    every convolution of the step runs several tiles per CTA (pair)."""
     torch, _capi, lib = env
     from dsen2_b200.train import Trainer
     from oracle import train_oracle as to
@@ -155,7 +165,45 @@ def test_gradients_vs_autograd(env, cfg):
             err = np.abs(got - ref).max() / (np.abs(ref).max() + 1e-12)
             worst = max(worst, err)
             assert err <= 2e-2, "layer %d %s: relative gradient error %.3e" % (i, ref.shape, err)
-    print('worst relative gradient error', worst)
+    n, P = cfg['n'], cfg['P']
+    label = 'training step %s, relative gradient' % cfg
+    ts.check(ts.pair_schedule(n, P, P), label, worst)
+    if cfg.get('F', 128) == 256:                     # the 256-feature step's last layer is the swapped tail
+        ts.check(ts.tail_schedule(n, P, P), label, worst)
+
+
+def test_mae_grad_at_the_training_batch(env):
+    """dsen2_mae_grad over DSen2's batch (128 x 6 x 32 x 32 = 786,432 elements), where its grid-stride loop runs several
+    times per thread: dpred = gscale * sign(fp32(pred - y)) bit for bit, +0 on exact ties; both double sums against float64
+    numpy, accumulated on top of what the buffer holds."""
+    torch, _capi, lib = env
+    total = 128 * 6 * 32 * 32
+    threads = min(-(-total // 256), 4 * ts.sm_count()) * 256      # grid_for(total, 256, 4)
+    loops = -(-total // threads)
+    print('mae_grad: %d elements over %d threads, %d iterations on the busiest thread' % (total, threads, loops))
+    assert loops >= 3
+    rng = np.random.RandomState(128)
+    pred = (0.8 + 0.4 * rng.randn(total)).astype(np.float32)
+    y = (pred + 0.1 * rng.randn(total)).astype(np.float32)
+    tie = rng.rand(total) < 0.01
+    y[tie] = pred[tie]
+    gscale = np.float32(3.0 / 7.0)
+    sums0 = np.array([123.5, -7.25])
+    tp, ty = torch.from_numpy(pred).cuda(), torch.from_numpy(y).cuda()
+    dpred = torch.full((total,), float('nan'), device='cuda')
+    sums = torch.from_numpy(sums0).cuda()
+    _capi.check(lib.dsen2_mae_grad(_capi.ptr(tp), _capi.ptr(ty), total, float(gscale), _capi.ptr(dpred), _capi.ptr(sums),
+                                   _capi.stream_ptr()), 'mae')
+    torch.cuda.synchronize()
+    d = pred - y                                                     # float32, as the kernel subtracts
+    got = dpred.cpu().numpy()
+    assert np.array_equal(got.view(np.uint32), (gscale * np.sign(d)).view(np.uint32))
+    assert tie.sum() > 1000 and not got[tie].view(np.uint32).any()   # +0, not -0
+    d64 = d.astype(np.float64)
+    ref = sums0 + np.array([np.abs(d64).sum(), (d64 * d64).sum()])
+    got_s = sums.cpu().numpy()
+    print('mae_grad sums: relative error %.3e %.3e' % tuple(np.abs(got_s - ref) / np.abs(ref)))
+    np.testing.assert_allclose(got_s, ref, rtol=1e-10, atol=0)
 
 
 @pytest.mark.parametrize('F', [128, 256])

@@ -380,22 +380,36 @@ class S2Model:
         equal to ``avoid`` (an int in [0, 65535], the nodata value) is written one step away from it
         (``dsen2_conv_tail16_stitch_u16`` in include/dsen2_b200.h).  ``add_offset``: a finite float (None: none) added to
         every band value before the preparation and subtracted from every output value before it is stored
-        (``dsen2_prep16_from_images_offset``, ``dsen2_conv_tail16_stitch_offset``)."""
+        (``dsen2_prep16_from_images_offset``, ``dsen2_conv_tail16_stitch_offset``).
+
+        Chip stacks: 4-D images (N, H, W, C) of N same-size chips and an (N, H, W, Cout) canvas.  [first_patch,
+        first_patch+n) is then a range of the flat list chip * ppc + patch (ppc = the filled patches of one chip), which
+        may straddle chips; each chip is prepared and stitched as the 3-D call on that chip does it
+        (``dsen2_prep16_from_chips``, ``dsen2_conv_tail16_stitch_chips``).  No ``patch_ids`` with stacks."""
         torch = _capi.require_cuda()
         if not self.xin16:
             raise _capi.DSen2Error("forward_images needs a network with resblocks (num_layers > 0)")
         dev = d10.device
-        H, W = int(d10.shape[0]), int(d10.shape[1])
+        chips = d10.dim() == 4
+        lead = (int(d10.shape[0]),) if chips else ()
+        H, W = int(d10.shape[len(lead)]), int(d10.shape[len(lead) + 1])
         imgs = [t for t in (d10, d20, d60) if t is not None]
         if any(t.dtype != d10.dtype for t in imgs) or d10.dtype not in (torch.float32, torch.uint16):
             raise ValueError("images must all be float32 or all be uint16")
+        if chips:
+            for t, div, c in zip(imgs, (1, 2, 6), self.in_channels):
+                if not (t.is_cuda and t.is_contiguous() and tuple(t.shape) == lead + (H // div, W // div, c)):
+                    raise ValueError("chip stack images must be contiguous CUDA tensors of shape %s, got %s"
+                                     % (lead + (H // div, W // div, c), tuple(t.shape)))
+            if patch_ids is not None:
+                raise ValueError("patch_ids are not supported with chip stacks")
         if patch_ids is not None and not (patch_ids.is_cuda and patch_ids.dtype == torch.int32 and patch_ids.is_contiguous()
                                           and tuple(patch_ids.shape) == (n,)):
             raise ValueError("patch_ids must be a contiguous CUDA int32 tensor of %d ids" % n)
         if not (canvas.is_cuda and canvas.dtype in (torch.float32, torch.uint16) and canvas.is_contiguous()
-                and tuple(canvas.shape) == (H, W, self.out_channels)):
+                and tuple(canvas.shape) == lead + (H, W, self.out_channels)):
             raise ValueError("canvas must be a contiguous CUDA float32 or uint16 tensor of shape %s"
-                             % ((H, W, self.out_channels),))
+                             % (lead + (H, W, self.out_channels),))
         u16 = canvas.dtype == torch.uint16
         if avoid is not None and not u16:
             raise ValueError("avoid applies to a uint16 canvas only")
@@ -410,6 +424,17 @@ class S2Model:
         buf = self._buffers(dev, n, patch, reuse_larger=patch_ids is not None)
         with torch.cuda.device(dev):
             st = _capi.stream_ptr()
+            if chips:
+                add, a = (0, 0.0) if add_offset is None else (1, float(add_offset))
+                self._timed(timers, 'prep', n, lambda: _capi.check(lib.dsen2_prep16_from_chips(
+                    ptr(d10), ptr(d20), ptr(d60), img_dtype, lead[0], H, W, patch, border, first_patch, n, float(mul), add,
+                    a, ptr(buf['xin_hi']), ptr(buf['xin_lo']), st), "dsen2_prep16_from_chips"))
+                self._trunk(buf, wts, biases, n, patch, st, timers)
+                self._timed(timers, 'conv_tail', n, lambda: _capi.check(lib.dsen2_conv_tail16_stitch_chips(
+                    *self._tail_args(buf, wts, biases), self.feature_size, n, patch, first_patch, border, lead[0], H, W,
+                    float(mul), add, a, _capi.IMG_U16 if u16 else _capi.IMG_F32, avoid, ptr(canvas), st),
+                    "dsen2_conv_tail16_stitch_chips"))
+                return canvas
             if add_offset is not None:
                 self._timed(timers, 'prep', n, lambda: _capi.check(lib.dsen2_prep16_from_images_offset(
                     ptr(d10), ptr(d20), ptr(d60), img_dtype, H, W, patch, border, first_patch, ptr(patch_ids), n,

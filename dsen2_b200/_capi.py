@@ -70,6 +70,11 @@ SIGNATURES = {
     "dsen2_conv_tail16_stitch_offset": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                                 c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_float, c_float,
                                                 c_int, c_int, c_void_p, c_void_p]),
+    "dsen2_prep16_from_chips": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                        c_int, c_float, c_int, c_float, c_void_p, c_void_p, c_void_p]),
+    "dsen2_conv_tail16_stitch_chips": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                               c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_int,
+                                               c_float, c_int, c_int, c_void_p, c_void_p]),
     "dsen2_conv_resq256": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p,
                                    c_void_p, c_void_p]),
     "dsen2_conv_tail": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,

@@ -81,7 +81,9 @@ __device__ __forceinline__ int tail_stitch_tile_of(int y, int size, int S, int n
   return (size % S != 0 && y >= size - S) ? n - 1 : y / S;
 }
 
-template <int KPM, bool IDS, typename OutT, bool ADD>
+// CHIPS (stitching form): the canvas is a stack of same-size chip canvases (num_chips, img_h, img_w, cout) and
+// first_patch + b indexes the flat list chip * ppc + patch (ppc = grid_ny * grid_nx); ownership stays inside the chip.
+template <int KPM, bool IDS, typename OutT, bool ADD, bool CHIPS>
 __global__ void __launch_bounds__(kTThreads, 1)
 conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
                          const __grid_constant__ CUtensorMap tm_w, const TailParams p) {
@@ -199,7 +201,13 @@ conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid
           d.obase = (long long)b * p.cout * d.ostride + (long long)y * p.W + x;
         } else {
           const int S = p.H - 2 * p.border;
-          const int patch = IDS ? __ldg(p.patch_ids + b) : p.first_patch + b;
+          int patch = IDS ? __ldg(p.patch_ids + b) : p.first_patch + b;
+          long long chip_base = 0;                     // CHIPS: first element of the chip's canvas (64-bit)
+          if constexpr (CHIPS) {
+            const int chip = patch / (p.grid_ny * p.grid_nx);
+            patch -= chip * (p.grid_ny * p.grid_nx);
+            chip_base = (long long)chip * p.img_h * p.img_w * p.cout;
+          }
           const int pty = patch / p.grid_nx, ptx = patch - pty * p.grid_nx;
           const int gy = min(pty * S, p.img_h - S) + y - p.border;
           const int gx = min(ptx * S, p.img_w - S) + x - p.border;
@@ -207,7 +215,7 @@ conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid
                     y >= p.border && y < p.H - p.border && x >= p.border && x < p.W - p.border &&
                     tail_stitch_tile_of(gy, p.img_h, S, p.grid_ny) == pty && tail_stitch_tile_of(gx, p.img_w, S, p.grid_nx) == ptx;
           d.ostride = 1;
-          d.obase = ((long long)gy * p.img_w + gx) * p.cout;
+          d.obase = chip_base + ((long long)gy * p.img_w + gx) * p.cout;
         }
       }
       if (d.write) {
@@ -302,12 +310,12 @@ __global__ void pack_tail16_weights_kernel(const float* __restrict__ hwio, int F
   }
 }
 
-template <int KPM, bool IDS, typename OutT, bool ADD>
+template <int KPM, bool IDS, typename OutT, bool ADD, bool CHIPS>
 static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_lo, const void* d_w, int sms, cudaStream_t stream) {
   using Cfg = TailCfg<KPM>;
   static bool configured[64] = {};
   if (needs_config(configured)) {
-    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM, IDS, OutT, ADD>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM, IDS, OutT, ADD, CHIPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   }
   const int F = KPM * 64;
   CUtensorMap hi, lo, w;
@@ -320,22 +328,22 @@ static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_
   const uint32_t wb[2] = {64, 128};
   if ((rc = make_tmap_f16_sw(&w, d_w, 2, wd, wb, 128)) != 0) return rc;
   const int grid = (int)(p.num_tiles < (uint32_t)sms ? p.num_tiles : (uint32_t)sms);
-  conv_tail_swapped_kernel<KPM, IDS, OutT, ADD><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
+  conv_tail_swapped_kernel<KPM, IDS, OutT, ADD, CHIPS><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
   return check_launch("conv_tail_swapped");
 }
 
-template <bool IDS, typename OutT, bool ADD>
+template <bool IDS, typename OutT, bool ADD, bool CHIPS = false>
 static int launch_tail_f(const TailParams& p, int features, const void* d_x_hi, const void* d_x_lo, const void* d_w, int sms,
                          cudaStream_t stream) {
-  return features == 256 ? launch_tail<4, IDS, OutT, ADD>(p, d_x_hi, d_x_lo, d_w, sms, stream)
-                         : launch_tail<2, IDS, OutT, ADD>(p, d_x_hi, d_x_lo, d_w, sms, stream);
+  return features == 256 ? launch_tail<4, IDS, OutT, ADD, CHIPS>(p, d_x_hi, d_x_lo, d_w, sms, stream)
+                         : launch_tail<2, IDS, OutT, ADD, CHIPS>(p, d_x_hi, d_x_lo, d_w, sms, stream);
 }
 
-// add: run the ADD instances, which subtract p.add_offset from every stitched value
+// add: run the ADD instances, which subtract p.add_offset from every stitched value; chips: the CHIPS instances (range form)
 template <typename OutT>
 static int tail16_common(TailParams& p, int features, const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
                          const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int n, int H, int W, OutT* d_out,
-                         bool add, void* stream) {
+                         bool add, void* stream, bool chips = false) {
   DSEN2_REQUIRE(d_x_hi && d_x_lo && d_w && d_bias && d_xin_hi && d_xin_lo && d_out, DSEN2_E_BADARG, "dsen2_conv_tail16: null pointer");
   DSEN2_REQUIRE(features == 128 || features == 256, DSEN2_E_BADARG, "dsen2_conv_tail16: feature_size must be 128 or 256 (got %d)",
                 features);
@@ -364,6 +372,9 @@ static int tail16_common(TailParams& p, int features, const void* d_x_hi, const 
   p.skip_hi = (const __half*)d_xin_hi; p.skip_lo = (const __half*)d_xin_lo; p.skip_ch0 = skip_ch0;
   p.cout = cout; p.out = d_out;
   const cudaStream_t st = (cudaStream_t)stream;
+  if (chips)
+    return add ? launch_tail_f<false, OutT, true, true>(p, features, d_x_hi, d_x_lo, d_w, sms, st)
+               : launch_tail_f<false, OutT, false, true>(p, features, d_x_hi, d_x_lo, d_w, sms, st);
   if (p.patch_ids)
     return add ? launch_tail_f<true, OutT, true>(p, features, d_x_hi, d_x_lo, d_w, sms, st)
                : launch_tail_f<true, OutT, false>(p, features, d_x_hi, d_x_lo, d_w, sms, st);
@@ -398,12 +409,13 @@ extern "C" int dsen2_conv_tail16(const void* d_x_hi, const void* d_x_lo, const v
 }
 
 // the stitching form: patches first_patch + b, or d_patch_ids[b] when d_patch_ids is not null; float or uint16 canvas;
-// with add, add_offset is subtracted from every value after the scale
+// with add, add_offset is subtracted from every value after the scale.  num_chips >= 0: the canvas is a stack of num_chips
+// chip canvases and first_patch + b indexes their flat patch list (no id list); -1: one canvas.
 template <typename OutT>
 static int tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias, const void* d_xin_hi,
                          const void* d_xin_lo, int skip_ch0, int cout, int feature_size, int n, int P, int first_patch,
                          const int* d_patch_ids, int border, int img_h, int img_w, float mul, int avoid, OutT* d_canvas,
-                         void* stream, bool add = false, float add_offset = 0.f) {
+                         void* stream, bool add = false, float add_offset = 0.f, int num_chips = -1) {
   const int S = P - 2 * border;
   DSEN2_REQUIRE(P > 0 && border >= 0 && S > 0 && img_h >= S && img_w >= S && first_patch >= 0, DSEN2_E_BADARG,
                 "dsen2_conv_tail16_stitch: bad stitch geometry (P %d border %d image %dx%d)", P, border, img_h, img_w);
@@ -416,11 +428,18 @@ static int tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w
   p.first_patch = first_patch; p.img_h = img_h; p.img_w = img_w; p.border = border;
   p.grid_ny = ceil_div(img_h, S); p.grid_nx = ceil_div(img_w, S);
   p.patch_ids = d_patch_ids;
-  DSEN2_REQUIRE(d_patch_ids || first_patch + n <= p.grid_ny * p.grid_nx, DSEN2_E_BADARG,
-                "dsen2_conv_tail16_stitch: patch range [%d,%d) exceeds the %d tiles of the canvas", first_patch,
-                first_patch + n, p.grid_ny * p.grid_nx);
+  if (num_chips >= 0) {
+    const long long flat = (long long)num_chips * p.grid_ny * p.grid_nx;
+    DSEN2_REQUIRE(!d_patch_ids && n >= 0 && flat < (1LL << 31) && (long long)first_patch + n <= flat, DSEN2_E_BADARG,
+                  "dsen2_conv_tail16_stitch_chips: patch range [%d,%lld) outside the %lld patches of %d chips", first_patch,
+                  (long long)first_patch + n, flat, num_chips);
+  } else {
+    DSEN2_REQUIRE(d_patch_ids || first_patch + n <= p.grid_ny * p.grid_nx, DSEN2_E_BADARG,
+                  "dsen2_conv_tail16_stitch: patch range [%d,%d) exceeds the %d tiles of the canvas", first_patch,
+                  first_patch + n, p.grid_ny * p.grid_nx);
+  }
   return tail16_common<OutT>(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, P, P,
-                             d_canvas, add, stream);
+                             d_canvas, add, stream, num_chips >= 0);
 }
 
 extern "C" int dsen2_conv_tail16_stitch(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
@@ -475,4 +494,27 @@ extern "C" int dsen2_conv_tail16_stitch_offset(const void* d_x_hi, const void* d
                                    add_offset);
   return tail16_stitch<float>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P, first,
                               d_patch_ids, border, img_h, img_w, mul, -1, (float*)d_canvas, stream, true, add_offset);
+}
+
+extern "C" int dsen2_conv_tail16_stitch_chips(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                              const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout,
+                                              int feature_size, int n, int P, int first_patch, int border, int num_chips,
+                                              int img_h, int img_w, float mul, int add, float add_offset, int canvas_dtype,
+                                              int avoid, void* d_canvas, void* stream) {
+  const char* name = "dsen2_conv_tail16_stitch_chips";
+  DSEN2_REQUIRE(num_chips >= 0, DSEN2_E_BADARG, "%s: num_chips %d < 0", name, num_chips);
+  DSEN2_REQUIRE(add == 0 || add == 1, DSEN2_E_BADARG, "%s: add must be 0 or 1 (got %d)", name, add);
+  DSEN2_REQUIRE(!add || isfinite(add_offset), DSEN2_E_BADARG, "%s: add_offset must be finite", name);
+  DSEN2_REQUIRE(canvas_dtype == DSEN2_IMG_F32 || canvas_dtype == DSEN2_IMG_U16, DSEN2_E_BADARG,
+                "%s: canvas_dtype must be DSEN2_IMG_F32 or DSEN2_IMG_U16 (got %d)", name, canvas_dtype);
+  DSEN2_REQUIRE(canvas_dtype == DSEN2_IMG_U16 || avoid == -1, DSEN2_E_BADARG,
+                "%s: avoid must be -1 for a float canvas (got %d)", name, avoid);
+  const float a = add ? add_offset : 0.f;
+  if (canvas_dtype == DSEN2_IMG_U16)
+    return tail16_stitch<uint16_t>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P,
+                                   first_patch, nullptr, border, img_h, img_w, mul, avoid, (uint16_t*)d_canvas, stream,
+                                   add != 0, a, num_chips);
+  return tail16_stitch<float>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P,
+                              first_patch, nullptr, border, img_h, img_w, mul, -1, (float*)d_canvas, stream, add != 0, a,
+                              num_chips);
 }

@@ -8,6 +8,7 @@
 //                               (patches.py:11-16: per-patch bilinear with mirror boundary) and the /2000 scaling
 //                               (supres.py:23-24,42-44) with the arithmetic of the standalone kernels.
 //   dsen2_prep16_from_images_offset : the same with a radiometric offset added to every loaded band value first
+//   dsen2_prep16_from_chips   : the same from stacks of same-size chips, patches indexed chip * ppc + patch
 // Training step (and networks without resblocks): "x_in", 64 channels per pixel = the three HORIZONTAL taps of the first
 // 3x3 convolution pre-gathered, x_in[n][y][x][t*16 + c] = X[n][c][y][x + t - 1] (zero outside the patch), because the
 // first layer's weight-gradient GEMM wants 128-byte pixel rows (dsen2_prep_from_patches).
@@ -112,9 +113,19 @@ __global__ void prep16_from_patches_kernel(const float* __restrict__ x0, int c0,
   }
 }
 
+// The source of chip `chip` of a stack of same-size images (N, H, W, C): the image pointer advanced by chip * H * W * C
+// elements, in 64 bits (100k chips of 120 x 120 x 4 are 5.8e9 elements).
+template <typename T, int C>
+__device__ __forceinline__ PrepSource chip_source(PrepSource s, int chip) {
+  s.img = reinterpret_cast<const T*>(s.img) + (long long)chip * s.H * s.W * C;
+  return s;
+}
+
 // IDS: batch entry b is patch ids[b] (a list of active patches) instead of first_patch + b.  ADD: add_offset is added to
 // every loaded band value (ld_band); it is the last parameter, so the other instances keep their parameter layout.
-template <typename T, bool IDS, bool ADD>
+// CHIPS: the images are stacks of same-size chips and first_patch + b indexes the flat list chip * ppc + patch, with ppc =
+// n_i * n_j the filled patches of one chip; the chip and its patch are resolved per patch index with one 32-bit division.
+template <typename T, bool IDS, bool ADD, bool CHIPS>
 __global__ void prep16_from_images_kernel(PrepSource s0, PrepSource s1, PrepSource s2, int nsrc, int plr, int blr, int P,
                                           Tiling tl, int first_patch, const int* __restrict__ ids, long long total,
                                           float divisor, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
@@ -125,7 +136,12 @@ __global__ void prep16_from_images_kernel(PrepSource s0, PrepSource s1, PrepSour
     const int local = (int)(idx / PP);
     const int rem = (int)(idx - (long long)local * PP);
     const int y = rem / P, x = rem - y * P;
-    const int patch = IDS ? __ldg(ids + local) : first_patch + local;
+    int patch = IDS ? __ldg(ids + local) : first_patch + local;
+    int chip = 0;
+    if constexpr (CHIPS) {
+      chip = patch / (tl.n_i * tl.n_j);
+      patch -= chip * (tl.n_i * tl.n_j);
+    }
     float v[16];
 #pragma unroll
     for (int c = 0; c < 16; ++c) v[c] = 0.f;
@@ -134,9 +150,15 @@ __global__ void prep16_from_images_kernel(PrepSource s0, PrepSource s1, PrepSour
       const int ti = patch / tl.n_j, tj = patch - ti * tl.n_j;
       const int si = ti < tl.k_i ? ti * tl.stride : tl.last_i;
       const int sj = tj < tl.k_j ? tj * tl.stride : tl.last_j;
-      prep_gather<T, 4, 0, ADD>(s0, si, sj, plr, blr, y, x, divisor, add_offset, v);     // 10 m bands   (DSen2Net.py:24,26 order)
-      prep_gather<T, 6, 4, ADD>(s1, si, sj, plr, blr, y, x, divisor, add_offset, v);     // 20 m bands
-      if (nsrc == 3) prep_gather<T, 2, 10, ADD>(s2, si, sj, plr, blr, y, x, divisor, add_offset, v);   // 60 m bands
+      if constexpr (CHIPS) {
+        prep_gather<T, 4, 0, ADD>(chip_source<T, 4>(s0, chip), si, sj, plr, blr, y, x, divisor, add_offset, v);
+        prep_gather<T, 6, 4, ADD>(chip_source<T, 6>(s1, chip), si, sj, plr, blr, y, x, divisor, add_offset, v);
+        if (nsrc == 3) prep_gather<T, 2, 10, ADD>(chip_source<T, 2>(s2, chip), si, sj, plr, blr, y, x, divisor, add_offset, v);
+      } else {
+        prep_gather<T, 4, 0, ADD>(s0, si, sj, plr, blr, y, x, divisor, add_offset, v);     // 10 m bands   (DSen2Net.py:24,26 order)
+        prep_gather<T, 6, 4, ADD>(s1, si, sj, plr, blr, y, x, divisor, add_offset, v);     // 20 m bands
+        if (nsrc == 3) prep_gather<T, 2, 10, ADD>(s2, si, sj, plr, blr, y, x, divisor, add_offset, v);   // 60 m bands
+      }
     }
     Half16 hi, lo;
     split16(v, hi, lo);
@@ -332,21 +354,43 @@ extern "C" int dsen2_prep16_from_patches(const float* d_x0, int c0, const float*
   return check_launch("prep16_from_patches");
 }
 
-template <typename T, bool IDS, bool ADD>
+template <typename T, bool IDS, bool ADD, bool CHIPS>
 static void launch_prep16(PrepSource s0, PrepSource s1, PrepSource s2, int nsrc, int plr, int blr, int P, Tiling tl,
                           int first_patch, const int* d_patch_ids, long long total, float divisor, float add_offset,
                           void* d_xin_hi, void* d_xin_lo, cudaStream_t stream) {
   const int block = 256;
-  prep16_from_images_kernel<T, IDS, ADD><<<grid_for(total, block), block, 0, stream>>>(
+  prep16_from_images_kernel<T, IDS, ADD, CHIPS><<<grid_for(total, block), block, 0, stream>>>(
       s0, s1, s2, nsrc, plr, blr, P, tl, first_patch, d_patch_ids, total, divisor, (__half*)d_xin_hi, (__half*)d_xin_lo,
       add_offset);
 }
 
-// add: run the ADD instances with add_offset (finite; checked by the caller)
+// the instance for (add, chips); the chip form exists for the range form only
+template <typename T, bool IDS>
+static void launch_prep16_of(bool add, bool chips, PrepSource s0, PrepSource s1, PrepSource s2, int nsrc, int plr, int blr,
+                             int P, Tiling tl, int first_patch, const int* d_patch_ids, long long total, float divisor,
+                             float add_offset, void* d_xin_hi, void* d_xin_lo, cudaStream_t st) {
+  if (!IDS && chips) {
+    if (add) launch_prep16<T, false, true, true>(s0, s1, s2, nsrc, plr, blr, P, tl, first_patch, nullptr, total, divisor,
+                                                 add_offset, d_xin_hi, d_xin_lo, st);
+    else launch_prep16<T, false, false, true>(s0, s1, s2, nsrc, plr, blr, P, tl, first_patch, nullptr, total, divisor,
+                                              add_offset, d_xin_hi, d_xin_lo, st);
+  } else if (add) {
+    launch_prep16<T, IDS, true, false>(s0, s1, s2, nsrc, plr, blr, P, tl, first_patch, d_patch_ids, total, divisor,
+                                       add_offset, d_xin_hi, d_xin_lo, st);
+  } else {
+    launch_prep16<T, IDS, false, false>(s0, s1, s2, nsrc, plr, blr, P, tl, first_patch, d_patch_ids, total, divisor,
+                                        add_offset, d_xin_hi, d_xin_lo, st);
+  }
+}
+
+// add: run the ADD instances with add_offset (finite; checked by the caller).  num_chips >= 0: the images are stacks of
+// num_chips same-size chips and [first_patch, first_patch + num_patches) a range of their flat filled-patch list (CHIPS
+// instances; IDS is false); -1: one image.
 template <bool IDS>
 static int prep16_from_images(const char* name, const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype,
                               int H, int W, int patch, int border, int first_patch, const int* d_patch_ids, int num_patches,
-                              float divisor, bool add, float add_offset, void* d_xin_hi, void* d_xin_lo, void* stream) {
+                              float divisor, bool add, float add_offset, void* d_xin_hi, void* d_xin_lo, void* stream,
+                              int num_chips = -1) {
   DSEN2_REQUIRE(d_img10 && d_img20 && d_xin_hi && d_xin_lo && (!IDS || d_patch_ids), DSEN2_E_BADARG, "%s: null pointer", name);
   DSEN2_REQUIRE(img_dtype == DSEN2_IMG_F32 || img_dtype == DSEN2_IMG_U16, DSEN2_E_BADARG,
                 "%s: img_dtype must be DSEN2_IMG_F32 or DSEN2_IMG_U16 (got %d)", name, img_dtype);
@@ -362,9 +406,16 @@ static int prep16_from_images(const char* name, const void* d_img10, const void*
   const int plr = patch / r, blr = border / r, gh = H / r, gw = W / r;
   DSEN2_REQUIRE(gh + 2 * blr >= plr && gw + 2 * blr >= plr, DSEN2_E_BADARG,
                 "%s: image %dx%d smaller than one patch (%d)", name, H, W, patch);
-  if (num_patches == 0) return 0;
   const Tiling tl = make_tiling(gh, gw, plr, blr);
-  DSEN2_REQUIRE(IDS || first_patch + num_patches <= (tl.k_i + 1) * (tl.k_j + 1), DSEN2_E_BADARG,
+  const bool chips = num_chips >= 0;
+  if (chips) {
+    const long long flat = (long long)num_chips * tl.n_i * tl.n_j;
+    DSEN2_REQUIRE(flat < (1LL << 31) && (long long)first_patch + num_patches <= flat, DSEN2_E_BADARG,
+                  "%s: patch range [%d,%lld) outside the %lld filled patches of %d chips", name, first_patch,
+                  (long long)first_patch + num_patches, flat, num_chips);
+  }
+  if (num_patches == 0) return 0;
+  DSEN2_REQUIRE(IDS || chips || first_patch + num_patches <= (tl.k_i + 1) * (tl.k_j + 1), DSEN2_E_BADARG,
                 "%s: patch range [%d,%d) exceeds the %d allocated patches", name, first_patch,
                 first_patch + num_patches, (tl.k_i + 1) * (tl.k_j + 1));
   PrepSource s0{d_img10, H, W, r, 1};
@@ -373,17 +424,12 @@ static int prep16_from_images(const char* name, const void* d_img10, const void*
   const long long total = (long long)num_patches * patch * patch;
   const int nsrc = d_img60 ? 3 : 2;
   const cudaStream_t st = (cudaStream_t)stream;
-  if (img_dtype == DSEN2_IMG_U16) {
-    if (add) launch_prep16<uint16_t, IDS, true>(s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
-                                                divisor, add_offset, d_xin_hi, d_xin_lo, st);
-    else launch_prep16<uint16_t, IDS, false>(s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
-                                             divisor, 0.f, d_xin_hi, d_xin_lo, st);
-  } else {
-    if (add) launch_prep16<float, IDS, true>(s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
-                                             divisor, add_offset, d_xin_hi, d_xin_lo, st);
-    else launch_prep16<float, IDS, false>(s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
-                                          divisor, 0.f, d_xin_hi, d_xin_lo, st);
-  }
+  if (img_dtype == DSEN2_IMG_U16)
+    launch_prep16_of<uint16_t, IDS>(add, chips, s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
+                                    divisor, add ? add_offset : 0.f, d_xin_hi, d_xin_lo, st);
+  else
+    launch_prep16_of<float, IDS>(add, chips, s0, s1, s2, nsrc, plr, blr, patch, tl, first_patch, d_patch_ids, total,
+                                 divisor, add ? add_offset : 0.f, d_xin_hi, d_xin_lo, st);
   return check_launch(name);
 }
 
@@ -412,6 +458,18 @@ extern "C" int dsen2_prep16_from_images_offset(const void* d_img10, const void* 
                                     num_patches, divisor, true, add_offset, d_xin_hi, d_xin_lo, stream);
   return prep16_from_images<false>(name, d_img10, d_img20, d_img60, img_dtype, H, W, patch, border, first_patch, nullptr,
                                    num_patches, divisor, true, add_offset, d_xin_hi, d_xin_lo, stream);
+}
+
+extern "C" int dsen2_prep16_from_chips(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype,
+                                       int num_chips, int H, int W, int patch, int border, int first_patch, int num_patches,
+                                       float divisor, int add, float add_offset, void* d_xin_hi, void* d_xin_lo,
+                                       void* stream) {
+  const char* name = "dsen2_prep16_from_chips";
+  DSEN2_REQUIRE(num_chips >= 0, DSEN2_E_BADARG, "%s: num_chips %d < 0", name, num_chips);
+  DSEN2_REQUIRE(add == 0 || add == 1, DSEN2_E_BADARG, "%s: add must be 0 or 1 (got %d)", name, add);
+  DSEN2_REQUIRE(!add || isfinite(add_offset), DSEN2_E_BADARG, "%s: add_offset must be finite", name);
+  return prep16_from_images<false>(name, d_img10, d_img20, d_img60, img_dtype, H, W, patch, border, first_patch, nullptr,
+                                   num_patches, divisor, add != 0, add_offset, d_xin_hi, d_xin_lo, stream, num_chips);
 }
 
 extern "C" int dsen2_pack_head16_weights(const float* d_hwio, int cin, int feature_size, void* d_packed, void* stream) {

@@ -21,6 +21,12 @@ expects DN = 10000 x reflectance.  With ``add_offset=a`` every band value x of t
 (uint16, or float32 as staged), becomes fl32(x + a) before the preparation, and every output value f becomes fl32(f - a):
 the output is in the product's own convention (quantised after that for uint16 output).  Nodata is still decided on the
 stored values, and nodata pixels are written as the stored v.
+
+Chip stacks (an extension): 4-D inputs (N, H, W, 4), (N, H/2, W/2, 6)[, (N, H/6, W/6, 2)] are N same-size scenes, the
+datasets of machine learning (BigEarthNet 120 x 120, SEN12MS 256 x 256).  The output is (N, H, W, Cout), and chip i of it
+is bit for bit what the 3-D call on chip i returns, for every ``out_dtype`` / ``add_offset``; but every device launch
+runs the patches of many chips.  Patches are numbered over the stack, chip * ppc + patch with ppc the filled patches of
+one chip, and a launch may straddle chips.  All float32 or all uint16; ``nodata`` is not supported with stacks.
 """
 
 import math
@@ -223,6 +229,60 @@ def active_patches(d10, d20, d60=None, nodata=0, first_patch=0, num_patches=None
     return _active(d10, d20, d60, first_patch, num_patches, nodata)
 
 
+def _stack_geometry(model, shapes, dtypes, nodata):
+    """(N, H, W, ppc) of a chip stack with images of ``shapes`` and element types ``dtypes`` (numpy names), ppc the filled
+    patches of one chip.  Rejected with ``ValueError``: ``nodata``, a network without resBlocks, leading sizes that
+    differ, shapes other than (N, H/d, W/d, C), mixed or other element types, and chips the 3-D path rejects: sizes that
+    are not multiples of the ratio, chips smaller than one patch stride (112 px at 20 m, 168 px at 60 m)."""
+    if nodata is not None:
+        raise ValueError("nodata is not supported with chip stacks")
+    if not model.xin16:
+        raise ValueError("chip stacks need a network with resBlocks (num_layers > 0)")
+    if len(set(dtypes)) != 1 or dtypes[0] not in ('float32', 'uint16'):
+        raise ValueError("chip stack images must all be float32 or all be uint16, got %s" % (list(dtypes),))
+    if any(len(sh) != 4 for sh in shapes) or len({int(sh[0]) for sh in shapes}) != 1:
+        raise ValueError("chip stacks must be 4-D with the same number of chips, got shapes %s" % (list(shapes),))
+    g = _GEOM[len(shapes) == 3]
+    r, P, B = g['ratio'], g['patch'], g['border']
+    N, H, W = (int(v) for v in shapes[0][:3])
+    if H % r or W % r:
+        raise ValueError("10 m chip size %dx%d must be a multiple of %d" % (H, W, r))
+    for sh, div, c in zip(shapes, (1, 2, 6), model.in_channels):
+        if tuple(int(v) for v in sh) != (N, H // div, W // div, c):
+            raise ValueError("expected a chip stack of shape %s, got %s" % ((N, H // div, W // div, c), tuple(sh)))
+    if min(H, W) < P - 2 * B:
+        raise ValueError("chips of %dx%d are smaller than one patch stride (%d)" % (H, W, P - 2 * B))
+    return N, H, W, patch_counts(H // r, W // r, P // r, B // r)[1]
+
+
+def _super_resolve_chips(model, d10, d20, d60, first_patch, num_patches, out, device_batch, timers, nodata, out_dtype,
+                         add_offset):
+    import torch
+    # rejected before the device is touched (add_offset: by the caller)
+    u16 = check_out_dtype(out_dtype, model)
+    imgs = [t for t in (d10, d20, d60) if t is not None]
+    N, H, W, ppc = _stack_geometry(model, [tuple(t.shape) for t in imgs], [str(t.dtype)[len('torch.'):] for t in imgs],
+                                   nodata)
+    g = _GEOM[d60 is not None]
+    shape = (N, H, W, model.out_channels)
+    _check_out(out, shape, torch.uint16 if u16 else torch.float32, "out")
+    if num_patches is None:
+        num_patches = N * ppc - first_patch
+    if first_patch < 0 or num_patches < 0 or first_patch + num_patches > N * ppc:
+        raise ValueError("patch range [%d, %d) outside the %d patches of %d chips"
+                         % (first_patch, first_patch + num_patches, N * ppc, N))
+    _capi.require_cuda()
+    if out is None:
+        out = _zeros_canvas(torch, shape, u16, d10.device)
+    if device_batch is None:
+        device_batch = default_device_batch(W, g['patch'], g['border'])
+    for p0 in range(first_patch, first_patch + num_patches, device_batch):
+        nb = min(device_batch, first_patch + num_patches - p0)
+        model.forward_images(d10, d20, d60, g['patch'], g['border'], p0, nb, out, float(SCALE), timers=timers,
+                             add_offset=add_offset)
+    return out
+
+
 def super_resolve_device(model, d10, d20, d60=None, first_patch=0, num_patches=None, out=None, device_batch=None,
                          timers=None, nodata=None, out_dtype=None, add_offset=None):
     """Device-level pipeline.  d10/d20(/d60): CUDA HWC tensors, all float32 or all uint16.  Processes patches
@@ -230,8 +290,14 @@ def super_resolve_device(model, d10, d20, d60=None, first_patch=0, num_patches=N
     patches.py:32-39 are never read by recompose_images, so they are skipped) and writes the pixels those
     patches own into ``out`` (H, W, Cout) of ``out_dtype`` (torch.float32 when None, or torch.uint16: see the module
     docstring; allocated zero-filled if None).  ``nodata``: see the module docstring; the active patches are found on
-    the device, and their number is the one value read back.  ``add_offset``: see the module docstring."""
+    the device, and their number is the one value read back.  ``add_offset``: see the module docstring.
+
+    Chip stacks (4-D images, module docstring): ``first_patch`` / ``num_patches`` index the flat patch list of the stack
+    (chip * ppc + patch), ``out`` is (N, H, W, Cout), and a device batch may straddle chips."""
     add_offset = check_add_offset(add_offset, model)
+    if d10.dim() == 4:
+        return _super_resolve_chips(model, d10, d20, d60, first_patch, num_patches, out, device_batch, timers, nodata,
+                                    out_dtype, add_offset)
     torch = _capi.require_cuda()
     u16 = check_out_dtype(out_dtype, model)
     nodata = check_nodata(nodata, model, d10.dtype == torch.uint16 or u16)
@@ -284,6 +350,13 @@ class _Slot:
         self.out = torch.empty((out_elems,), dtype=out_dtype).pin_memory()
         self.ev_h2d, self.ev_d2h = torch.cuda.Event(), torch.cuda.Event()
         self.used_in = self.used_out = False
+
+
+def _staging_pool(torch, dev):
+    """The worker threads that fill and drain the pinned staging slots (numpy releases the GIL for the copies)."""
+    from concurrent.futures import ThreadPoolExecutor
+    return ThreadPoolExecutor(max_workers=4, thread_name_prefix='dsen2-stage', initializer=torch.cuda.set_device,
+                              initargs=(dev,))
 
 
 class HostPipeline:
@@ -437,9 +510,7 @@ class HostPipeline:
                 or self._slots[0].out.numel() < out_elems:
             self._slots = [_Slot(torch, shapes, self.dtype, out_elems, self.out_dtype) for _ in range(self.RING)]
         if self._pool is None:
-            from concurrent.futures import ThreadPoolExecutor
-            self._pool = ThreadPoolExecutor(max_workers=4, thread_name_prefix='dsen2-stage',
-                                            initializer=torch.cuda.set_device, initargs=(self.dev,))
+            self._pool = _staging_pool(torch, self.dev)
         return self._slots
 
     def run_numpy(self, a10, a20, a60=None, out=None, first_patch=0, num_patches=None, timers=None, nodata=None,
@@ -545,6 +616,163 @@ class HostPipeline:
         return out
 
 
+class ChipPipeline:
+    """Host-buffer front end for stacks of same-size chips (module docstring).  The unit is whole chips: a chunk is the
+    chips whose patches fill about one device batch (``default_device_batch``; at least one chip), so its inputs and
+    outputs are contiguous slices of the stacks, one copy per resolution.  Chunk k+1 uploads while chunk k computes and
+    chunk k-1 downloads, through a ring of device chunk buffers: a stack larger than device memory streams through.
+    Pinned torch tensors are copied directly; pageable numpy arrays go through pinned staging slots (``_Slot``) filled and
+    drained by worker threads, as in ``HostPipeline.run_numpy``.  ``dtype`` / ``out_dtype`` as for ``HostPipeline``.
+    Reusable across calls of one chip shape and any number of chips."""
+
+    RING = 3
+
+    def __init__(self, model, H, W, run_60=False, device=None, chunk_chips=None, dtype=None, out_dtype=None):
+        u16 = check_out_dtype(out_dtype, model)
+        torch = _capi.require_cuda()
+        self.torch, self.model, self.run_60 = torch, model, run_60
+        self.H, self.W = int(H), int(W)
+        self.dtype = torch.float32 if dtype is None else dtype
+        self.out_dtype = torch.uint16 if u16 else torch.float32
+        self.divs = (1, 2, 6) if run_60 else (1, 2)
+        in_shapes = [(1, self.H // d, self.W // d, c) for d, c in zip(self.divs, model.in_channels)]
+        _, _, _, self.ppc = _stack_geometry(model, in_shapes, [str(self.dtype)[len('torch.'):]] * len(in_shapes), None)
+        g = _GEOM[run_60]
+        self.device_batch = default_device_batch(self.W, g['patch'], g['border'])
+        self.chunk = int(chunk_chips) if chunk_chips else max(1, self.device_batch // self.ppc)
+        self.in_shapes = [(self.chunk,) + s[1:] for s in in_shapes]
+        self.out_shape = (self.chunk, self.H, self.W, model.out_channels)
+        self.dev = torch.device('cuda', torch.cuda.current_device()) if device is None else device
+        # no zero fill: the chips of a chunk own every pixel of their canvases
+        self.d_in = [[torch.empty(s, dtype=self.dtype, device=self.dev) for s in self.in_shapes] for _ in range(self.RING)]
+        self.d_out = [torch.empty(self.out_shape, dtype=self.out_dtype, device=self.dev) for _ in range(self.RING)]
+        self.ev_free = [torch.cuda.Event() for _ in range(self.RING)]      # the last download from a ring entry
+        self.up, self.down = torch.cuda.Stream(self.dev), torch.cuda.Stream(self.dev)
+        self._slots, self._pool = None, None
+
+    def _check(self, srcs, dtype_names):
+        N, _, _, _ = _stack_geometry(self.model, [tuple(a.shape) for a in srcs], dtype_names, None)
+        if tuple(srcs[0].shape[1:3]) != (self.H, self.W):
+            raise ValueError("chips of %dx%d do not match the pipeline's %dx%d" % (*srcs[0].shape[1:3], self.H, self.W))
+        return N
+
+    def _chunks(self, N):
+        return [(c0, min(N, c0 + self.chunk)) for c0 in range(0, N, self.chunk)]
+
+    def _compute(self, e, n, timers, add_offset):
+        """The network over the n chips of ring entry e, on the current stream."""
+        d = [t[:n] for t in self.d_in[e]] + [None] * (3 - len(self.divs))
+        super_resolve_device(self.model, *d, out=self.d_out[e][:n], device_batch=self.device_batch, timers=timers,
+                             out_dtype=self.out_dtype, add_offset=add_offset)
+
+    def run(self, h10, h20, h60=None, hout=None, timers=None, add_offset=None):
+        """Pinned torch stacks in (dtype = the pipeline's), pinned (N, H, W, Cout) tensor of ``out_dtype`` out."""
+        add_offset = check_add_offset(add_offset, self.model)
+        torch = self.torch
+        srcs = [h10, h20] + ([h60] if self.run_60 else [])
+        if any(h.dtype != self.dtype for h in srcs):
+            raise ValueError("host image dtype does not match the pipeline's %s" % self.dtype)
+        N = self._check(srcs, [str(h.dtype)[len('torch.'):] for h in srcs])
+        if hout is None:
+            hout = torch.empty((N,) + self.out_shape[1:], dtype=self.out_dtype).pin_memory()
+        _check_out(hout, (N,) + self.out_shape[1:], self.out_dtype, "hout")
+        main = torch.cuda.current_stream(self.dev)
+        self.up.wait_stream(main)
+        self.down.wait_stream(main)
+        for k, (c0, c1) in enumerate(self._chunks(N)):
+            e = k % self.RING
+            with torch.cuda.stream(self.up):
+                if k >= self.RING:
+                    self.up.wait_event(self.ev_free[e])     # chunk k - RING has been computed and downloaded
+                for d, h in zip(self.d_in[e], srcs):
+                    d[:c1 - c0].copy_(h[c0:c1], non_blocking=True)
+                ev_up = torch.cuda.Event()
+                ev_up.record(self.up)
+            main.wait_event(ev_up)
+            self._compute(e, c1 - c0, timers, add_offset)
+            ev_c = torch.cuda.Event()
+            ev_c.record(main)
+            self.down.wait_event(ev_c)
+            with torch.cuda.stream(self.down):
+                hout[c0:c1].copy_(self.d_out[e][:c1 - c0], non_blocking=True)
+                self.ev_free[e].record(self.down)
+        main.wait_stream(self.down)
+        return hout
+
+    def run_numpy(self, a10, a20, a60=None, out=None, timers=None, add_offset=None):
+        """Pageable numpy stacks in -> numpy (N, H, W, Cout) array of ``out_dtype`` out (allocated if None).  The stacks'
+        element type must be float32 or uint16; a type that is not the pipeline's is cast while it is staged."""
+        add_offset = check_add_offset(add_offset, self.model)
+        torch = self.torch
+        srcs = [a10, a20] + ([a60] if self.run_60 else [])
+        N = self._check(srcs, [a.dtype.name for a in srcs])
+        np_out = np.dtype(_np_dtype_of(torch, self.out_dtype))
+        if out is None:
+            out = np.empty((N,) + self.out_shape[1:], np_out)
+        _check_out(out, (N,) + self.out_shape[1:], np_out, "out")
+        chunks = self._chunks(N)
+        if not chunks:
+            return out
+        if self._slots is None:
+            out_elems = int(np.prod(self.out_shape))
+            self._slots = [_Slot(torch, self.in_shapes, self.dtype, out_elems, self.out_dtype) for _ in range(self.RING)]
+            self._pool = _staging_pool(torch, self.dev)
+        slots = self._slots
+
+        def stage_in(k):
+            slot = slots[k % self.RING]
+            if slot.used_in:
+                slot.ev_h2d.synchronize()            # the previous upload from this slot has left it
+            c0, c1 = chunks[k]
+            for buf, a in zip(slot.inp, srcs):
+                buf[:c1 - c0].numpy()[...] = a[c0:c1]
+
+        def drain(k, part, parts, ev, src):
+            ev.synchronize()
+            c0, c1 = chunks[k]
+            a, b = c0 + (c1 - c0) * part // parts, c0 + (c1 - c0) * (part + 1) // parts
+            if b > a:
+                out[a:b] = src[a - c0:b - c0]
+
+        main = torch.cuda.current_stream(self.dev)
+        self.up.wait_stream(main)
+        self.down.wait_stream(main)
+        fin = {k: self._pool.submit(stage_in, k) for k in range(min(self.RING, len(chunks)))}
+        fout = {}
+        for k, (c0, c1) in enumerate(chunks):
+            e, n = k % self.RING, c1 - c0
+            slot = slots[e]
+            fin.pop(k).result()
+            with torch.cuda.stream(self.up):
+                if k >= self.RING:
+                    self.up.wait_event(self.ev_free[e])
+                for d, buf in zip(self.d_in[e], slot.inp):
+                    d[:n].copy_(buf[:n], non_blocking=True)
+                slot.ev_h2d.record(self.up)
+                slot.used_in = True
+            main.wait_event(slot.ev_h2d)
+            if k + self.RING < len(chunks):
+                fin[k + self.RING] = self._pool.submit(stage_in, k + self.RING)
+            self._compute(e, n, timers, add_offset)
+            ev_c = torch.cuda.Event()
+            ev_c.record(main)
+            self.down.wait_event(ev_c)
+            for f in fout.pop(k - self.RING, ()):    # the slot's previous contents have been copied out
+                f.result()
+            dst = slot.out[:n * int(np.prod(self.out_shape[1:]))].view((n,) + self.out_shape[1:])
+            with torch.cuda.stream(self.down):
+                dst.copy_(self.d_out[e][:n], non_blocking=True)
+                slot.ev_d2h.record(self.down)
+                self.ev_free[e].record(self.down)
+            src = dst.numpy()
+            fout[k] = [self._pool.submit(drain, k, part, 2, slot.ev_d2h, src) for part in range(2)]
+        for fs in fout.values():
+            for f in fs:
+                f.result()
+        main.wait_stream(self.down)
+        return out
+
+
 _pipe_cache = {}
 
 
@@ -559,6 +787,40 @@ def _pipeline_for(model, H, W, run_60, dtype, out_dtype):
             _pipe_cache.clear()
         pipe = _pipe_cache[key] = HostPipeline(model, H, W, run_60=run_60, dtype=dtype, out_dtype=out_dtype)
     return pipe
+
+
+_chip_pipe_cache = {}
+
+
+def _chip_pipeline_for(model, H, W, run_60, dtype, out_dtype):
+    """ChipPipeline objects (device chunk ring + pinned staging ring), kept for the last chip shapes used like
+    ``_pipeline_for``, so a caller that works through a dataset stack after stack pays the allocations once."""
+    torch = _capi.require_cuda()
+    key = (id(model), H, W, run_60, dtype, out_dtype, torch.cuda.current_device())
+    pipe = _chip_pipe_cache.get(key)
+    if pipe is None or pipe.model is not model:
+        if len(_chip_pipe_cache) >= 2:
+            _chip_pipe_cache.clear()
+        pipe = _chip_pipe_cache[key] = ChipPipeline(model, H, W, run_60=run_60, dtype=dtype, out_dtype=out_dtype)
+    return pipe
+
+
+def _run_chips(model, arrays, out=None, nodata=None, out_dtype=np.float32, add_offset=None):
+    # rejected before the device is touched
+    u16 = check_out_dtype(out_dtype, model)
+    add_offset = check_add_offset(add_offset, model)
+    arrays = [np.asarray(a) for a in arrays]
+    N, H, W, _ = _stack_geometry(model, [a.shape for a in arrays], [a.dtype.name for a in arrays], nodata)
+    np_out = np.dtype(np.uint16 if u16 else np.float32)
+    _check_out(out, (N, H, W, model.out_channels), np_out, "out")
+    if N == 0:
+        return np.empty((0, H, W, model.out_channels), np_out) if out is None else out
+    torch = _capi.require_cuda()
+    dtype = torch.uint16 if arrays[0].dtype == np.uint16 else torch.float32
+    pipe = _chip_pipeline_for(model, H, W, len(arrays) == 3, dtype, torch.uint16 if u16 else torch.float32)
+    res = pipe.run_numpy(*arrays, out=out, add_offset=add_offset)
+    torch.cuda.current_stream().synchronize()
+    return res
 
 
 def _run(model, arrays, out=None, nodata=None, out_dtype=np.float32, add_offset=None):
@@ -594,16 +856,20 @@ def DSen2_20(d10, d20, deep=False, model=None, out=None, nodata=None, out_dtype=
     ``nodata`` the input value of pixels without data (module docstring): they come out as ``nodata`` and empty patches are
     skipped; ``out_dtype`` np.uint16: digital numbers, rounded and saturated on the device (module docstring);
     ``add_offset`` the radiometric offset of the product (-1000 for processing baseline 04.00 and later; module docstring):
-    removed from the inputs and restored on the output, on the device."""
+    removed from the inputs and restored on the output, on the device.  Chip stacks: d10 (N,H,W,4), d20 (N,H/2,W/2,6),
+    all float32 or all uint16 -> (N,H,W,6) (module docstring)."""
     input_shape = ((4, None, None), (6, None, None))
     if model is None:
         model = _load_model(input_shape, deep, run_60=False)
-    return _run(model, [d10, d20], out, nodata, out_dtype, add_offset)
+    run = _run_chips if np.ndim(d10) == 4 else _run
+    return run(model, [d10, d20], out, nodata, out_dtype, add_offset)
 
 
 def DSen2_60(d10, d20, d60, deep=False, model=None, out=None, nodata=None, out_dtype=np.float32, add_offset=None):
-    """supres.py:33-50.  + d60 (H/6,W/6,2) -> (H,W,2) float32 (or ``out_dtype``)."""
+    """supres.py:33-50.  + d60 (H/6,W/6,2) -> (H,W,2) float32 (or ``out_dtype``).  Chip stacks: + d60 (N,H/6,W/6,2) ->
+    (N,H,W,2)."""
     input_shape = ((4, None, None), (6, None, None), (2, None, None))
     if model is None:
         model = _load_model(input_shape, deep, run_60=True)
-    return _run(model, [d10, d20, d60], out, nodata, out_dtype, add_offset)
+    run = _run_chips if np.ndim(d10) == 4 else _run
+    return run(model, [d10, d20, d60], out, nodata, out_dtype, add_offset)

@@ -262,6 +262,26 @@ int dsen2_conv_tail16_stitch_offset(const void* d_x_hi, const void* d_x_lo, cons
                                     int n, int P, int first_patch, const int* d_patch_ids, int border, int img_h, int img_w,
                                     float mul, float add_offset, int canvas_dtype, int avoid, void* d_canvas, void* stream);
 
+/* Chip stacks (an extension: datasets of many small same-size scenes, e.g. 120 x 120 or 256 x 256 chips).  The images are
+ * stacks (num_chips, H, W, 4), (num_chips, H/2, W/2, 6) and, for the 60 m path, (num_chips, H/6, W/6, 2), contiguous; the
+ * canvas is (num_chips, img_h, img_w, cout).  Patches are numbered over the whole stack, g = chip * ppc + p, with ppc the
+ * FILLED patches of one chip (dsen2_patch_counts' second count, n_i * n_j) and p the patch's index in the chip's own tiling,
+ * so one call can run [first_patch, first_patch + num_patches) across chip boundaries.  Each chip is tiled, prepared and
+ * stitched exactly as the single-image entry points do it for that image (the same geometry is rejected), so the
+ * prepared input of a patch and the pixels it writes are bit-identical to theirs; a patch writes only into its own chip.
+ * The offset is an explicit switch: add = 0 runs the arithmetic of dsen2_prep16_from_images / dsen2_conv_tail16_stitch(_u16),
+ * add = 1 that of the _offset entry points with the finite add_offset (-0 + 0 is +0, so an add of 0 is not "no offset").
+ * DSEN2_E_BADARG also for num_chips < 0, add not 0 / 1, and a range outside [0, num_chips * ppc) (num_chips * ppc < 2^31).
+ * There is no id-list form.                                                                                          */
+int dsen2_prep16_from_chips(const void* d_img10, const void* d_img20, const void* d_img60, int img_dtype, int num_chips,
+                            int H, int W, int patch, int border, int first_patch, int num_patches, float divisor, int add,
+                            float add_offset, void* d_xin_hi, void* d_xin_lo, void* stream);
+/* canvas_dtype DSEN2_IMG_F32 / DSEN2_IMG_U16; avoid as dsen2_conv_tail16_stitch_u16 (-1 for a float canvas). */
+int dsen2_conv_tail16_stitch_chips(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                   const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
+                                   int n, int P, int first_patch, int border, int num_chips, int img_h, int img_w, float mul,
+                                   int add, float add_offset, int canvas_dtype, int avoid, void* d_canvas, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Nodata (csrc/nodata.cu; an extension: the reference super-resolves nodata like data).  Images, img_dtype, H, W, patch
  * and border as dsen2_prep16_from_images (d_img60 == NULL: 20 m path); `nodata` is the fill value v (not NaN).  Output pixel

@@ -465,6 +465,38 @@ class S2Model:
                 ptr(canvas), st), name))
         return canvas
 
+    def forward_scenes(self, table, patch_scene, num_scenes, total, run_60, img_dtype, u16, patch, border, first_patch, n,
+                       mul, timers=None, add_offset=None):
+        """Fused tile pipeline over a scene list (scenes of any sizes): patches [first_patch, first_patch+n) of the flat
+        list first_i + p are prepared, run through the network and stitched into their scenes' canvases.  ``table``: the
+        device copy of a ``dsen2_scene_table`` (uint8 CUDA tensor), ``patch_scene`` its patch -> scene map (int32 CUDA
+        tensor of ``total`` entries), ``num_scenes`` / ``total`` / ``run_60`` as the table was built.  ``img_dtype``:
+        ``_capi.IMG_F32`` / ``IMG_U16`` of every scene's images; ``u16``: the canvases are uint16.  ``add_offset`` as for
+        ``forward_images`` (``dsen2_prep16_from_scenes``, ``dsen2_conv_tail16_stitch_scenes``)."""
+        torch = _capi.require_cuda()
+        if not self.xin16:
+            raise _capi.DSen2Error("forward_scenes needs a network with resblocks (num_layers > 0)")
+        if not (patch_scene.is_cuda and patch_scene.dtype == torch.int32 and patch_scene.is_contiguous()
+                and patch_scene.numel() >= total and table.is_cuda):
+            raise ValueError("table and patch_scene must be CUDA tensors (patch_scene: contiguous int32, %d entries)" % total)
+        dev = table.device
+        wts, biases, _wp, _bp = self._ensure_packed(dev)
+        if n == 0:
+            return
+        lib, ptr = _capi.lib(), _capi.ptr
+        buf = self._buffers(dev, n, patch, reuse_larger=True)      # chunks of a scene list have any patch count
+        add, a = (0, 0.0) if add_offset is None else (1, float(add_offset))
+        with torch.cuda.device(dev):
+            st = _capi.stream_ptr()
+            self._timed(timers, 'prep', n, lambda: _capi.check(lib.dsen2_prep16_from_scenes(
+                ptr(table), ptr(patch_scene), num_scenes, total, img_dtype, int(run_60), patch, border, first_patch, n,
+                float(mul), add, a, ptr(buf['xin_hi']), ptr(buf['xin_lo']), st), "dsen2_prep16_from_scenes"))
+            self._trunk(buf, wts, biases, n, patch, st, timers)
+            self._timed(timers, 'conv_tail', n, lambda: _capi.check(lib.dsen2_conv_tail16_stitch_scenes(
+                *self._tail_args(buf, wts, biases), self.feature_size, n, patch, first_patch, border, ptr(table),
+                ptr(patch_scene), num_scenes, total, float(mul), add, a, _capi.IMG_U16 if u16 else _capi.IMG_F32, -1, st),
+                "dsen2_conv_tail16_stitch_scenes"))
+
     def launches_per_forward(self):
         return 2 * self.num_layers + 3             # input preparation + first layer + 2 per resblock + last layer
 

@@ -75,7 +75,16 @@ SIGNATURES = {
     "dsen2_conv_tail16_stitch_chips": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                                c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, c_int,
                                                c_float, c_int, c_int, c_void_p, c_void_p]),
-    "dsen2_conv_resq256": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p,
+    "dsen2_scene_table_bytes": (c_size_t, [c_int]),
+    "dsen2_scene_table": (c_int, [c_int, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p),
+                                  POINTER(c_int), POINTER(c_int), c_int, c_int, c_void_p, c_void_p, c_longlong,
+                                  POINTER(c_longlong)]),
+    "dsen2_prep16_from_scenes": (c_int, [c_void_p, c_void_p, c_int, c_longlong, c_int, c_int, c_int, c_int, c_int, c_int,
+                                         c_float, c_int, c_float, c_void_p, c_void_p, c_void_p]),
+    "dsen2_conv_tail16_stitch_scenes": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
+                                                c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_longlong,
+                                                c_float, c_int, c_float, c_int, c_int, c_void_p]),
+    "dsen2_conv_resq256":(c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p,
                                    c_void_p, c_void_p]),
     "dsen2_conv_tail": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                                 c_int, c_void_p, c_void_p]),

@@ -48,13 +48,26 @@ struct TailParams {
   const __half* skip_lo;
   int skip_ch0, cout;
   float out_mul;
-  void* out;                          // float, or (stitched canvas only) uint16_t: the OutT of the kernel instance
+  // Instances with SCENES take the scene list in the fields of the single-canvas geometry they do not read (each scene's
+  // canvas, size and grid are in its table entry): the struct stays at 128 bytes.  A larger parameter struct is read
+  // through its address instead of with direct parameter loads, which changes the code of every other instance.
+  union {
+    void* out;                        // float, or (stitched canvas only) uint16_t: the OutT of the kernel instance
+    const SceneGeom* scenes;          // SCENES: the scene table (num_scenes entries)
+  };
   int tail_mode;                      // 0: NCHW (n, cout, H, W) predictions; 1: stitched HWC canvas
-  int first_patch, img_h, img_w, border, grid_ny, grid_nx;
-  const int* patch_ids;               // stitching form with IDS: batch entry b is patch patch_ids[b], not first_patch + b
+  int first_patch;
+  union { int img_h; int num_scenes; };
+  union { int img_w; int num_flat; };  // SCENES: entries of patch_scene, the flat patches of the list
+  int border, grid_ny, grid_nx;
+  union {
+    const int* patch_ids;             // stitching form with IDS: batch entry b is patch patch_ids[b], not first_patch + b
+    const int* patch_scene;           // SCENES: the scene of every flat patch
+  };
   int avoid;                          // uint16 canvas: a value the network must not write (the nodata value), -1 none
   float add_offset;                   // instances with ADD: subtracted from every stitched value (the product's radiometric offset)
 };
+static_assert(sizeof(TailParams) == 128, "TailParams grew: see the comment on its unions");
 
 // The uint16 (digital number) canvas value of the float f the float canvas receives: NaN -> 0, else rint(clip(f, 0, 65535))
 // (round half to even; fmaxf returns 0 for a NaN f).  A value equal to `avoid` (>= 0) moves one step away from it, so a
@@ -83,7 +96,9 @@ __device__ __forceinline__ int tail_stitch_tile_of(int y, int size, int S, int n
 
 // CHIPS (stitching form): the canvas is a stack of same-size chip canvases (num_chips, img_h, img_w, cout) and
 // first_patch + b indexes the flat list chip * ppc + patch (ppc = grid_ny * grid_nx); ownership stays inside the chip.
-template <int KPM, bool IDS, typename OutT, bool ADD, bool CHIPS>
+// SCENES (stitching form): first_patch + b indexes the flat patch list of a scene list; locate() resolves the tile's scene
+// once (the map p.patch_scene, then its table entry) and writes into that scene's own canvas with its own geometry.
+template <int KPM, bool IDS, typename OutT, bool ADD, bool CHIPS, bool SCENES>
 __global__ void __launch_bounds__(kTThreads, 1)
 conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
                          const __grid_constant__ CUtensorMap tm_w, const TailParams p) {
@@ -187,8 +202,10 @@ conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid
     // Where a tile's pixel of this thread goes (and whether this patch owns it), and its global skip.  The skip is loaded
     // ONE TILE AHEAD: a dependent global load inside the per-tile chain (wait, copy, barrier, gather, barrier) would put
     // a DRAM latency on every tile -- measured: the tile took 4.4 us for 1.2 us of MMAs.
+    // SCENES: `out` receives the canvas of the tile's scene (the other instances write into p.out)
     struct Dest { bool write; long long obase, ostride; };
-    auto locate = [&](uint32_t tile, Dest& d, __half (&sk_hi)[(kTMaxCout + 1) / 2], __half (&sk_lo)[(kTMaxCout + 1) / 2]) {
+    auto locate = [&](uint32_t tile, Dest& d, __half (&sk_hi)[(kTMaxCout + 1) / 2], __half (&sk_lo)[(kTMaxCout + 1) / 2],
+                      OutT*& out) {
       const uint32_t rowi = tile / (uint32_t)p.tiles_x;
       const int tx = (int)(tile - rowi * (uint32_t)p.tiles_x) + p.tx0;
       const int b = (int)(rowi / (uint32_t)p.tiles_y), ty = (int)(rowi - (uint32_t)b * (uint32_t)p.tiles_y);
@@ -199,6 +216,26 @@ conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid
         if (p.tail_mode == 0) {
           d.ostride = (long long)p.H * p.W;
           d.obase = (long long)b * p.cout * d.ostride + (long long)y * p.W + x;
+        } else if constexpr (SCENES) {
+          // a scene or patch index outside the table writes nothing
+          const int S = p.H - 2 * p.border;
+          const int patch = p.first_patch + b;
+          const int sc = patch < p.num_flat ? __ldg(p.patch_scene + patch) : -1;
+          d.write = sc >= 0 && sc < p.num_scenes;
+          if (d.write) {
+            const SceneGeom* g = p.scenes + sc;
+            const int img_h = g->src[0].H, img_w = g->src[0].W, gny = g->tl.n_i, gnx = g->tl.n_j;
+            const int q = patch - g->first;
+            const int pty = q / gnx, ptx = q - pty * gnx;
+            const int gy = min(pty * S, img_h - S) + y - p.border;
+            const int gx = min(ptx * S, img_w - S) + x - p.border;
+            d.write = q >= 0 && q < gny * gnx &&
+                      y >= p.border && y < p.H - p.border && x >= p.border && x < p.W - p.border &&
+                      tail_stitch_tile_of(gy, img_h, S, gny) == pty && tail_stitch_tile_of(gx, img_w, S, gnx) == ptx;
+            d.ostride = 1;
+            d.obase = ((long long)gy * img_w + gx) * p.cout;
+            out = static_cast<OutT*>(g->canvas);
+          }
         } else {
           const int S = p.H - 2 * p.border;
           int patch = IDS ? __ldg(p.patch_ids + b) : p.first_patch + b;
@@ -228,12 +265,13 @@ conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid
       }
     };
     Dest cur, nxt;
+    OutT *cur_out = nullptr, *nxt_out = nullptr;
     __half ch[(kTMaxCout + 1) / 2], cl[(kTMaxCout + 1) / 2], nh[(kTMaxCout + 1) / 2], nl[(kTMaxCout + 1) / 2];
 #pragma unroll
     for (int i = 0; i < (kTMaxCout + 1) / 2; ++i) ch[i] = cl[i] = nh[i] = nl[i] = __float2half_rn(0.f);
-    locate(blockIdx.x, cur, ch, cl);
+    locate(blockIdx.x, cur, ch, cl, cur_out);
     for (uint32_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-      locate(tile + gridDim.x, nxt, nh, nl);                 // next tile's destination and skip loads, in flight during this tile
+      locate(tile + gridDim.x, nxt, nh, nl, nxt_out);                 // next tile's destination and skip loads, in flight during this tile
       const bool write = cur.write;
       const long long obase = cur.obase, ostride = cur.ostride;
       // ---- phase 1: accumulator rows -> shared memory
@@ -274,13 +312,14 @@ conv_tail_swapped_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid
             const float skip = __half2float(ch[i]) + __half2float(cl[i]);
             // Add (DSen2Net.py:38), x SCALE; ADD: - add_offset, back to the product's convention (__fsub_rn is never
             // contracted into an FMA with the multiply)
-            store_out(static_cast<OutT*>(p.out) + obase + (c_lo + i) * ostride,
+            store_out((SCENES ? cur_out : static_cast<OutT*>(p.out)) + obase + (c_lo + i) * ostride,
                       ADD ? __fsub_rn((v + skip) * p.out_mul, p.add_offset) : (v + skip) * p.out_mul, p.avoid);
           }
         }
       }
       asm volatile("bar.sync 1, 256;" ::: "memory");          // the shared-memory copy may be overwritten
       cur = nxt;
+      cur_out = nxt_out;
 #pragma unroll
       for (int i = 0; i < (kTMaxCout + 1) / 2; ++i) { ch[i] = nh[i]; cl[i] = nl[i]; }
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
@@ -310,12 +349,12 @@ __global__ void pack_tail16_weights_kernel(const float* __restrict__ hwio, int F
   }
 }
 
-template <int KPM, bool IDS, typename OutT, bool ADD, bool CHIPS>
+template <int KPM, bool IDS, typename OutT, bool ADD, bool CHIPS, bool SCENES>
 static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_lo, const void* d_w, int sms, cudaStream_t stream) {
   using Cfg = TailCfg<KPM>;
   static bool configured[64] = {};
   if (needs_config(configured)) {
-    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM, IDS, OutT, ADD, CHIPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+    DSEN2_CUDA(cudaFuncSetAttribute(conv_tail_swapped_kernel<KPM, IDS, OutT, ADD, CHIPS, SCENES>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   }
   const int F = KPM * 64;
   CUtensorMap hi, lo, w;
@@ -328,23 +367,25 @@ static int launch_tail(const TailParams& p, const void* d_x_hi, const void* d_x_
   const uint32_t wb[2] = {64, 128};
   if ((rc = make_tmap_f16_sw(&w, d_w, 2, wd, wb, 128)) != 0) return rc;
   const int grid = (int)(p.num_tiles < (uint32_t)sms ? p.num_tiles : (uint32_t)sms);
-  conv_tail_swapped_kernel<KPM, IDS, OutT, ADD, CHIPS><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
+  conv_tail_swapped_kernel<KPM, IDS, OutT, ADD, CHIPS, SCENES><<<grid, kTThreads, Cfg::SMEM_BYTES, stream>>>(hi, lo, w, p);
   return check_launch("conv_tail_swapped");
 }
 
-template <bool IDS, typename OutT, bool ADD, bool CHIPS = false>
+template <bool IDS, typename OutT, bool ADD, bool CHIPS = false, bool SCENES = false>
 static int launch_tail_f(const TailParams& p, int features, const void* d_x_hi, const void* d_x_lo, const void* d_w, int sms,
                          cudaStream_t stream) {
-  return features == 256 ? launch_tail<4, IDS, OutT, ADD, CHIPS>(p, d_x_hi, d_x_lo, d_w, sms, stream)
-                         : launch_tail<2, IDS, OutT, ADD, CHIPS>(p, d_x_hi, d_x_lo, d_w, sms, stream);
+  return features == 256 ? launch_tail<4, IDS, OutT, ADD, CHIPS, SCENES>(p, d_x_hi, d_x_lo, d_w, sms, stream)
+                         : launch_tail<2, IDS, OutT, ADD, CHIPS, SCENES>(p, d_x_hi, d_x_lo, d_w, sms, stream);
 }
 
-// add: run the ADD instances, which subtract p.add_offset from every stitched value; chips: the CHIPS instances (range form)
+// add: run the ADD instances, which subtract p.add_offset from every stitched value; chips: the CHIPS instances (range form);
+// scenes: the SCENES instances (range form), with p.scenes and p.patch_scene set and no d_out (the canvases are in the table)
 template <typename OutT>
 static int tail16_common(TailParams& p, int features, const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
                          const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int n, int H, int W, OutT* d_out,
-                         bool add, void* stream, bool chips = false) {
-  DSEN2_REQUIRE(d_x_hi && d_x_lo && d_w && d_bias && d_xin_hi && d_xin_lo && d_out, DSEN2_E_BADARG, "dsen2_conv_tail16: null pointer");
+                         bool add, void* stream, bool chips = false, bool scenes = false) {
+  DSEN2_REQUIRE(d_x_hi && d_x_lo && d_w && d_bias && d_xin_hi && d_xin_lo && (scenes || d_out), DSEN2_E_BADARG,
+                "dsen2_conv_tail16: null pointer");
   DSEN2_REQUIRE(features == 128 || features == 256, DSEN2_E_BADARG, "dsen2_conv_tail16: feature_size must be 128 or 256 (got %d)",
                 features);
   DSEN2_REQUIRE(n >= 0 && H > 0 && W > 0 && cout > 0 && cout <= kTMaxCout && skip_ch0 >= 0 && skip_ch0 + cout <= 16, DSEN2_E_BADARG,
@@ -370,8 +411,12 @@ static int tail16_common(TailParams& p, int features, const void* d_x_hi, const 
   p.num_tiles = (uint32_t)tiles;
   p.bias = d_bias;
   p.skip_hi = (const __half*)d_xin_hi; p.skip_lo = (const __half*)d_xin_lo; p.skip_ch0 = skip_ch0;
-  p.cout = cout; p.out = d_out;
+  p.cout = cout;
+  if (!scenes) p.out = d_out;
   const cudaStream_t st = (cudaStream_t)stream;
+  if (scenes)
+    return add ? launch_tail_f<false, OutT, true, false, true>(p, features, d_x_hi, d_x_lo, d_w, sms, st)
+               : launch_tail_f<false, OutT, false, false, true>(p, features, d_x_hi, d_x_lo, d_w, sms, st);
   if (chips)
     return add ? launch_tail_f<false, OutT, true, true>(p, features, d_x_hi, d_x_lo, d_w, sms, st)
                : launch_tail_f<false, OutT, false, true>(p, features, d_x_hi, d_x_lo, d_w, sms, st);
@@ -517,4 +562,42 @@ extern "C" int dsen2_conv_tail16_stitch_chips(const void* d_x_hi, const void* d_
   return tail16_stitch<float>(d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, feature_size, n, P,
                               first_patch, nullptr, border, img_h, img_w, mul, -1, (float*)d_canvas, stream, add != 0, a,
                               num_chips);
+}
+
+extern "C" int dsen2_conv_tail16_stitch_scenes(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                               const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout,
+                                               int feature_size, int n, int P, int first_patch, int border,
+                                               const void* d_table, const int* d_patch_scene, int num_scenes,
+                                               long long total_patches, float mul, int add, float add_offset,
+                                               int canvas_dtype, int avoid, void* stream) {
+  const char* name = "dsen2_conv_tail16_stitch_scenes";
+  DSEN2_REQUIRE(d_table && d_patch_scene, DSEN2_E_BADARG, "%s: null pointer", name);
+  DSEN2_REQUIRE(num_scenes >= 0, DSEN2_E_BADARG, "%s: num_scenes %d < 0", name, num_scenes);
+  DSEN2_REQUIRE(add == 0 || add == 1, DSEN2_E_BADARG, "%s: add must be 0 or 1 (got %d)", name, add);
+  DSEN2_REQUIRE(!add || isfinite(add_offset), DSEN2_E_BADARG, "%s: add_offset must be finite", name);
+  DSEN2_REQUIRE(canvas_dtype == DSEN2_IMG_F32 || canvas_dtype == DSEN2_IMG_U16, DSEN2_E_BADARG,
+                "%s: canvas_dtype must be DSEN2_IMG_F32 or DSEN2_IMG_U16 (got %d)", name, canvas_dtype);
+  DSEN2_REQUIRE(canvas_dtype == DSEN2_IMG_U16 || avoid == -1, DSEN2_E_BADARG,
+                "%s: avoid must be -1 for a float canvas (got %d)", name, avoid);
+  DSEN2_REQUIRE(avoid >= -1 && avoid <= 65535, DSEN2_E_BADARG, "%s: avoid %d outside [-1, 65535]", name, avoid);
+  const int S = P - 2 * border;
+  DSEN2_REQUIRE(P > 0 && border >= 0 && S > 0, DSEN2_E_BADARG, "%s: bad stitch geometry (P %d border %d)", name, P, border);
+  DSEN2_REQUIRE(total_patches >= 0 && total_patches < (1LL << 31) && first_patch >= 0 && n >= 0 &&
+                (long long)first_patch + n <= total_patches, DSEN2_E_BADARG,
+                "%s: patch range [%d,%lld) outside the %lld patches of %d scenes", name, first_patch,
+                (long long)first_patch + n, total_patches, num_scenes);
+  TailParams p{};
+  p.tail_mode = 1;
+  p.out_mul = mul;
+  p.avoid = avoid;
+  p.add_offset = add ? add_offset : 0.f;
+  p.first_patch = first_patch; p.border = border;
+  p.scenes = static_cast<const SceneGeom*>(d_table);
+  p.patch_scene = d_patch_scene;
+  p.num_scenes = num_scenes; p.num_flat = (int)total_patches;
+  if (canvas_dtype == DSEN2_IMG_U16)
+    return tail16_common<uint16_t>(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, P, P,
+                                   nullptr, add != 0, stream, false, true);
+  return tail16_common<float>(p, feature_size, d_x_hi, d_x_lo, d_w, d_bias, d_xin_hi, d_xin_lo, skip_ch0, cout, n, P, P,
+                              nullptr, add != 0, stream, false, true);
 }

@@ -9,6 +9,7 @@
 //                               (supres.py:23-24,42-44) with the arithmetic of the standalone kernels.
 //   dsen2_prep16_from_images_offset : the same with a radiometric offset added to every loaded band value first
 //   dsen2_prep16_from_chips   : the same from stacks of same-size chips, patches indexed chip * ppc + patch
+//   dsen2_prep16_from_scenes  : the same from lists of scenes of any sizes, through a scene table (dsen2_scene_table)
 // Training step (and networks without resblocks): "x_in", 64 channels per pixel = the three HORIZONTAL taps of the first
 // 3x3 convolution pre-gathered, x_in[n][y][x][t*16 + c] = X[n][c][y][x + t - 1] (zero outside the patch), because the
 // first layer's weight-gradient GEMM wants 128-byte pixel rows (dsen2_prep_from_patches).
@@ -35,13 +36,6 @@ __device__ __forceinline__ void store32(__half* dst, const Half16& h) {
   d[0] = s[0];
   d[1] = s[1];
 }
-
-struct PrepSource {
-  const void* img;    // (H, W, C) HWC, float32 or uint16 DN; C = 4 / 6 / 2 for the 10 / 20 / 60 m inputs
-  int H, W;
-  int ratio;          // source pixels per tiling-grid pixel
-  int s;              // upsampling factor to the 10 m patch (1 = none)
-};
 
 // A band value as the arithmetic below takes it: the stored element, or with ADD fl32(x + add_offset) (the radiometric
 // offset of Sentinel-2 products since processing baseline 04.00).  ADD is a template switch, not an add of 0: -0 + 0 is +0.
@@ -125,11 +119,15 @@ __device__ __forceinline__ PrepSource chip_source(PrepSource s, int chip) {
 // every loaded band value (ld_band); it is the last parameter, so the other instances keep their parameter layout.
 // CHIPS: the images are stacks of same-size chips and first_patch + b indexes the flat list chip * ppc + patch, with ppc =
 // n_i * n_j the filled patches of one chip; the chip and its patch are resolved per patch index with one 32-bit division.
-template <typename T, bool IDS, bool ADD, bool CHIPS>
+// SCENES: first_patch + b indexes the flat patch list of a scene list of any sizes; the scene comes from the map
+// patch_scene (num_flat entries) and its images and tiling from its entry of the scene table (num_scenes entries) instead
+// of s0..s2 / tl.  The table and the map are the last parameters, so the other instances keep their parameter layout.
+template <typename T, bool IDS, bool ADD, bool CHIPS, bool SCENES>
 __global__ void prep16_from_images_kernel(PrepSource s0, PrepSource s1, PrepSource s2, int nsrc, int plr, int blr, int P,
                                           Tiling tl, int first_patch, const int* __restrict__ ids, long long total,
                                           float divisor, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
-                                          float add_offset) {
+                                          float add_offset, const SceneGeom* __restrict__ scenes,
+                                          const int* __restrict__ patch_scene, int num_scenes, int num_flat) {
   const int PP = P * P;
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
@@ -146,7 +144,23 @@ __global__ void prep16_from_images_kernel(PrepSource s0, PrepSource s1, PrepSour
 #pragma unroll
     for (int c = 0; c < 16; ++c) v[c] = 0.f;
     // surplus patches of the allocated stack stay zero (patches.py:32-39), and so do ids outside the tiling
-    if ((!IDS || patch >= 0) && patch < tl.n_i * tl.n_j) {
+    if constexpr (SCENES) {
+      // a scene or patch index outside the table prepares a zero input
+      const int sc = patch >= 0 && patch < num_flat ? __ldg(patch_scene + patch) : -1;
+      if (sc >= 0 && sc < num_scenes) {
+        const SceneGeom* g = scenes + sc;
+        const Tiling t = g->tl;
+        const int q = patch - g->first;
+        if (q >= 0 && q < t.n_i * t.n_j) {
+          const int ti = q / t.n_j, tj = q - ti * t.n_j;
+          const int si = ti < t.k_i ? ti * t.stride : t.last_i;
+          const int sj = tj < t.k_j ? tj * t.stride : t.last_j;
+          prep_gather<T, 4, 0, ADD>(g->src[0], si, sj, plr, blr, y, x, divisor, add_offset, v);
+          prep_gather<T, 6, 4, ADD>(g->src[1], si, sj, plr, blr, y, x, divisor, add_offset, v);
+          if (nsrc == 3) prep_gather<T, 2, 10, ADD>(g->src[2], si, sj, plr, blr, y, x, divisor, add_offset, v);
+        }
+      }
+    } else if ((!IDS || patch >= 0) && patch < tl.n_i * tl.n_j) {
       const int ti = patch / tl.n_j, tj = patch - ti * tl.n_j;
       const int si = ti < tl.k_i ? ti * tl.stride : tl.last_i;
       const int sj = tj < tl.k_j ? tj * tl.stride : tl.last_j;
@@ -354,14 +368,15 @@ extern "C" int dsen2_prep16_from_patches(const float* d_x0, int c0, const float*
   return check_launch("prep16_from_patches");
 }
 
-template <typename T, bool IDS, bool ADD, bool CHIPS>
+template <typename T, bool IDS, bool ADD, bool CHIPS, bool SCENES = false>
 static void launch_prep16(PrepSource s0, PrepSource s1, PrepSource s2, int nsrc, int plr, int blr, int P, Tiling tl,
                           int first_patch, const int* d_patch_ids, long long total, float divisor, float add_offset,
-                          void* d_xin_hi, void* d_xin_lo, cudaStream_t stream) {
+                          void* d_xin_hi, void* d_xin_lo, cudaStream_t stream, const SceneGeom* d_scenes = nullptr,
+                          const int* d_patch_scene = nullptr, int num_scenes = 0, int num_flat = 0) {
   const int block = 256;
-  prep16_from_images_kernel<T, IDS, ADD, CHIPS><<<grid_for(total, block), block, 0, stream>>>(
+  prep16_from_images_kernel<T, IDS, ADD, CHIPS, SCENES><<<grid_for(total, block), block, 0, stream>>>(
       s0, s1, s2, nsrc, plr, blr, P, tl, first_patch, d_patch_ids, total, divisor, (__half*)d_xin_hi, (__half*)d_xin_lo,
-      add_offset);
+      add_offset, d_scenes, d_patch_scene, num_scenes, num_flat);
 }
 
 // the instance for (add, chips); the chip form exists for the range form only
@@ -470,6 +485,105 @@ extern "C" int dsen2_prep16_from_chips(const void* d_img10, const void* d_img20,
   DSEN2_REQUIRE(!add || isfinite(add_offset), DSEN2_E_BADARG, "%s: add_offset must be finite", name);
   return prep16_from_images<false>(name, d_img10, d_img20, d_img60, img_dtype, H, W, patch, border, first_patch, nullptr,
                                    num_patches, divisor, add != 0, add_offset, d_xin_hi, d_xin_lo, stream, num_chips);
+}
+
+extern "C" size_t dsen2_scene_table_bytes(int num_scenes) {
+  return num_scenes > 0 ? (size_t)num_scenes * sizeof(SceneGeom) : 0;
+}
+
+extern "C" int dsen2_scene_table(int num_scenes, const void* const* d_img10s, const void* const* d_img20s,
+                                 const void* const* d_img60s, void* const* d_canvases, const int* Hs, const int* Ws, int patch,
+                                 int border, void* h_table, int* h_patch_scene, long long max_patches,
+                                 long long* total_patches) {
+  const char* name = "dsen2_scene_table";
+  DSEN2_REQUIRE(num_scenes >= 0, DSEN2_E_BADARG, "%s: num_scenes %d < 0", name, num_scenes);
+  DSEN2_REQUIRE(total_patches && (num_scenes == 0 || (d_img10s && d_img20s && d_canvases && Hs && Ws && h_table)),
+                DSEN2_E_BADARG, "%s: null pointer", name);
+  const int r = d_img60s ? 6 : 2;                // the tiling grid is the coarsest input (patches.py:45-53,114-122)
+  DSEN2_REQUIRE(patch > 0 && border >= 0 && patch % r == 0 && border % r == 0 && patch > 2 * border, DSEN2_E_BADARG,
+                "%s: patch %d / border %d must be multiples of %d", name, patch, border, r);
+  const int plr = patch / r, blr = border / r, S = patch - 2 * border;
+  SceneGeom* table = static_cast<SceneGeom*>(h_table);
+  long long first = 0;
+  for (int i = 0; i < num_scenes; ++i) {
+    const int H = Hs[i], W = Ws[i];
+    DSEN2_REQUIRE(d_img10s[i] && d_img20s[i] && (!d_img60s || d_img60s[i]) && d_canvases[i], DSEN2_E_BADARG,
+                  "%s: scene %d: null pointer", name, i);
+    DSEN2_REQUIRE(H > 0 && W > 0 && H % r == 0 && W % r == 0, DSEN2_E_BADARG,
+                  "%s: scene %d: 10 m size %dx%d must be a multiple of %d", name, i, H, W, r);
+    DSEN2_REQUIRE(H / r + 2 * blr >= plr && W / r + 2 * blr >= plr, DSEN2_E_BADARG,
+                  "%s: scene %d: image %dx%d smaller than one patch (%d)", name, i, H, W, patch);
+    DSEN2_REQUIRE(H >= S && W >= S, DSEN2_E_BADARG, "%s: scene %d: image %dx%d smaller than one patch stride (%d)", name,
+                  i, H, W, S);
+    SceneGeom g{};
+    g.src[0] = PrepSource{d_img10s[i], H, W, r, 1};
+    g.src[1] = PrepSource{d_img20s[i], H / 2, W / 2, r / 2, 2};
+    g.src[2] = PrepSource{d_img60s ? d_img60s[i] : nullptr, H / 6, W / 6, 1, 6};
+    g.tl = make_tiling(H / r, W / r, plr, blr);
+    g.canvas = d_canvases[i];
+    const long long count = (long long)g.tl.n_i * g.tl.n_j;
+    DSEN2_REQUIRE(first + count < (1LL << 31), DSEN2_E_BADARG, "%s: %lld patches or more in the flat list (at most 2^31 - 1)",
+                  name, first + count);
+    g.first = (int)first;
+    if (h_patch_scene) {
+      DSEN2_REQUIRE(first + count <= max_patches, DSEN2_E_BADARG,
+                    "%s: the patch -> scene map has %lld entries, the scene list more", name, max_patches);
+      for (long long k = first; k < first + count; ++k) h_patch_scene[k] = i;
+    }
+    table[i] = g;
+    first += count;
+  }
+  *total_patches = first;
+  return 0;
+}
+
+extern "C" int dsen2_prep16_from_scenes(const void* d_table, const int* d_patch_scene, int num_scenes,
+                                        long long total_patches, int img_dtype, int run_60, int patch, int border,
+                                        int first_patch, int num_patches, float divisor, int add, float add_offset,
+                                        void* d_xin_hi, void* d_xin_lo, void* stream) {
+  const char* name = "dsen2_prep16_from_scenes";
+  DSEN2_REQUIRE(d_table && d_patch_scene && d_xin_hi && d_xin_lo, DSEN2_E_BADARG, "%s: null pointer", name);
+  DSEN2_REQUIRE(num_scenes >= 0, DSEN2_E_BADARG, "%s: num_scenes %d < 0", name, num_scenes);
+  DSEN2_REQUIRE(img_dtype == DSEN2_IMG_F32 || img_dtype == DSEN2_IMG_U16, DSEN2_E_BADARG,
+                "%s: img_dtype must be DSEN2_IMG_F32 or DSEN2_IMG_U16 (got %d)", name, img_dtype);
+  DSEN2_REQUIRE(run_60 == 0 || run_60 == 1, DSEN2_E_BADARG, "%s: run_60 must be 0 or 1 (got %d)", name, run_60);
+  DSEN2_REQUIRE(add == 0 || add == 1, DSEN2_E_BADARG, "%s: add must be 0 or 1 (got %d)", name, add);
+  DSEN2_REQUIRE(!add || isfinite(add_offset), DSEN2_E_BADARG, "%s: add_offset must be finite", name);
+  const int r = run_60 ? 6 : 2;
+  DSEN2_REQUIRE(patch > 0 && border >= 0 && patch % r == 0 && border % r == 0 && patch > 2 * border, DSEN2_E_BADARG,
+                "%s: patch %d / border %d must be multiples of %d", name, patch, border, r);
+  DSEN2_REQUIRE(divisor != 0.f, DSEN2_E_BADARG, "%s: bad patch range / divisor", name);
+  DSEN2_REQUIRE(total_patches >= 0 && total_patches < (1LL << 31) && first_patch >= 0 && num_patches >= 0 &&
+                (long long)first_patch + num_patches <= total_patches, DSEN2_E_BADARG,
+                "%s: patch range [%d,%lld) outside the %lld patches of %d scenes", name, first_patch,
+                (long long)first_patch + num_patches, total_patches, num_scenes);
+  DSEN2_REQUIRE(((uintptr_t)d_xin_hi % 16) == 0 && ((uintptr_t)d_xin_lo % 16) == 0, DSEN2_E_ALIGN,
+                "%s: outputs must be 16-byte aligned", name);
+  if (num_patches == 0) return 0;
+  const PrepSource none{};
+  const Tiling tl{};
+  const long long total = (long long)num_patches * patch * patch;
+  const int nsrc = run_60 ? 3 : 2, plr = patch / r, blr = border / r;
+  const cudaStream_t st = (cudaStream_t)stream;
+  const SceneGeom* scenes = static_cast<const SceneGeom*>(d_table);
+  const int flat = (int)total_patches;
+  const float a = add ? add_offset : 0.f;
+  if (img_dtype == DSEN2_IMG_U16) {
+    if (add) launch_prep16<uint16_t, false, true, false, true>(none, none, none, nsrc, plr, blr, patch, tl, first_patch, nullptr,
+                                                               total, divisor, a, d_xin_hi, d_xin_lo, st, scenes,
+                                                               d_patch_scene, num_scenes, flat);
+    else launch_prep16<uint16_t, false, false, false, true>(none, none, none, nsrc, plr, blr, patch, tl, first_patch, nullptr,
+                                                            total, divisor, a, d_xin_hi, d_xin_lo, st, scenes,
+                                                            d_patch_scene, num_scenes, flat);
+  } else {
+    if (add) launch_prep16<float, false, true, false, true>(none, none, none, nsrc, plr, blr, patch, tl, first_patch, nullptr,
+                                                            total, divisor, a, d_xin_hi, d_xin_lo, st, scenes,
+                                                            d_patch_scene, num_scenes, flat);
+    else launch_prep16<float, false, false, false, true>(none, none, none, nsrc, plr, blr, patch, tl, first_patch, nullptr,
+                                                         total, divisor, a, d_xin_hi, d_xin_lo, st, scenes, d_patch_scene,
+                                                         num_scenes, flat);
+  }
+  return check_launch(name);
 }
 
 extern "C" int dsen2_pack_head16_weights(const float* d_hwio, int cin, int feature_size, void* d_packed, void* stream) {

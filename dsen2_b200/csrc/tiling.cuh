@@ -44,6 +44,24 @@ __host__ __device__ inline Tiling make_tiling(int grid_h, int grid_w, int patch_
   return t;
 }
 
+struct PrepSource {
+  const void* img;    // (H, W, C) HWC, float32 or uint16 DN; C = 4 / 6 / 2 for the 10 / 20 / 60 m inputs
+  int H, W;
+  int ratio;          // source pixels per tiling-grid pixel
+  int s;              // upsampling factor to the 10 m patch (1 = none)
+};
+
+// One scene of a scene list (dsen2_scene_table): everything the preparation and the last layer take from the single
+// geometry of a 3-D call, precomputed on the host, so that a kernel resolves a flat patch's scene with loads only (the
+// patch -> scene map, then this entry).  The 10 m size is src[0].H x src[0].W; the stitch grid is tl.n_i x tl.n_j.
+struct SceneGeom {
+  PrepSource src[3];  // 10, 20, 60 m images as the 3-D preparation takes them (src[2].img null on the 20 m path)
+  Tiling tl;          // the scene's own tiling: n_i * n_j filled patches
+  int first;          // flat index of the scene's first patch (prefix sum of the filled-patch counts before it)
+  void* canvas;       // (H, W, cout) output of the scene: float or uint16, the canvas type of the call
+};
+static_assert(sizeof(SceneGeom) == 112, "the scene table layout is private, but its size is what dsen2_scene_table_bytes reports");
+
 __device__ __forceinline__ int sym_index(int j, int n) {  // numpy pad(mode='symmetric')
   if (j < 0) j = -j - 1;
   if (j >= n) j = 2 * n - 1 - j;

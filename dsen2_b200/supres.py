@@ -27,6 +27,14 @@ datasets of machine learning (BigEarthNet 120 x 120, SEN12MS 256 x 256).  The ou
 is bit for bit what the 3-D call on chip i returns, for every ``out_dtype`` / ``add_offset``; but every device launch
 runs the patches of many chips.  Patches are numbered over the stack, chip * ppc + patch with ppc the filled patches of
 one chip, and a launch may straddle chips.  All float32 or all uint16; ``nodata`` is not supported with stacks.
+
+Scene lists (an extension): lists of N scenes of any sizes, d10s[i] (H_i, W_i, 4), d20s[i] (H_i/2, W_i/2, 6)[, d60s[i]
+(H_i/6, W_i/6, 2)] -- the chips of a grid with its remainder row and column, windows around parcels, ROIs of several
+products (``DSen2_20_scenes``, ``DSen2_60_scenes``, ``super_resolve_scenes_device``, ``ScenePipeline``).  The output is a
+list of (H_i, W_i, Cout) arrays, and scene i of it is bit for bit what the 3-D call on scene i returns, for every
+``out_dtype`` / ``add_offset``.  Patches are numbered over the list, first_i + p with first_i the filled patches of the
+scenes before i, and a launch may straddle scenes: a scene table (``dsen2_scene_table``) gives each launch every scene's
+geometry.  All float32 or all uint16; ``nodata`` is not supported with scene lists.
 """
 
 import math
@@ -773,6 +781,312 @@ class ChipPipeline:
         return out
 
 
+def _scene_geometry(model, shapes, dtypes, nodata):
+    """(run_60, [(H_i, W_i)]) of a scene list: ``shapes`` / ``dtypes`` (numpy names) hold one list per resolution (10, 20
+    [, 60] m).  Rejected with ``ValueError``: ``nodata``, a network without resBlocks, lists of different lengths, a scene
+    whose shapes do not fit its (H, W), mixed or other element types, and scenes the 3-D path rejects: sizes that are not
+    multiples of the ratio, scenes smaller than one patch stride (112 px at 20 m, 168 px at 60 m)."""
+    if nodata is not None:
+        raise ValueError("nodata is not supported with scene lists")
+    if not model.xin16:
+        raise ValueError("scene lists need a network with resBlocks (num_layers > 0)")
+    if len({len(sh) for sh in shapes}) != 1:
+        raise ValueError("scene lists of different lengths: %s" % [len(sh) for sh in shapes])
+    names = {d for ds in dtypes for d in ds}
+    if len(names) > 1 or not names <= {'float32', 'uint16'}:
+        raise ValueError("scene images must all be float32 or all be uint16, got %s" % sorted(names))
+    run_60 = len(shapes) == 3
+    g = _GEOM[run_60]
+    r, S = g['ratio'], g['patch'] - 2 * g['border']
+    sizes = []
+    for i, sh in enumerate(zip(*shapes)):
+        if len(sh[0]) != 3:
+            raise ValueError("scene %d: expected HWC images, got shape %s" % (i, tuple(sh[0])))
+        H, W = int(sh[0][0]), int(sh[0][1])
+        if H % r or W % r:
+            raise ValueError("scene %d: 10 m size %dx%d must be a multiple of %d" % (i, H, W, r))
+        for s_, div, c in zip(sh, (1, 2, 6), model.in_channels):
+            if tuple(int(v) for v in s_) != (H // div, W // div, c):
+                raise ValueError("scene %d: expected an image of shape %s, got %s" % (i, (H // div, W // div, c), tuple(s_)))
+        if min(H, W) < S:
+            raise ValueError("scene %d: %dx%d is smaller than one patch stride (%d)" % (i, H, W, S))
+        sizes.append((H, W))
+    return run_60, sizes
+
+
+def _check_outs(outs, sizes, C, dtype, what):
+    if outs is None:
+        return
+    if len(outs) != len(sizes):
+        raise ValueError("%s must be a list of %d arrays, got %d" % (what, len(sizes), len(outs)))
+    for o, (H, W) in zip(outs, sizes):
+        _check_out(o, (H, W, C), dtype, what)
+
+
+def _scene_table(run_60, sizes, p10, p20, p60, pout):
+    """Host scene table (uint8 numpy array), patch -> scene map (int32 numpy array) and flat patch count of a list whose
+    scenes' images and canvases are at the device addresses p10[i], p20[i], p60[i] (run_60) and pout[i].  The tiling is
+    ``dsen2_scene_table``'s: the first call counts the patches, the second fills the map."""
+    import ctypes
+    lib, N = _capi.lib(), len(sizes)
+    g = _GEOM[run_60]
+    arr = lambda t, vs: (t * max(1, N))(*vs)
+    args = [arr(ctypes.c_void_p, p10), arr(ctypes.c_void_p, p20), arr(ctypes.c_void_p, p60) if run_60 else None,
+            arr(ctypes.c_void_p, pout), arr(ctypes.c_int, [h for h, _ in sizes]), arr(ctypes.c_int, [w for _, w in sizes]),
+            g['patch'], g['border']]
+    table = np.empty(max(1, lib.dsen2_scene_table_bytes(N)), np.uint8)
+    total = ctypes.c_longlong(0)
+    _capi.check(lib.dsen2_scene_table(N, *args, table.ctypes.data, None, 0, ctypes.byref(total)), "dsen2_scene_table")
+    pmap = np.empty(max(1, total.value), np.int32)
+    _capi.check(lib.dsen2_scene_table(N, *args, table.ctypes.data, pmap.ctypes.data, pmap.size, ctypes.byref(total)),
+                "dsen2_scene_table")
+    return table, pmap, total.value
+
+
+def super_resolve_scenes_device(model, d10s, d20s, d60s=None, outs=None, first_patch=0, num_patches=None,
+                                device_batch=None, timers=None, out_dtype=None, add_offset=None):
+    """Scene lists on the device (module docstring).  d10s / d20s (/ d60s): lists of contiguous CUDA HWC tensors, all
+    float32 or all uint16.  Processes patches [first_patch, first_patch+num_patches) of the flat patch list of the scenes
+    (first_i + p) and writes the pixels they own into ``outs[i]`` (H_i, W_i, Cout) of ``out_dtype`` (torch.float32 when
+    None, or torch.uint16).  When ``outs`` is None, one flat canvas is allocated (zero-filled unless the range is the whole
+    list, whose scenes own every pixel of their canvases) and a list of per-scene views of it is returned.  A device
+    batch, and the range, may straddle scenes; ranks shard a list by contiguous ranges."""
+    add_offset = check_add_offset(add_offset, model)
+    u16 = check_out_dtype(out_dtype, model)
+    lists = [list(d10s), list(d20s)] + ([list(d60s)] if d60s is not None else [])
+    run_60, sizes = _scene_geometry(model, [[tuple(t.shape) for t in l] for l in lists],
+                                    [[str(t.dtype)[len('torch.'):] for t in l] for l in lists], None)
+    import torch
+    dtype = torch.uint16 if u16 else torch.float32
+    C = model.out_channels
+    _check_outs(outs, sizes, C, dtype, "outs")
+    if any(not (t.is_cuda and t.is_contiguous()) for l in lists for t in l) or \
+            (outs is not None and any(not (o.is_cuda and o.is_contiguous()) for o in outs)):
+        raise ValueError("scene images and outputs must be contiguous CUDA tensors")
+    if not sizes:
+        return [] if outs is None else outs
+    _capi.require_cuda()
+    g = _GEOM[run_60]
+    dev = lists[0][0].device
+    if outs is None:
+        full = first_patch == 0 and num_patches is None
+        flat = (torch.empty if full else torch.zeros)((sum(H * W for H, W in sizes) * C,), dtype=dtype, device=dev)
+        outs, o = [], 0
+        for H, W in sizes:
+            outs.append(flat[o:o + H * W * C].view(H, W, C))
+            o += H * W * C
+    pl = lambda l: [t.data_ptr() for t in l]
+    table, pmap, total = _scene_table(run_60, sizes, pl(lists[0]), pl(lists[1]), pl(lists[2]) if run_60 else None,
+                                      pl(outs))
+    if num_patches is None:
+        num_patches = total - first_patch
+    if first_patch < 0 or num_patches < 0 or first_patch + num_patches > total:
+        raise ValueError("patch range [%d, %d) outside the %d patches of %d scenes"
+                         % (first_patch, first_patch + num_patches, total, len(sizes)))
+    if device_batch is None:
+        device_batch = default_device_batch(max(W for _, W in sizes), g['patch'], g['border'])
+    d_table, d_map = torch.from_numpy(table).to(dev), torch.from_numpy(pmap).to(dev)
+    img_dtype = _capi.IMG_U16 if lists[0][0].dtype == torch.uint16 else _capi.IMG_F32
+    for p0 in range(first_patch, first_patch + num_patches, device_batch):
+        nb = min(device_batch, first_patch + num_patches - p0)
+        model.forward_scenes(d_table, d_map, len(sizes), total, run_60, img_dtype, u16, g['patch'], g['border'], p0, nb,
+                             float(SCALE), timers=timers, add_offset=add_offset)
+    return outs
+
+
+class ScenePipeline:
+    """Host-buffer front end for scene lists (module docstring).  A chunk is consecutive scenes whose patches fill about
+    one device batch (``chunk_patches``, default 300 patches of 128 x 128), and at least one scene.  Its images are packed
+    per resolution into a pinned staging slot (``_Slot``) by worker threads -- scenes may be non-contiguous numpy views,
+    such as windows sliced from a product -- uploaded with one copy per resolution into a ring of device chunk buffers, run
+    on the chunk's own scene table, downloaded as one copy and scattered into the per-scene outputs by the worker threads.
+    Chunk k+1 uploads while chunk k computes and chunk k-1 downloads.  Slots and device buffers are sized for the largest
+    chunk and grow on demand.  ``dtype`` / ``out_dtype`` as for ``HostPipeline``; one pipeline serves lists of any scene
+    sizes."""
+
+    RING = 3
+
+    def __init__(self, model, run_60=False, device=None, chunk_patches=None, dtype=None, out_dtype=None):
+        u16 = check_out_dtype(out_dtype, model)
+        torch = _capi.require_cuda()
+        self.torch, self.model, self.run_60 = torch, model, run_60
+        self.dtype = torch.float32 if dtype is None else dtype
+        if self.dtype not in (torch.float32, torch.uint16):
+            raise ValueError("device images are float32 or uint16")
+        self.out_dtype = torch.uint16 if u16 else torch.float32
+        g = _GEOM[run_60]
+        self.P, self.B, self.r = g['patch'], g['border'], g['ratio']
+        self.divs = (1, 2, 6) if run_60 else (1, 2)
+        self.chunk_patches = int(chunk_patches) if chunk_patches else max(1, (300 * 128 * 128) // (self.P * self.P))
+        self.dev = torch.device('cuda', torch.cuda.current_device()) if device is None else device
+        self.up, self.down = torch.cuda.Stream(self.dev), torch.cuda.Stream(self.dev)
+        self.ev_free = [torch.cuda.Event() for _ in range(self.RING)]      # the last download from a ring entry
+        self._used = [False] * self.RING
+        self._cap = None             # capacity: elements per resolution, output elements, scenes, patches of a chunk
+        self._slots, self._pool, self._counts = None, None, {}
+
+    def _count(self, H, W):
+        if (H, W) not in self._counts:
+            self._counts[(H, W)] = patch_counts(H // self.r, W // self.r, self.P // self.r, self.B // self.r)[1]
+        return self._counts[(H, W)]
+
+    def _plan(self, sizes):
+        """Chunks (s0, s1, patches, per resolution and for the output the element offsets of the chunk's scenes)."""
+        C = self.model.out_channels
+        chunks, s0, n = [], 0, 0
+        for i, (H, W) in enumerate(sizes):
+            n += self._count(H, W)
+            if n >= self.chunk_patches or i == len(sizes) - 1:
+                sz = sizes[s0:i + 1]
+                offs = [[0] + np.cumsum([(h // d) * (w // d) * c for h, w in sz]).tolist()
+                        for d, c in zip(self.divs, self.model.in_channels)]
+                offs.append([0] + np.cumsum([h * w * C for h, w in sz]).tolist())
+                chunks.append((s0, i + 1, n, offs))
+                s0, n = i + 1, 0
+        return chunks
+
+    def _buffers(self, chunks):
+        """Pinned slots and device ring entries that hold the largest chunk of ``chunks`` (grown on demand)."""
+        torch = self.torch
+        need = [max(c[3][j][-1] for c in chunks) for j in range(len(self.divs) + 1)]
+        need += [max(c[1] - c[0] for c in chunks), max(c[2] for c in chunks)]
+        if self._cap is not None and all(a >= b for a, b in zip(self._cap, need)):
+            return
+        if self._cap is not None:                # the previous buffers are dropped: their last copies must have ended
+            need = [max(a, b) for a, b in zip(self._cap, need)]
+            torch.cuda.current_stream(self.dev).wait_stream(self.down)
+            self.down.synchronize()
+        self._cap = need
+        nin, nout, ns, npat = need[:len(self.divs)], need[-3], need[-2], need[-1]
+        tb = _capi.lib().dsen2_scene_table_bytes(ns)
+        self._slots = [_Slot(torch, [(n,) for n in nin], self.dtype, nout, self.out_dtype) for _ in range(self.RING)]
+        for sl in self._slots:
+            sl.table = torch.empty((tb,), dtype=torch.uint8).pin_memory()
+            sl.pmap = torch.empty((npat,), dtype=torch.int32).pin_memory()
+        mk = lambda n, dt: torch.empty((n,), dtype=dt, device=self.dev)
+        self.d_in = [[mk(n, self.dtype) for n in nin] for _ in range(self.RING)]
+        self.d_out = [mk(nout, self.out_dtype) for _ in range(self.RING)]
+        self.d_table = [mk(tb, torch.uint8) for _ in range(self.RING)]
+        self.d_map = [mk(npat, torch.int32) for _ in range(self.RING)]
+        self._used = [False] * self.RING
+        if self._pool is None:
+            self._pool = _staging_pool(torch, self.dev)
+
+    def _check(self, srcs, dtype_names):
+        if len(srcs) != len(self.divs):
+            raise ValueError("this pipeline takes %d image lists" % len(self.divs))
+        return _scene_geometry(self.model, [[tuple(a.shape) for a in l] for l in srcs], dtype_names, None)[1]
+
+    def run(self, h10s, h20s, h60s=None, houts=None, timers=None, add_offset=None):
+        """Lists of pinned torch tensors in (dtype = the pipeline's) -> list of pinned (H_i, W_i, Cout) tensors of
+        ``out_dtype`` (allocated if None; ``houts`` is returned as given)."""
+        add_offset = check_add_offset(add_offset, self.model)
+        torch = self.torch
+        srcs = [list(h10s), list(h20s)] + ([list(h60s)] if self.run_60 else [])
+        if any(h.dtype != self.dtype for l in srcs for h in l):
+            raise ValueError("host image dtype does not match the pipeline's %s" % self.dtype)
+        sizes = self._check(srcs, [[str(h.dtype)[len('torch.'):] for h in l] for l in srcs])
+        C = self.model.out_channels
+        if houts is None:
+            houts = [torch.empty((H, W, C), dtype=self.out_dtype).pin_memory() for H, W in sizes]
+        _check_outs(houts, sizes, C, self.out_dtype, "houts")
+        self._stream([[h.numpy() for h in l] for l in srcs], [o.numpy() for o in houts], sizes, timers, add_offset)
+        return houts
+
+    def run_numpy(self, a10s, a20s, a60s=None, outs=None, timers=None, add_offset=None):
+        """Lists of numpy arrays in (any strides; an element type that is not the pipeline's is cast while it is staged) ->
+        list of numpy (H_i, W_i, Cout) arrays of ``out_dtype`` (allocated if None; ``outs`` is returned as given)."""
+        add_offset = check_add_offset(add_offset, self.model)
+        srcs = [[np.asarray(a) for a in l] for l in [a10s, a20s] + ([a60s] if self.run_60 else [])]
+        sizes = self._check(srcs, [[a.dtype.name for a in l] for l in srcs])
+        np_out = np.dtype(_np_dtype_of(self.torch, self.out_dtype))
+        C = self.model.out_channels
+        if outs is None:
+            outs = [np.empty((H, W, C), np_out) for H, W in sizes]
+        _check_outs(outs, sizes, C, np_out, "outs")
+        self._stream(srcs, outs, sizes, timers, add_offset)
+        return outs
+
+    def _stream(self, srcs, outs, sizes, timers, add_offset):
+        torch = self.torch
+        if not sizes:
+            return
+        chunks = self._plan(sizes)
+        self._buffers(chunks)
+        slots, lib, nres = self._slots, _capi.lib(), len(self.divs)
+        isz = torch.empty((), dtype=self.dtype).element_size()
+        osz = torch.empty((), dtype=self.out_dtype).element_size()
+        img_dtype = _capi.IMG_U16 if self.dtype == torch.uint16 else _capi.IMG_F32
+        u16 = self.out_dtype == torch.uint16
+
+        def stage_in(k):
+            e = k % self.RING
+            slot = slots[e]
+            if slot.used_in:
+                slot.ev_h2d.synchronize()            # the previous upload from this slot (images, table, map) has left it
+            s0, s1, _, offs = chunks[k]
+            for j in range(nres):
+                buf = slot.inp[j].numpy()
+                for i in range(s0, s1):
+                    a = srcs[j][i]
+                    buf[offs[j][i - s0]:offs[j][i - s0 + 1]].reshape(a.shape)[...] = a
+            at = lambda t, o, sz: [t.data_ptr() + v * sz for v in o[:-1]]
+            p = [at(self.d_in[e][j], offs[j], isz) for j in range(nres)]
+            table, pmap, _ = _scene_table(self.run_60, sizes[s0:s1], p[0], p[1], p[2] if self.run_60 else None,
+                                          at(self.d_out[e], offs[-1], osz))
+            slot.table.numpy()[:table.size] = table
+            slot.pmap.numpy()[:pmap.size] = pmap
+
+        def drain(k, part, parts, ev, src):
+            ev.synchronize()
+            s0, s1, _, offs = chunks[k]
+            a, b = s0 + (s1 - s0) * part // parts, s0 + (s1 - s0) * (part + 1) // parts
+            for i in range(a, b):
+                outs[i][...] = src[offs[-1][i - s0]:offs[-1][i - s0 + 1]].reshape(outs[i].shape)
+
+        main = torch.cuda.current_stream(self.dev)
+        self.up.wait_stream(main)
+        self.down.wait_stream(main)
+        fin = {k: self._pool.submit(stage_in, k) for k in range(min(self.RING, len(chunks)))}
+        fout = {}
+        for k, (s0, s1, n, offs) in enumerate(chunks):
+            e = k % self.RING
+            slot = slots[e]
+            fin.pop(k).result()
+            with torch.cuda.stream(self.up):
+                if self._used[e]:
+                    self.up.wait_event(self.ev_free[e])      # the entry's previous chunk has been computed and downloaded
+                for j in range(nres):
+                    self.d_in[e][j][:offs[j][-1]].copy_(slot.inp[j][:offs[j][-1]], non_blocking=True)
+                nt = lib.dsen2_scene_table_bytes(s1 - s0)
+                self.d_table[e][:nt].copy_(slot.table[:nt], non_blocking=True)
+                self.d_map[e][:n].copy_(slot.pmap[:n], non_blocking=True)
+                slot.ev_h2d.record(self.up)
+                slot.used_in = True
+            main.wait_event(slot.ev_h2d)
+            if k + self.RING < len(chunks):
+                fin[k + self.RING] = self._pool.submit(stage_in, k + self.RING)
+            for p0 in range(0, n, self.chunk_patches):
+                self.model.forward_scenes(self.d_table[e], self.d_map[e], s1 - s0, n, self.run_60, img_dtype, u16, self.P,
+                                          self.B, p0, min(self.chunk_patches, n - p0), float(SCALE), timers=timers,
+                                          add_offset=add_offset)
+            ev_c = torch.cuda.Event()
+            ev_c.record(main)
+            self.down.wait_event(ev_c)
+            for f in fout.pop(k - self.RING, ()):    # the slot's previous contents have been copied out
+                f.result()
+            with torch.cuda.stream(self.down):
+                slot.out[:offs[-1][-1]].copy_(self.d_out[e][:offs[-1][-1]], non_blocking=True)
+                slot.ev_d2h.record(self.down)
+                self.ev_free[e].record(self.down)
+            self._used[e] = True
+            fout[k] = [self._pool.submit(drain, k, part, 2, slot.ev_d2h, slot.out.numpy()) for part in range(2)]
+        for fs in fout.values():
+            for f in fs:
+                f.result()
+        main.wait_stream(self.down)
+
+
 _pipe_cache = {}
 
 
@@ -803,6 +1117,41 @@ def _chip_pipeline_for(model, H, W, run_60, dtype, out_dtype):
             _chip_pipe_cache.clear()
         pipe = _chip_pipe_cache[key] = ChipPipeline(model, H, W, run_60=run_60, dtype=dtype, out_dtype=out_dtype)
     return pipe
+
+
+_scene_pipe_cache = {}
+
+
+def _scene_pipeline_for(model, run_60, dtype, out_dtype):
+    """ScenePipeline objects (device chunk ring + pinned staging ring), kept for the last configurations used like
+    ``_chip_pipeline_for``; one serves lists of any scene sizes."""
+    torch = _capi.require_cuda()
+    key = (id(model), run_60, dtype, out_dtype, torch.cuda.current_device())
+    pipe = _scene_pipe_cache.get(key)
+    if pipe is None or pipe.model is not model:
+        if len(_scene_pipe_cache) >= 2:
+            _scene_pipe_cache.clear()
+        pipe = _scene_pipe_cache[key] = ScenePipeline(model, run_60=run_60, dtype=dtype, out_dtype=out_dtype)
+    return pipe
+
+
+def _run_scenes(model, lists, out=None, nodata=None, out_dtype=np.float32, add_offset=None):
+    # rejected before the device is touched
+    u16 = check_out_dtype(out_dtype, model)
+    add_offset = check_add_offset(add_offset, model)
+    lists = [[np.asarray(a) for a in l] for l in lists]
+    run_60, sizes = _scene_geometry(model, [[a.shape for a in l] for l in lists], [[a.dtype.name for a in l] for l in lists],
+                                    nodata)
+    np_out = np.dtype(np.uint16 if u16 else np.float32)
+    _check_outs(out, sizes, model.out_channels, np_out, "out")
+    if not sizes:
+        return [] if out is None else out
+    torch = _capi.require_cuda()
+    dtype = torch.uint16 if lists[0][0].dtype == np.uint16 else torch.float32
+    pipe = _scene_pipeline_for(model, run_60, dtype, torch.uint16 if u16 else torch.float32)
+    res = pipe.run_numpy(*lists, outs=out, add_offset=add_offset)
+    torch.cuda.current_stream().synchronize()
+    return res
 
 
 def _run_chips(model, arrays, out=None, nodata=None, out_dtype=np.float32, add_offset=None):
@@ -873,3 +1222,23 @@ def DSen2_60(d10, d20, d60, deep=False, model=None, out=None, nodata=None, out_d
         model = _load_model(input_shape, deep, run_60=True)
     run = _run_chips if np.ndim(d10) == 4 else _run
     return run(model, [d10, d20, d60], out, nodata, out_dtype, add_offset)
+
+
+def DSen2_20_scenes(d10s, d20s, deep=False, model=None, out=None, out_dtype=np.float32, add_offset=None, nodata=None):
+    """Scene lists (module docstring): d10s[i] (H_i,W_i,4), d20s[i] (H_i/2,W_i/2,6), scenes of any sizes, all float32 or
+    all uint16 (numpy arrays; views sliced from a larger product are fine) -> list of (H_i,W_i,6) arrays of ``out_dtype``,
+    scene i bit for bit ``DSen2_20(d10s[i], d20s[i])``.  ``out``: a list of preallocated outputs, returned as given.  The
+    other arguments as for ``DSen2_20``; ``nodata`` is rejected."""
+    input_shape = ((4, None, None), (6, None, None))
+    if model is None:
+        model = _load_model(input_shape, deep, run_60=False)
+    return _run_scenes(model, [d10s, d20s], out, nodata, out_dtype, add_offset)
+
+
+def DSen2_60_scenes(d10s, d20s, d60s, deep=False, model=None, out=None, out_dtype=np.float32, add_offset=None,
+                    nodata=None):
+    """``DSen2_20_scenes`` for the 60 m path: + d60s[i] (H_i/6,W_i/6,2) -> list of (H_i,W_i,2)."""
+    input_shape = ((4, None, None), (6, None, None), (2, None, None))
+    if model is None:
+        model = _load_model(input_shape, deep, run_60=True)
+    return _run_scenes(model, [d10s, d20s, d60s], out, nodata, out_dtype, add_offset)

@@ -282,6 +282,38 @@ int dsen2_conv_tail16_stitch_chips(const void* d_x_hi, const void* d_x_lo, const
                                    int n, int P, int first_patch, int border, int num_chips, int img_h, int img_w, float mul,
                                    int add, float add_offset, int canvas_dtype, int avoid, void* d_canvas, void* stream);
 
+/* Scene lists (an extension: many scenes of different sizes, e.g. grid chips with their remainders, or windows around
+ * parcels).  Scene i has its own images (H_i, W_i, 4), (H_i/2, W_i/2, 6)[, (H_i/6, W_i/6, 2)] and canvas (H_i, W_i, cout),
+ * each contiguous and element-aligned, in separate allocations or not.  Patches are numbered over the whole list,
+ * g = first_i + p, with first_i the sum of the filled-patch counts of scenes 0..i-1 and p the patch's index in scene i's
+ * own tiling, so one call can run [first_patch, first_patch + num_patches) across scene boundaries.  Each scene is tiled,
+ * prepared and stitched exactly as the single-image entry points do it, so its output is bit-identical to theirs; a patch
+ * writes only into its own scene.
+ *
+ * A scene table describes the list.  dsen2_scene_table fills it on the host (no GPU involved) from the per-scene device
+ * pointers and 10 m sizes: d_img60s NULL is the 20 m path; patch / border as for dsen2_prep16_from_images (128 / 8 at 20 m,
+ * 192 / 12 at 60 m).  It rejects each scene as dsen2_prep16_from_images would (sizes not multiples of the ratio), and a
+ * scene smaller than one patch stride (patch - 2 border), with DSEN2_E_BADARG and the scene's index in the message.  It
+ * writes the flat patch count to *total_patches (< 2^31) and, when h_patch_scene is not NULL, the scene of every flat
+ * patch into h_patch_scene[0, total) (max_patches entries available).  h_table holds dsen2_scene_table_bytes(num_scenes)
+ * bytes; its layout is private to the library and holds device addresses.  The caller copies the table and the map to the
+ * device (an ordinary asynchronous copy) and passes the device copies, with num_scenes, the total and run_60 (0: 20 m,
+ * 1: 60 m, as the table was built), to the two steps below.  add / add_offset, canvas_dtype and avoid as for the _chips
+ * pair.  DSEN2_E_BADARG also for null pointers, num_scenes < 0, add not 0 / 1, and a range outside [0, total) or a total of
+ * 2^31 or more.  A scene or patch index outside the table prepares a zero input and writes nothing.  No id-list form. */
+size_t dsen2_scene_table_bytes(int num_scenes);
+int dsen2_scene_table(int num_scenes, const void* const* d_img10s, const void* const* d_img20s, const void* const* d_img60s,
+                      void* const* d_canvases, const int* Hs, const int* Ws, int patch, int border, void* h_table,
+                      int* h_patch_scene, long long max_patches, long long* total_patches);
+int dsen2_prep16_from_scenes(const void* d_table, const int* d_patch_scene, int num_scenes, long long total_patches,
+                             int img_dtype, int run_60, int patch, int border, int first_patch, int num_patches,
+                             float divisor, int add, float add_offset, void* d_xin_hi, void* d_xin_lo, void* stream);
+int dsen2_conv_tail16_stitch_scenes(const void* d_x_hi, const void* d_x_lo, const void* d_w, const float* d_bias,
+                                    const void* d_xin_hi, const void* d_xin_lo, int skip_ch0, int cout, int feature_size,
+                                    int n, int P, int first_patch, int border, const void* d_table, const int* d_patch_scene,
+                                    int num_scenes, long long total_patches, float mul, int add, float add_offset,
+                                    int canvas_dtype, int avoid, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Nodata (csrc/nodata.cu; an extension: the reference super-resolves nodata like data).  Images, img_dtype, H, W, patch
  * and border as dsen2_prep16_from_images (d_img60 == NULL: 20 m path); `nodata` is the fill value v (not NaN).  Output pixel

@@ -6,7 +6,7 @@ from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_longl
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_lib", "libdsen2_b200.so")
 
-IMG_F32, IMG_U16 = 0, 1
+IMG_F32, IMG_U16, IMG_F64 = 0, 1, 2
 
 # name -> (restype, argtypes); must list every symbol the header declares (checked by tests)
 SIGNATURES = {
@@ -98,6 +98,9 @@ SIGNATURES = {
     "dsen2_mae_grad": (c_int, [c_void_p, c_void_p, c_longlong, c_float, c_void_p, c_void_p, c_void_p]),
     "dsen2_nadam_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong] + [c_float] * 10 + [c_void_p]),
     "dsen2_nadam_step_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p]),
+    "dsen2_image_quality_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "dsen2_image_quality": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p,
+                                    c_size_t, c_void_p, c_void_p]),
 }
 
 

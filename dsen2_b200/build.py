@@ -6,7 +6,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "_lib", "libdsen2_b200.so")
-SOURCES = ["patch_kernels.cu", "prep_kernels.cu", "conv_api.cu", "conv_pair.cu", "conv_tail.cu", "nodata.cu", "train_kernels.cu"]
+SOURCES = ["patch_kernels.cu", "prep_kernels.cu", "conv_api.cu", "conv_pair.cu", "conv_tail.cu", "nodata.cu", "train_kernels.cu",
+           "metrics.cu"]
 
 
 def needs_build():

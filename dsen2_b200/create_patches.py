@@ -161,10 +161,11 @@ def write_patches(data10, data20, data60, name, roi, test_data=False, save_prefi
     print("Success.")
 
 
-def readS2fromFile(data_file, test_data=False, roi_x_y=None, save_prefix="../data/", write_images=False, run_60=False,
-                   true_data=False):
-    """``create_patches.py:19-316``.  ``data_file``: a SAFE directory (its ``MTD_MSIL1C.xml`` is opened through GDAL) or a
-    ``.npz`` product container."""
+def read_bands(data_file, roi_x_y=None, run_60=False, true_data=False):
+    """``create_patches.py:19-205``: the bands of the ROI (rounded to 36-pixel boundaries) of the UTM zone with the largest
+    coverage, 10 / 20 / 60 m, in the product's own dtype -> (data10, data20, data60, (xmin, ymin, xmax, ymax)), or None
+    for an empty region.  ``data_file``: a SAFE directory (its ``MTD_MSIL1C.xml`` is opened through GDAL) or a ``.npz``
+    product container."""
     path = data_file if data_file.endswith('.npz') else data_file + '/MTD_MSIL1C.xml'
     src = open_source(path)
     cands = []
@@ -181,7 +182,7 @@ def readS2fromFile(data_file, test_data=False, roi_x_y=None, save_prefix="../dat
     print("Image size: width=%d x height=%d" % (xmax - xmin + 1, ymax - ymin + 1))
     if xmax < xmin or ymax < ymin:
         print("Invalid region of interest / UTM Zone combination")
-        return 0
+        return None
     ds = src.open(utm_idx)
     (n10, i10), (n20, i20), (n60, i60) = select_bands(ds.descriptions(0), ds.descriptions(1), ds.descriptions(2), run_60)
     for label, names in (("10m", n10), ("20m", n20), ("60m", n60)):
@@ -192,8 +193,19 @@ def readS2fromFile(data_file, test_data=False, roi_x_y=None, save_prefix="../dat
     data60 = ds.read(2, w60, i60) if i60 else None
     if (run_60 or true_data) and data60 is None:
         raise SystemExit("the product has none of the 60 m bands B1 / B9 that --run_60 / --true_data need")
+    return data10, data20, data60, (xmin, ymin, xmax, ymax)
+
+
+def readS2fromFile(data_file, test_data=False, roi_x_y=None, save_prefix="../data/", write_images=False, run_60=False,
+                   true_data=False):
+    """``create_patches.py:19-316``.  ``data_file``: a SAFE directory (its ``MTD_MSIL1C.xml`` is opened through GDAL) or a
+    ``.npz`` product container."""
+    bands = read_bands(data_file, roi_x_y, run_60, true_data)
+    if bands is None:
+        return 0
+    data10, data20, data60, roi = bands
     name = os.path.split(data_file.rstrip('/'))[1]           # :234-238
-    write_patches(data10, data20, data60, name, (xmin, ymin, xmax, ymax), test_data, save_prefix, write_images, run_60, true_data)
+    write_patches(data10, data20, data60, name, roi, test_data, save_prefix, write_images, run_60, true_data)
     return 0
 
 

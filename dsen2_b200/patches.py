@@ -214,22 +214,41 @@ def downPixelAggr(img, SCALE=2):
     img = np.asarray(img)
     if img.ndim == 2:
         img = img[:, :, None]
-    integer = int(np.issubdtype(img.dtype, np.integer))
+    integer = np.issubdtype(img.dtype, np.integer)
     if integer and (img.dtype.itemsize > 2 or (img.size and img.min() < 0)):
         raise ValueError("downPixelAggr: integer images must be uint8 / uint16 / non-negative int16 (exact in float32)")
-    sigma = 1.0 / SCALE
+    d = torch.from_numpy(np.ascontiguousarray(img, dtype=np.float32)).cuda()
+    return np.squeeze(down_pixel_aggr_device(d, SCALE, integer=integer).cpu().numpy())
+
+
+
+def down_pixel_aggr_device(img, scale, integer=None):
+    """``downPixelAggr`` on the device: CUDA (H, W, C) float32 or uint16 -> CUDA float64 (H // scale, W // scale, C).
+    ``integer``: blur as scipy blurs an integer image (every pass truncated); None = whether ``img`` is uint16.  A float32
+    image holding the values of an integer image (``downPixelAggr``'s upload) passes ``integer=True``."""
+    torch = _capi.require_cuda()
+    if img.dim() != 3 or img.dtype not in (torch.float32, torch.uint16) or not img.is_cuda:
+        raise ValueError("down_pixel_aggr_device: a CUDA (H, W, C) float32 or uint16 tensor, got %s %s"
+                         % (img.dtype, tuple(img.shape)))
+    if integer is None:
+        integer = img.dtype == torch.uint16
+    if img.dtype == torch.uint16:                        # uint16 -> float32 is exact; through int32 (the int16 bits)
+        img = img.view(torch.int16).to(torch.int32).bitwise_and_(0xffff).to(torch.float32)
+    img = img.contiguous()
+    sigma = 1.0 / scale
     radius = int(4.0 * sigma + 0.5)                      # scipy.ndimage.gaussian_filter1d, truncate = 4.0
     x = np.arange(-radius, radius + 1)
     w = np.exp(-0.5 / (sigma * sigma) * x ** 2)
     w = w / w.sum()
-    H, W, C = img.shape
-    d = torch.from_numpy(np.ascontiguousarray(img, dtype=np.float32)).cuda()
-    dw = torch.from_numpy(w).cuda()
-    tmp = torch.empty_like(d)
-    out = torch.empty((H // SCALE, W // SCALE, C), dtype=torch.float64, device=d.device)
-    _capi.check(_capi.lib().dsen2_down_pixel_aggr(_capi.ptr(d), integer, H, W, C, SCALE, _capi.ptr(dw), radius, _capi.ptr(tmp),
-                                                  _capi.ptr(out), _capi.stream_ptr()), "dsen2_down_pixel_aggr")
-    return np.squeeze(out.cpu().numpy())
+    dw = torch.from_numpy(w).to(img.device)
+    H, W, C = (int(s) for s in img.shape)
+    tmp = torch.empty_like(img)
+    out = torch.empty((H // scale, W // scale, C), dtype=torch.float64, device=img.device)
+    with torch.cuda.device(img.device):
+        rc = _capi.lib().dsen2_down_pixel_aggr(_capi.ptr(img), int(bool(integer)), H, W, C, scale, _capi.ptr(dw), radius,
+                                               _capi.ptr(tmp), _capi.ptr(out), _capi.stream_ptr())
+    _capi.check(rc, "dsen2_down_pixel_aggr")
+    return out
 
 
 def save_test_patches(dset_10, dset_20, file, patchSize=128, border=4, interp=True):

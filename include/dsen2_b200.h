@@ -338,6 +338,27 @@ int dsen2_nodata_fill_u16(const void* d_img10, const void* d_img20, const void* 
                           int patch, int border, int first_patch, int num_patches, float nodata, int cout,
                           uint16_t* d_canvas, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Image quality (csrc/metrics.cu; an extension: the measures the DSen2 paper reports, on the device).  d_est (the estimate)
+ * and d_ref (the reference) are contiguous HWC (H, W, C), 1 <= C <= 16, each of its own element type est_dtype / ref_dtype:
+ * DSEN2_IMG_F32, DSEN2_IMG_U16 or DSEN2_IMG_F64 (the float64 of the bicubic baseline; only this entry point takes it).
+ * Every value is read exactly as float64 and all arithmetic is float64.  use_nodata != 0: a pixel is invalid iff every band
+ * of the REFERENCE equals `nodata` in the reference's element type; otherwise every pixel is valid.
+ * d_sums receives 5 C + 2 float64 sums: per band b, over the valid pixels, E_b = sum (est - ref)^2, S_b = sum ref, the
+ * number n of valid pixels, sum Q_b and the number of used windows (UIQ: Wang-Bovik Q of every 8 x 8 window, origins moved
+ * one pixel at a time, whose 64 pixels are valid; means first, then centred sums; a window is used iff
+ * (var_est + var_ref) (mean_est^2 + mean_ref^2) != 0); then the sum of the spectral angles acos(clamp(<est, ref> /
+ * (|est| |ref|), -1, 1)) in RADIANS over the valid pixels whose two vectors are non-zero, and their number.  Deterministic:
+ * fixed reduction trees, no floating-point atomics; the same inputs on the same device give bit-identical sums.  Nothing is
+ * allocated: d_workspace holds dsen2_image_quality_workspace_bytes(H, W, C) bytes (0 for arguments out of range).
+ * DSEN2_E_BADARG: null pointers, H or W < 1, C outside 1..16, an unknown dtype, a NaN nodata, a workspace too small, a
+ * uint16 reference with a nodata that is not an integer in [0, 65535].  H or W < 8 is no error: no window is used.       */
+#define DSEN2_IMG_F64 2
+size_t dsen2_image_quality_workspace_bytes(int H, int W, int C);
+int dsen2_image_quality(const void* d_est, int est_dtype, const void* d_ref, int ref_dtype, int H, int W, int C,
+                        int use_nodata, float nodata, void* d_workspace, size_t workspace_bytes,
+                        double* d_sums, void* stream);
+
 /* Whole s2model forward (model.predict on one batch, supres.py:65) for n patches of (P, P).
  * d_weights[i] / d_bias[i] are the packed layers in Keras topological order (2*num_layers+2 entries):
  *   [0] dsen2_pack_head16_weights (dsen2_pack_head_weights when num_layers == 0, feature_size 128 only),
